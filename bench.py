@@ -12,6 +12,10 @@ losses, one backward, gradient all-reduce (N > 1), Adam.  Under torchrun every r
 (`baseline/_ref`, vendored by ``__graft_entry__.build()``; ``PredictionEngine.train`` around ``DSTDGCN``) on all host
 threads, same workload, batch and dropout as the GPU arm, on a bounded sample; it never touches the GPU library.  The GPU
 arm additionally reports ``gpu_eager_baseline``: the same reference loop with the model on the B200 (torch eager).
+
+``--dump-outputs DIR`` writes what the last timed step computed to ``DIR/<name>.npy`` (train: the loss, the model state
+after the update and the step's gradients; infer: the predictions).  Inputs and weights are seeded, so two builds run
+with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -116,6 +120,37 @@ def perturb(model):
             elif leaf == "R_t":
                 p.fill_(0.01)
     return model
+
+
+DUMP_LIMIT = 64_000_000          # bytes
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Write each numpy array of `arrays` to ``out_dir/<name>.npy``: float64 stays float64, integer counters become
+    float64, everything else float32.  If the files would exceed `limit` bytes in all, the largest arrays keep a fixed,
+    seeded sample of their elements (flattened, in index order), so the same inputs always write the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].size)
+    budget = limit
+    for i, (name, a) in enumerate(items):
+        a = np.asarray(a, dtype=np.float64 if a.dtype == np.float64 or a.dtype.kind in "iu" else np.float32)
+        share = (budget // (len(items) - i) - 128) // a.itemsize          # 128 B: the .npy header
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        budget -= os.path.getsize(path)
+    return limit - budget
+
+
+def train_step_outputs(step, loss):
+    """What a caller of ``TrainStep`` holds after a step: the loss it returned, the model state after the Adam update
+    (parameters and BatchNorm running statistics) and the parameter gradients of that step."""
+    out = {"loss": loss.detach().cpu().numpy()}
+    out.update({f"state.{k}": v.detach().cpu().numpy() for k, v in step.model.state_dict().items()})
+    out.update({f"grad.{k}": step.grad_of(k).detach().cpu().numpy() for k, _ in step.flat.named})
+    return out
 
 
 class ClockSampler:
@@ -450,6 +485,8 @@ def run_infer(args, model, be, dev, rank, world, t, v, t_in):
         sampler.start()
     ms = timed(False, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"predictions": static_out.cpu().numpy()})
     ms_e2e = timed(True, args.steps)
     if rank == 0:
         total = args.batch * world * args.steps
@@ -564,7 +601,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=90.0,
                     help="--impl reference: budget of CPU work for the timed sample (0 = run exactly --steps)")
     ap.add_argument("--no-gpu-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.batch is None:
         args.batch = DEFAULT_BATCH.get(args.workload, 256)
     args.global_batch_fixed = None
@@ -626,9 +669,11 @@ def main():
             dist.barrier()
             torch.cuda.synchronize()
 
+    last_loss = [None]
+
     def run_resident(k):
         for i in range(k):
-            step(*resident[i % nbuf])
+            last_loss[0] = step(*resident[i % nbuf])
 
     def run_e2e(k):
         for i in range(k):
@@ -659,6 +704,8 @@ def main():
         sampler.start()
     ms, launches = timed(run_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, train_step_outputs(step, last_loss[0]))
     run_e2e(2)
     ms_e2e, _ = timed(run_e2e, args.steps)
     if world == 1 and not args.no_secondary and not args.no_graph:

@@ -7,6 +7,8 @@ import re
 import subprocess
 import sys
 
+import numpy as np
+import pytest
 import torch
 
 import bench
@@ -75,3 +77,53 @@ def test_reference_arm_prints_the_contract_line():
         assert cb["kind"] == "reference"                                      # the unmodified reference, not the port
     assert line["e2e"] == {"value": line["value"], "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["config"]["batch_per_gpu"] == 4 and "h36m" in line["config"]["workload"]
+
+
+def test_dump_outputs_samples_large_arrays_within_the_limit(tmp_path):
+    """Small arrays are written whole, larger ones as the same seeded sample every time, all within the byte limit."""
+    rng = np.random.default_rng(1)
+    arrays = {"small": rng.standard_normal(10).astype(np.float32), "count": np.array(7, dtype=np.int64),
+              "wide": rng.standard_normal((300, 300)).astype(np.float32), "big": rng.standard_normal(100_000)}
+    limit = 256 << 10
+    for run in ("a", "b"):
+        assert bench.dump_outputs(str(tmp_path / run), arrays, limit=limit) <= limit
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["big.npy", "count.npy", "small.npy", "wide.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= limit
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in arrays}
+    assert got["small"].dtype == np.float32 and np.array_equal(got["small"], arrays["small"])
+    assert got["count"].dtype == np.float64 and got["count"] == 7
+    assert got["big"].dtype == np.float64 and got["wide"].dtype == np.float32
+    for n in ("big", "wide"):
+        assert 0 < got[n].size < arrays[n].size and np.isin(got[n], arrays[n]).all()
+    for n in arrays:
+        assert np.array_equal(got[n], np.load(tmp_path / "b" / f"{n}.npy"))
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_identical_from_run_to_run(tmp_path):
+    """`bench.py --dump-outputs`: the loss, model state and gradients of the last timed step, float32 / float64 files
+    within 64 MB, bit-identical for two runs with the same arguments (seeded inputs and weights, deterministic kernels)."""
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--batch", "8", "--steps", "3",
+                            "--warmup", "3", "--no-secondary", "--no-cpu-baseline", "--no-gpu-eager-baseline",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 3
+        files = sorted(os.listdir(out))
+        assert sum(os.path.getsize(out / f) for f in files) <= bench.DUMP_LIMIT
+        dumps.append({f: np.load(out / f) for f in files})
+    a, b = dumps
+    assert a.keys() == b.keys() and "loss.npy" in a and np.isfinite(a["loss.npy"]).all()
+    assert "state.encoders.0.0.stgcn.0.0.W_s.npy" in a and "grad.encoders.0.0.stgcn.0.0.W_s.npy" in a
+    for f in a:
+        assert a[f].dtype in (np.float32, np.float64), f
+        assert np.array_equal(a[f], b[f]), f
