@@ -13,8 +13,6 @@
 // Tile format (validated in isolation by tools/umma_test.cu): K-major, no swizzle, 8 x 16 B core matrices,
 //   element (row r, k) at (r/8)*SBO + (k/4)*LBO + (r%8)*16 + (k%4)*4 bytes with LBO = 144 B (not 128: the 16-byte skew
 //   makes the lane = channel stores of the aggregation bank-conflict free) and SBO = (KD/4)*LBO.
-#include <stdlib.h>
-
 #include "kernels.cuh"
 #include "umma.cuh"
 
@@ -472,8 +470,6 @@ static bool tc_geom(int Cin, int Cout, int P, int K, int nb, TcGeom& g, bool wit
 }
 
 bool aggmix_tc_supported(int Cin, int Cout, int P, int K, int nb) {
-  const char* off = getenv("DSTD_DISABLE_TC");      // read per call: tests flip it to cover the CUDA-core kernel too
-  if (off && off[0] && off[0] != '0') return false;
   TcGeom g;
   return tc_geom(Cin, Cout, P, K, nb, g);
 }

@@ -17,8 +17,6 @@
 //      mbarrier that frees the two buffers of that stage (tcgen05.commit), so the conversion of chunk c + 1 and the bulk
 //      copy of its weights overlap the tensor work of chunk c;
 //   epilogue: tcgen05.ld (lane = output row) -> fp32 staging in the freed buffers -> coalesced stores along positions.
-#include <stdlib.h>
-
 #include "kernels.cuh"
 #include "umma.cuh"
 
@@ -521,11 +519,7 @@ __global__ void __launch_bounds__(BT_NT, 2) wgrad_tc_kernel(WgradParams q, Wgrad
   if (warp == 0) umma::tmem_dealloc(tmem, (uint32_t)g.tmem_cols);
 }
 
-bool wgrad_tc_supported(int M, int Cd) {
-  const char* e = getenv("DSTD_BGEMM_TC");
-  if (e && atoi(e) == 0) return false;
-  return M >= 128 && Cd >= 128;
-}
+bool wgrad_tc_supported(int M, int Cd) { return M >= 128 && Cd >= 128; }
 
 // partial must hold wgrad_splits(G) * M * Cd floats (the split count used here never exceeds it); fills q.S
 int launch_wgrad_tc(WgradParams& q, cudaStream_t st) {
@@ -540,8 +534,6 @@ int launch_wgrad_tc(WgradParams& q, cudaStream_t st) {
 }
 
 bool bgemm_tc_supported(int M, int Kd) {
-  const char* e = getenv("DSTD_BGEMM_TC");            // read per call: the tests compare both paths
-  if (e && atoi(e) == 0) return false;
   if (M < 128 || Kd < 64) return false;               // small products stay on the CUDA-core kernel
   const BgemmTcGeom g = tc_geom(M, Kd);
   return g.mtiles <= 5 && g.smem <= (size_t)MAX_DYN_SMEM;

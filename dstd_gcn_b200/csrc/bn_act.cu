@@ -9,8 +9,6 @@
 //
 // Statistics use shifted sums (shift = y[0,c,0,v]) accumulated in fp32 per thread and combined in fp64, so the
 // E[x^2]-E[x]^2 cancellation does not bite on millimetre-scale poses.
-#include <stdlib.h>
-
 #include <initializer_list>
 
 #include "kernels.cuh"
@@ -20,34 +18,17 @@ namespace dstd {
 
 constexpr int BN_THREADS_MAX = 512;
 constexpr int BN_MAXJ = 8;       // positions per thread  -> T*V <= 4096
-// samples in flight per thread (memory-level parallelism): 8 for the dataset shapes (T*V <= 1024), 4 beyond
-static int bn_env(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
 // samples per pipeline stage: the largest of 4/2/1 not above `cap` whose `planes_per_u` staged planes fit `budget`
 static int bn_pick_u(size_t plane_bytes, int planes_per_u, int cap, size_t budget) {
   int u = 4;
   while (u > 1 && (u > cap || (size_t)u * planes_per_u * plane_bytes > budget)) u >>= 1;
   return u;
 }
-static int bn_u_cap() {        // forward apply
-  static const int u = bn_env("DSTD_BN_U", 4);
-  return u;
-}
-static int bn_ub_cap() {       // backward kernels
-  static const int u = bn_env("DSTD_BN_UB", 4);
-  return u;
-}
 static const size_t BN_SMEM_BUDGET = 111 * 1024;   // two CTAs per SM (9 planes of 4 samples at H3.6M = 110.9 KB)
 
-int bn_act_splits(int N, int C) {
-  (void)C;
-  static const int per_cta = [] {
-    const char* e = getenv("DSTD_BN_SAMPLES_PER_CTA");     // tuning knob; default measured best on B200
-    int v = e ? atoi(e) : 32;   // 16 was best with one stream; with the two-stream step 32-64 is (+2 %)
-    return v < 1 ? 1 : v;
-  }();
+// per_cta: Switches::bn_samples_per_cta.  The default 32 is measured best on B200: 16 was best with one stream, with the
+// two-stream step 32-64 is (+2 %)
+static int bn_act_splits(int N, int per_cta) {
   int s = (N + per_cta - 1) / per_cta;
   if (s > 128) s = 128;
   if (s < 1) s = 1;
@@ -1275,11 +1256,9 @@ static bool bnf_slab_ok(const View4& w, int T, int V) {
   const bool dense = bnf_tfast(w) ? (w.sp == 1 && w.sk == T) : (w.sk == 1 && w.sp == V);
   return dense && w.sc == (long long)T * V && (reinterpret_cast<unsigned long long>(w.p) & 15ull) == 0 && (w.sn & 3ll) == 0;
 }
-static BnFastPlan bnf_plan(int C, int T, int V, const float* mask, std::initializer_list<const View4*> ws) {
+static BnFastPlan bnf_plan(bool fast, int C, int T, int V, const float* mask, std::initializer_list<const View4*> ws) {
   BnFastPlan pl{false, 0, 0, 0, false};
-  const char* e = getenv("DSTD_BN_FAST");          // read per call: the tests compare both paths
-  if (e && atoi(e) == 0) return pl;
-  if (mask || V > 32) return pl;
+  if (!fast || mask || V > 32) return pl;
   const int TV = T * V;
   pl.ch = (TV % 4 == 0) ? 1 : (TV % 2 == 0) ? 2 : 4;
   const int chtv = pl.ch * TV;
@@ -1384,11 +1363,12 @@ extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t 
                "bn_act_forward: eval mode needs running statistics");
   DSTD_REQUIRE(a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws, DSTD_ERR_WORKSPACE,
                "bn_act_forward: workspace too small");
+  const Switches sw = read_switches();
   cudaStream_t st = (cudaStream_t)stream;
   BnFwdP q;
   q.N = a->N; q.C = a->C; q.T = a->T; q.V = a->V;
   q.vc_order = a->vc_order; q.training = a->training;
-  q.S = bn_act_splits(a->N, a->C);
+  q.S = bn_act_splits(a->N, sw.bn_samples_per_cta);
   q.eps = a->eps; q.momentum = a->momentum;
   q.y = mk(a->y); q.r = mk(a->r); q.out = mk(a->out);
   q.gamma = a->gamma; q.beta = a->beta;
@@ -1402,7 +1382,7 @@ extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t 
   const size_t tvb = (size_t)q.T * q.V * sizeof(float);
   const size_t sm2 = 2 * tvb;
   const int nst = q.r.p ? 2 : 1;                       // staged tensors: y (, r); two pipeline stages
-  const int u = bn_pick_u(tvb, 2 * nst, bn_u_cap(), BN_SMEM_BUDGET);
+  const int u = bn_pick_u(tvb, 2 * nst, 4, BN_SMEM_BUDGET);
   const size_t smu = (size_t)2 * nst * u * tvb;
   const int cv = q.C * q.V;
   if (q.training) {
@@ -1414,7 +1394,7 @@ extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t 
     count_launch();
     DSTD_LAUNCH_CHECK("bn_eval_stats");
   }
-  const BnFastPlan fp = bnf_plan(q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.out});
+  const BnFastPlan fp = bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.out});
   const int fu = fp.ok ? bnf_pick_u((size_t)fp.ch * tvb, nst, fp.big) : 0;
   if (fu) {   // bulk-copy staged kernel (see "fast path")
     const dim3 grid(q.C / fp.ch, q.S);
@@ -1448,11 +1428,12 @@ extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t
                "bn_act: T*V=%d or V=%d outside the compiled limits", a->T * a->V, a->V);
   DSTD_REQUIRE(a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws, DSTD_ERR_WORKSPACE,
                "bn_act_backward: workspace too small");
+  const Switches sw = read_switches();
   cudaStream_t st = (cudaStream_t)stream;
   BnBwdP q;
   q.N = a->N; q.C = a->C; q.T = a->T; q.V = a->V;
   q.vc_order = a->vc_order; q.training = a->training;
-  q.S = bn_act_splits(a->N, a->C);
+  q.S = bn_act_splits(a->N, sw.bn_samples_per_cta);
   q.y = mk(a->y); q.r = mk(a->r); q.gout = mk(a->gout); q.gy = mk(a->gy); q.gr = mk(a->gr); q.gadd = mk(a->gr_add);
   q.gamma = a->gamma; q.beta = a->beta; q.prelu = a->prelu; q.mask = a->mask;
   q.save_mean = a->save_mean; q.save_invstd = a->save_invstd;
@@ -1467,7 +1448,7 @@ extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t
     const bool use_r = q.r.p && q.prelu, has_gr = q.gr.p != nullptr, add = q.gadd.p != nullptr;
     const bool combo = use_r ? has_gr : (!has_gr && !add);     // the instantiations the model uses
     const bool gr_same = !has_gr || bnf_tfast(q.gr) == bnf_tfast(q.gy);
-    const BnFastPlan fp = (combo && gr_same) ? bnf_plan(q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
+    const BnFastPlan fp = (combo && gr_same) ? bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
                                              : BnFastPlan{false, 0, 0, 0, false};
     const int u1 = fp.ok ? bnf_pick_u((size_t)fp.ch * tv, nst, fp.big) : 0;
     const int u2 = fp.ok ? bnf_pick_u((size_t)fp.ch * tv, nst + (add ? 1 : 0), fp.big) : 0;
@@ -1498,7 +1479,7 @@ extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t
       return DSTD_OK;
     }
   }
-  const int ub = bn_pick_u(tv, 2 * nst + 1, bn_ub_cap(), BN_SMEM_BUDGET);
+  const int ub = bn_pick_u(tv, 2 * nst + 1, 4, BN_SMEM_BUDGET);
   size_t sm_red = (size_t)2 * nst * ub * tv;
   if (sm_red < 2 * tv) sm_red = 2 * tv;
   DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, g.nj, ub, dim3(q.C, q.S), g.threads, sm_red, st, q);

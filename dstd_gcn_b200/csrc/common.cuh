@@ -21,6 +21,20 @@ int num_sms();              // multiprocessors of the current device (148 on B20
 int* device_error_word();   // device pointer to the word (nullptr when it cannot be set up, e.g. under stream capture)
 int poll_device_error(const char* fn);
 
+// The library's environment switches (README.md, "Environment switches").  An entry point that depends on one calls
+// read_switches() once at its start, so a switch flipped between calls takes effect on the next call.  A flag that is
+// unset or empty takes its default, "0" turns it off and any other value turns it on.
+struct Switches {
+  bool unit_tc;           // DSTD_UNIT_TC (off); also on when DSTD_PRECISION selects a reduced mode
+  int unit_terms;         // DSTD_PRECISION: 6 split products per k-step (fp32 parity), 3 (bf16x2) or 1 (bf16)
+  bool aggmix_tc;         // tcgen05 fused forward; off with DSTD_DISABLE_TC
+  bool bgemm_tc;          // DSTD_BGEMM_TC (on): channel GEMMs and weight gradients on tcgen05 where the shape allows
+  bool agg_gen_mma;       // DSTD_AGG_GEN_MMA (off): mma.sync forward aggregation of the shape-generic path
+  bool bn_fast;           // DSTD_BN_FAST (on)
+  int bn_samples_per_cta; // DSTD_BN_SAMPLES_PER_CTA (32)
+};
+Switches read_switches();
+
 #define DSTD_REQUIRE(cond, code, ...)      \
   do {                                     \
     if (!(cond)) {                         \
@@ -38,11 +52,12 @@ int poll_device_error(const char* fn);
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
-// bump allocator over the caller's workspace
+// bump allocator over the caller's workspace; over a null base it only counts: need() is then the workspace size that
+// the same sequence of take() calls requires (arena_need of their byte counts)
 struct Arena {
-  char* base;
+  uintptr_t base;
   size_t cap, off;
-  Arena(void* p, size_t n) : base((char*)p), cap(n), off(0) {}
+  Arena(void* p, size_t n) : base((uintptr_t)p), cap(n), off(0) {}
   template <typename T>
   T* take(size_t count) {
     size_t o = align_up(off, 256);
@@ -50,6 +65,7 @@ struct Arena {
     return (T*)(base + o);
   }
   bool ok() const { return off <= cap; }
+  size_t need() const { return align_up(off, 256) + 256; }
 };
 static inline size_t arena_need(std::initializer_list<size_t> bytes) {
   size_t o = 0;

@@ -2,96 +2,23 @@
 //
 //   pd[p,v,w] = sum_{r,q} Wrm[p, r*P+q] * tanh(m1[r,q,v] - m2[r,q,w]) + brm[p]
 //
-// The pairwise tanh tensor D [2P,K,K] (135-216 KB/sample in the reference) never leaves the SM:
-//   forward : each thread owns NP (v,w) pairs and all P outputs (register tile), computes every tanh once in
-//             registers and streams Wrm^T rows from shared memory (broadcast float4 loads).
-//   backward: per sample, (v,w)-row chunks of D are rebuilt in shared memory and used by two register-blocked
-//             contractions: gWrm += gXm * D^T (accumulated in registers across the whole batch split) and
-//             gD = Wrm^T gXm -> gS = gD (1 - D^2) -> row/column sums give gm1 / gm2.
-#include <stdlib.h>
-
+// Both directions run on mma.sync m16n8k8 TF32 with 3xTF32 compensation (hi*hi + hi*lo + lo*hi), and the pairwise
+// tanh tensor D [2P,K,K] (135-216 KB/sample in the reference) never leaves the SM:
+//   forward : pd = Wrm D + brm, CTA = (sample, branch); the B fragments (D values) are computed in registers in
+//             fragment layout, the A fragments (Wrm) come from shared memory.
+//   backward: persistent CTAs over batch splits; per pair row v, gD = Wrm^T gxm, D evaluated in the accumulator
+//             layout of gD, gS = alpha gD (1 - D^2) and its row/column sums (gm1 / gm2), and gWrm += gxm D^T kept in
+//             registers across the split.
+//   limits: P <= 40, K <= 40 (larger shapes run generic.cu).
 #include "kernels.cuh"
 
 namespace dstd {
 
 // ================================================================================= forward
-template <int RT, int NP>
-__global__ void __launch_bounds__(256) dynadj_fwd_kernel(DynAdjFwdParams q) {
-  extern __shared__ __align__(16) float smem[];
-  const int P = q.P, K = q.K, PK = P * K, KK = K * K, P2 = 2 * P;
-  float* ms = smem;                       // [4][PK]
-  float* wT = ms + ((4 * PK + 3) & ~3);   // [2P][RT]
-  float* bs = wT + P2 * RT;               // [RT]
-  const int n = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
-  const float* mg = q.m + ((long long)(n * q.nb + b) * 4) * PK;
-  const float* wrm = q.w_rm[b];
-  const float* brm = q.b_rm[b];
-  float* pdg = q.pd + (long long)(n * q.nb + b) * P * KK;
-
-  for (int i = tid; i < 4 * PK; i += blockDim.x) ms[i] = __ldg(mg + i);
-
-  const int items = (KK + NP - 1) / NP;
-  for (int p0 = 0; p0 < P; p0 += RT) {
-    __syncthreads();
-    for (int i = tid; i < P2 * RT; i += blockDim.x) {
-      int k = i / RT, pp = i - k * RT;
-      wT[i] = (p0 + pp < P) ? __ldg(wrm + (long long)(p0 + pp) * P2 + k) : 0.f;
-    }
-    for (int i = tid; i < RT; i += blockDim.x) bs[i] = (p0 + i < P) ? __ldg(brm + p0 + i) : 0.f;
-    __syncthreads();
-    for (int item = tid; item < items; item += blockDim.x) {
-      int vi[NP], wi[NP];
-#pragma unroll
-      for (int i = 0; i < NP; ++i) {
-        int e = item * NP + i;
-        if (e >= KK) e = KK - 1;
-        vi[i] = e / K;
-        wi[i] = e - vi[i] * K;
-      }
-      float acc[RT][NP];
-#pragma unroll
-      for (int pp = 0; pp < RT; ++pp)
-#pragma unroll
-        for (int i = 0; i < NP; ++i) acc[pp][i] = bs[pp];
-#pragma unroll 2
-      for (int k = 0; k < P2; ++k) {
-        const int r = (k >= P) ? 1 : 0;
-        const float* m1 = ms + r * PK + (k - r * P) * K;
-        const float* m2 = m1 + 2 * PK;
-        float d[NP];
-#pragma unroll
-        for (int i = 0; i < NP; ++i) d[i] = fast_tanh(m1[vi[i]] - m2[wi[i]]);
-        const float4* w4 = reinterpret_cast<const float4*>(wT + k * RT);
-#pragma unroll
-        for (int p4 = 0; p4 < RT / 4; ++p4) {
-          float4 w = w4[p4];
-#pragma unroll
-          for (int i = 0; i < NP; ++i) {
-            acc[p4 * 4 + 0][i] = fmaf(w.x, d[i], acc[p4 * 4 + 0][i]);
-            acc[p4 * 4 + 1][i] = fmaf(w.y, d[i], acc[p4 * 4 + 1][i]);
-            acc[p4 * 4 + 2][i] = fmaf(w.z, d[i], acc[p4 * 4 + 2][i]);
-            acc[p4 * 4 + 3][i] = fmaf(w.w, d[i], acc[p4 * 4 + 3][i]);
-          }
-        }
-      }
-#pragma unroll
-      for (int pp = 0; pp < RT; ++pp) {
-        if (p0 + pp < P) {
-#pragma unroll
-          for (int i = 0; i < NP; ++i) {
-            int e = item * NP + i;
-            if (e < KK) pdg[(long long)(p0 + pp) * KK + e] = acc[pp][i];
-          }
-        }
-      }
-    }
-  }
-}
-
-// ---- tensor-path forward: pd[p][e] = sum_k Wrm[p][k] D[k][e] + brm[p] as mma.sync m16n8k8 TF32 (3xTF32) with the
-// B fragments (the pairwise tanh values) COMPUTED IN REGISTERS in fragment layout: every D element is evaluated by
-// exactly one lane, never stored, and feeds all 16-row tiles of p; the A fragments (Wrm) come from shared memory.
-// The CUDA-core version above is limited by the shared-memory return path (one broadcast weight delivery per FMA).
+// pd[p][e] = sum_k Wrm[p][k] D[k][e] + brm[p] as mma.sync m16n8k8 TF32 (3xTF32) with the B fragments (the pairwise
+// tanh values) COMPUTED IN REGISTERS in fragment layout: every D element is evaluated by exactly one lane, never stored,
+// and feeds all 16-row tiles of p; the A fragments (Wrm) come from shared memory.  A CUDA-core version with a register
+// tile of p was limited by the shared-memory return path (one broadcast weight delivery per FMA; DESIGN.md section 3).
 __device__ __forceinline__ void fsplit3(float x, uint32_t& hi, uint32_t& lo) {
   hi = __float_as_uint(x) & 0xffffe000u;
   lo = __float_as_uint(x - __uint_as_float(hi));
@@ -200,61 +127,17 @@ static int dynadj_fwd_mma_launch(const DynAdjFwdParams& q, cudaStream_t st) {
   return check_launch("dynadj_fwd_mma");
 }
 
-template <int RT>
-static int dynadj_fwd_launch(const DynAdjFwdParams& q, cudaStream_t st) {
-  constexpr int NP = 2;
-  const int KK = q.K * q.K, PK = q.P * q.K;
-  int items = (KK + NP - 1) / NP;
-  int rounds = cdiv(items, 256);
-  int threads = cdiv(cdiv(items, rounds), 32) * 32;
-  size_t smem = ((size_t)((4 * PK + 3) & ~3) + (size_t)2 * q.P * RT + RT) * sizeof(float);
-  auto kern = dynadj_fwd_kernel<RT, NP>;
-  if (smem > 48 * 1024) {
-    DSTD_REQUIRE(smem <= 220 * 1024, DSTD_ERR_UNSUPPORTED, "dynadj_fwd: P=%d K=%d needs %zu B shared memory", q.P, q.K,
-                 smem);
-    ensure_max_smem((const void*)kern);
-  }
-  kern<<<dim3(q.N, q.nb), threads, smem, st>>>(q);
-  count_launch();
-  return check_launch("dynadj_fwd");
-}
+bool dynadj_supported(int P, int K) { return P >= 1 && P <= 40 && K >= 1 && K <= 40; }
 
 int launch_dynadj_fwd(const DynAdjFwdParams& q, cudaStream_t st) {
-  static const bool simt = getenv("DSTD_DYNADJ_FWD_SIMT") != nullptr;   // A/B switch: CUDA-core version
-  if (!simt) {
-    if (q.P <= 16) return dynadj_fwd_mma_launch<1>(q, st);
-    if (q.P <= 32) return dynadj_fwd_mma_launch<2>(q, st);
-    if (q.P <= 48) return dynadj_fwd_mma_launch<3>(q, st);
-  }
-  if (q.P <= 24) return dynadj_fwd_launch<24>(q, st);
-  if (q.P <= 28) return dynadj_fwd_launch<28>(q, st);
-  if (q.P <= 36) return dynadj_fwd_launch<36>(q, st);
-  return dynadj_fwd_launch<40>(q, st);   // P > 40: several register-tile passes (tanh recomputed per pass)
+  DSTD_REQUIRE(dynadj_supported(q.P, q.K), DSTD_ERR_UNSUPPORTED,
+               "dynadj_fwd: P=%d K=%d outside the compiled tile limits (P, K <= 40)", q.P, q.K);
+  if (q.P <= 16) return dynadj_fwd_mma_launch<1>(q, st);
+  if (q.P <= 32) return dynadj_fwd_mma_launch<2>(q, st);
+  return dynadj_fwd_mma_launch<3>(q, st);
 }
 
 // ================================================================================= backward
-struct BwdGeom {
-  int RV, ECP, WLD;
-  size_t smem_floats;
-};
-static BwdGeom bwd_geom(int P, int K) {
-  BwdGeom g;
-  g.RV = 100 / K;
-  if (g.RV < 1) g.RV = 1;
-  if (g.RV > K) g.RV = K;
-  int ec = g.RV * K;
-  g.ECP = ec <= 36 ? 36 : ec <= 68 ? 68 : ec <= 100 ? 100 : ((ec + 31) / 32 * 32 + 4);
-  g.WLD = ((2 * P + 7) / 8) * 8;
-  size_t pk4 = (size_t)((4 * P * K + 3) & ~3);
-  g.smem_floats = 2 * pk4 + (size_t)2 * P * g.ECP + (size_t)(2 * P + 1) * g.ECP + (size_t)P * g.WLD +
-                  (size_t)((K * K + 3) & ~3) + 32;
-  return g;
-}
-
-bool dynadj_supported(int P, int K) {
-  if (P > 40 || P < 1 || K < 1) return false;
-  return bwd_geom(P, K).smem_floats * sizeof(float) <= 220 * 1024;
-}
 
 // batch splits = persistent CTAs per branch: one CTA per SM in total (the tensor-path kernel keeps its gWrm tile in
 // registers across its samples, so fewer, longer CTAs amortise the prologue and the partial write-out)
@@ -262,236 +145,6 @@ int dynadj_bwd_splits(int N, int nb) {
   int s = num_sms() / (nb < 1 ? 1 : nb);
   if (s < 1) s = 1;
   return N < s ? N : s;
-}
-
-template <int TMA, int TNA>
-__global__ void __launch_bounds__(256) dynadj_bwd_kernel(DynAdjBwdParams q, int RV, int ECP, int WLD) {
-  extern __shared__ __align__(16) float smem[];
-  const int P = q.P, K = q.K, PK = P * K, KK = K * K, P2 = 2 * P;
-  const int pk4 = (4 * PK + 3) & ~3;
-  float* ms = smem;                    // [4][PK]
-  float* gms = ms + pk4;               // [4][PK]
-  float* gX = gms + pk4;               // [2][P][ECP]  double buffered (cp.async prefetch of the next chunk)
-  float* Ds = gX + 2 * P * ECP;        // [2P+1][ECP]
-  float* Ws = Ds + (P2 + 1) * ECP;     // [P][WLD]
-  float* gA = Ws + P * WLD;            // [KK]
-  float* red = gA + ((KK + 3) & ~3);   // [32]
-
-  const int tid = threadIdx.x, lane = tid & 31, ty = tid >> 5;
-  const int b = blockIdx.y;
-  const float alpha = q.alpha ? __ldg(q.alpha) : 1.0f;
-  const float* wrm = q.w_rm[b];
-
-  for (int i = tid; i < P * WLD; i += 256) {
-    int p = i / WLD, k = i - p * WLD;
-    Ws[i] = (k < P2) ? __ldg(wrm + (long long)p * P2 + k) : 0.f;
-  }
-  for (int i = tid; i < KK; i += 256) gA[i] = 0.f;
-
-  float accW[TMA][TNA];
-#pragma unroll
-  for (int a = 0; a < TMA; ++a)
-#pragma unroll
-    for (int c = 0; c < TNA; ++c) accW[a][c] = 0.f;
-  float galpha = 0.f;
-
-  // clamped row/column indices of this thread's gWrm tile
-  int prow[TMA], kcol[TNA];
-#pragma unroll
-  for (int a = 0; a < TMA; ++a) prow[a] = min(ty + 8 * a, P - 1);
-#pragma unroll
-  for (int c = 0; c < TNA; ++c) kcol[c] = min(lane + 32 * c, P2);
-
-  const int n_kt = (P2 + 7) / 8, n_et = ECP / 4;
-
-  // per-lane decode of the <= 4 chunk columns it touches (ec = lane + 32 i -> local row vl, column w)
-  int c_vl[4], c_w[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int ec = lane + 32 * i;
-    c_vl[i] = ec / K;
-    c_w[i] = ec - c_vl[i] * K;
-  }
-  const int nchunks = (K + RV - 1) / RV;
-  const int nsamp = (q.N - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  const long long total = (long long)nsamp * nchunks;     // (sample, chunk) steps of this CTA
-
-  // cp.async prefetch of the gxm chunk of step `st` into buffer st & 1 (zero filled beyond the chunk)
-  auto prefetch = [&](long long st) {
-    const int n = (int)blockIdx.x + (int)(st / nchunks) * (int)gridDim.x;
-    const int v0 = (int)(st % nchunks) * RV;
-    const int EC = min(RV, K - v0) * K, e0 = v0 * K;
-    const float* src = q.gxm + ((long long)n * q.nb + b) * P * KK + e0;
-    float* dst = gX + (st & 1) * P * ECP;
-    for (int p = ty; p < P; p += 8)
-      for (int ec = lane; ec < ECP; ec += 32) cp_async4(dst + p * ECP + ec, src + (long long)p * KK + ec, ec < EC);
-  };
-  if (total > 0) prefetch(0);
-
-  // optional per-phase cycle counters (-DDSTD_PHASE_TIMING, printed by CTA 0)
-#ifdef DSTD_PHASE_TIMING
-  long long tph[6] = {0, 0, 0, 0, 0, 0}, tlast = clock64();
-#define DPH(i) do { __syncthreads(); long long _t = clock64(); tph[i] += _t - tlast; tlast = _t; } while (0)
-#else
-#define DPH(i) do {} while (0)
-#endif
-  for (long long st = 0; st < total; ++st) {
-    const int n = (int)blockIdx.x + (int)(st / nchunks) * (int)gridDim.x;
-    const int ci = (int)(st % nchunks);
-    const int v0 = ci * RV, rows = min(RV, K - v0), EC = rows * K, e0 = v0 * K;
-    const long long nb_ = (long long)n * q.nb + b;
-    const float* gXc = gX + (st & 1) * P * ECP;
-    if (ci == 0) {   // new sample: its reduction rows, zeroed gradient rows
-      __syncthreads();
-      const float* mg = q.m + nb_ * 4 * PK;
-      for (int i = tid; i < 4 * PK; i += 256) {
-        ms[i] = __ldg(mg + i);
-        gms[i] = 0.f;
-      }
-    }
-    cp_async_wait_all();
-    __syncthreads();                       // chunk st landed; everyone is done with the other buffer and with Ds
-    if (st + 1 < total) prefetch(st + 1);  // overlaps with the whole chunk below
-
-    DPH(0);
-    // 2. rebuild D chunk (+ ones row for the bias gradient); galpha += gxm * pd on the way
-    {
-      const float* pdg = q.pd + nb_ * P * KK + e0;
-      for (int k = ty; k <= P2; k += 8) {
-        const int r = (k >= P) ? 1 : 0, qq = k - r * P;
-        const float* m1 = ms + r * PK + qq * K + v0;
-        const float* m2 = ms + (2 + r) * PK + qq * K;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int ec = lane + 32 * i;
-          if (ec < ECP) {
-            float d = 0.f;
-            if (ec < EC) d = (k < P2) ? fast_tanh(m1[c_vl[i]] - m2[c_w[i]]) : 1.0f;
-            Ds[k * ECP + ec] = d;
-          }
-        }
-      }
-      for (int p = ty; p < P; p += 8) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int ec = lane + 32 * i;
-          if (ec < EC) galpha = fmaf(gXc[p * ECP + ec], __ldg(pdg + (long long)p * KK + ec), galpha);
-        }
-      }
-    }
-    __syncthreads();
-    DPH(1);
-    // 3a. static-adjacency gradient: sum over p
-    if (tid < EC) {
-      float s = 0.f;
-      for (int p = 0; p < P; ++p) s += gXc[p * ECP + tid];
-      gA[e0 + tid] += s;
-    }
-    // 3b. gWrm (+bias column) += gXm * D^T
-    for (int e4 = 0; e4 < ECP; e4 += 4) {
-      float4 g4[TMA], d4[TNA];
-#pragma unroll
-      for (int a = 0; a < TMA; ++a) g4[a] = *reinterpret_cast<const float4*>(gXc + prow[a] * ECP + e4);
-#pragma unroll
-      for (int c = 0; c < TNA; ++c) d4[c] = *reinterpret_cast<const float4*>(Ds + kcol[c] * ECP + e4);
-#pragma unroll
-      for (int a = 0; a < TMA; ++a)
-#pragma unroll
-        for (int c = 0; c < TNA; ++c) {
-          accW[a][c] = fmaf(g4[a].x, d4[c].x, accW[a][c]);
-          accW[a][c] = fmaf(g4[a].y, d4[c].y, accW[a][c]);
-          accW[a][c] = fmaf(g4[a].z, d4[c].z, accW[a][c]);
-          accW[a][c] = fmaf(g4[a].w, d4[c].w, accW[a][c]);
-        }
-    }
-    __syncthreads();
-    DPH(2);
-    // 4. gS = alpha * (Wrm^T gXm) * (1 - D^2), written over D
-    for (int tile = tid; tile < n_kt * n_et; tile += 256) {
-      const int kt = tile / n_et, et = tile - kt * n_et;
-      float acc[8][4];
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-      const float* wp = Ws + kt * 8;
-      const float* gp = gXc + et * 4;
-#pragma unroll 5
-      for (int p = 0; p < P; ++p) {
-        const float4 w0 = *reinterpret_cast<const float4*>(wp + p * WLD);
-        const float4 w1 = *reinterpret_cast<const float4*>(wp + p * WLD + 4);
-        const float4 g = *reinterpret_cast<const float4*>(gp + p * ECP);
-        const float wv[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-        const float gv[4] = {g.x, g.y, g.z, g.w};
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(wv[i], gv[j], acc[i][j]);
-      }
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const int k = kt * 8 + i;
-        if (k < P2) {
-          float4* dp = reinterpret_cast<float4*>(Ds + k * ECP + et * 4);
-          float4 d = *dp;
-          d.x = alpha * acc[i][0] * (1.0f - d.x * d.x);
-          d.y = alpha * acc[i][1] * (1.0f - d.y * d.y);
-          d.z = alpha * acc[i][2] * (1.0f - d.z * d.z);
-          d.w = alpha * acc[i][3] * (1.0f - d.w * d.w);
-          *dp = d;
-        }
-      }
-    }
-    __syncthreads();
-    DPH(3);
-    // 5. gm1[k,v] = sum_w gS (lanes 24.. : one local row each) ; gm2[k,w] = -sum_v gS (lanes 0..K-1, K <= 24;
-    //    wider K: second pass)
-    for (int k = ty; k < P2; k += 8) {
-      const int r = (k >= P) ? 1 : 0, qq = k - r * P;
-      const float* drow = Ds + k * ECP;
-      for (int w = lane; w < K; w += 32) {
-        float s = 0.f;
-        for (int vl = 0; vl < rows; ++vl) s += drow[vl * K + w];
-        gms[(2 + r) * PK + qq * K + w] -= s;
-      }
-      const int vl = 31 - lane;              // the last lanes take the row sums
-      if (vl < rows) {
-        float s = 0.f;
-        for (int w = 0; w < K; ++w) s += drow[vl * K + w];
-        gms[r * PK + qq * K + v0 + vl] += s;
-      }
-    }
-    DPH(4);
-    if (ci == nchunks - 1) {                 // sample finished: its gm rows go out
-      __syncthreads();
-      float* gmg = q.gm + nb_ * 4 * PK;
-      for (int i = tid; i < 4 * PK; i += 256) gmg[i] = gms[i];
-    }
-  }
-
-#ifdef DSTD_PHASE_TIMING
-  if (blockIdx.x == 0 && blockIdx.y == 0 && tid == 0)
-    printf("dynadj_bwd phases (cycles, CTA 0): wait/stage %lld rebuildD %lld gA+gWrm %lld gS %lld sums %lld\n", tph[0],
-           tph[1], tph[2], tph[3], tph[4]);
-#endif
-  // per-split partials
-  const long long sb = (long long)blockIdx.x * q.nb + b;
-  float* pw = q.part_wrm + sb * P * (P2 + 1);
-#pragma unroll
-  for (int a = 0; a < TMA; ++a) {
-    int p = ty + 8 * a;
-    if (p >= P) continue;
-#pragma unroll
-    for (int c = 0; c < TNA; ++c) {
-      int k = lane + 32 * c;
-      if (k <= P2) pw[p * (P2 + 1) + k] = alpha * accW[a][c];
-    }
-  }
-  __syncthreads();
-  float* pa = q.part_adj + sb * KK;
-  for (int i = tid; i < KK; i += 256) pa[i] = gA[i];
-  float ga = block_sum(galpha, red);
-  if (tid == 0) q.part_alpha[sb] = ga;
 }
 
 // ---- tensor-path backward.  Per (sample, branch) and per row v of the pair grid, with channels k = 0..2P-1:
@@ -504,9 +157,8 @@ __global__ void __launch_bounds__(256) dynadj_bwd_kernel(DynAdjBwdParams q, int 
 //         k-slot permutation slot t <-> pair 2t, slot t+4 <-> pair 2t+1 makes the C layout of (i) a B layout) and
 //         A = gxm chunk rows; accumulators live in registers across the whole batch split.
 // A warp owns one 16-channel tile (kt) and every VS-th row v.  All products are 3xTF32 (hi*hi + hi*lo + lo*hi); every
-// cross-warp sum is done in a fixed order (no atomics), so results are run-to-run identical.
-// The CUDA-core kernel above rebuilds D in shared memory and is limited by the shared-memory return path
-// (profiles/r01_dynadj_bwd_phase_cycles.md).
+// cross-warp sum is done in a fixed order (no atomics), so results are run-to-run identical.  A CUDA-core version that
+// rebuilt D in shared memory was limited by the shared-memory return path (DESIGN.md section 3).
 template <int KSTEPS, int WT>
 __global__ void __launch_bounds__(384) dynadj_bwd_mma_kernel(DynAdjBwdParams q, int KT, int VS) {
   constexpr int MTP = (KSTEPS + 1) / 2;   // 16-row tiles of p
@@ -791,33 +443,14 @@ static int dynadj_bwd_mma_launch(const DynAdjBwdParams& q, cudaStream_t st) {
 
 int launch_dynadj_bwd(const DynAdjBwdParams& q, cudaStream_t st) {
   DSTD_REQUIRE(dynadj_supported(q.P, q.K), DSTD_ERR_UNSUPPORTED,
-               "dynadj_bwd: P=%d K=%d outside the compiled tile limits (P<=40)", q.P, q.K);
-  static const bool simt = getenv("DSTD_DYNADJ_BWD_SIMT") != nullptr;   // A/B switch: CUDA-core version
-  if (!simt) {
-    const int ks = q.P <= 24 ? 3 : 5, wt = q.K <= 24 ? 3 : q.K <= 32 ? 4 : 5;
-    if (ks == 3 && wt == 3) return dynadj_bwd_mma_launch<3, 3>(q, st);
-    if (ks == 3 && wt == 4) return dynadj_bwd_mma_launch<3, 4>(q, st);
-    if (ks == 3 && wt == 5) return dynadj_bwd_mma_launch<3, 5>(q, st);
-    if (ks == 5 && wt == 3) return dynadj_bwd_mma_launch<5, 3>(q, st);
-    if (ks == 5 && wt == 4) return dynadj_bwd_mma_launch<5, 4>(q, st);
-    return dynadj_bwd_mma_launch<5, 5>(q, st);
-  }
-  BwdGeom g = bwd_geom(q.P, q.K);
-  size_t smem = g.smem_floats * sizeof(float);
-  int tma = cdiv(q.P, 8), tna = cdiv(2 * q.P + 1, 32);
-  dim3 grid(q.S, q.nb);
-#define DSTD_DYN_BWD(A, C)                                                                        \
-  {                                                                                               \
-    auto kern = dynadj_bwd_kernel<A, C>;                                                          \
-    if (smem > 48 * 1024) ensure_max_smem((const void*)kern);                                                  \
-    kern<<<grid, 256, smem, st>>>(q, g.RV, g.ECP, g.WLD);                                         \
-  }
-  if (tma <= 3 && tna <= 2) DSTD_DYN_BWD(3, 2)
-  else if (tma <= 4 && tna <= 2) DSTD_DYN_BWD(4, 2)
-  else DSTD_DYN_BWD(5, 3)
-#undef DSTD_DYN_BWD
-  count_launch();
-  return check_launch("dynadj_bwd");
+               "dynadj_bwd: P=%d K=%d outside the compiled tile limits (P, K <= 40)", q.P, q.K);
+  const int ks = q.P <= 24 ? 3 : 5, wt = q.K <= 24 ? 3 : q.K <= 32 ? 4 : 5;
+  if (ks == 3 && wt == 3) return dynadj_bwd_mma_launch<3, 3>(q, st);
+  if (ks == 3 && wt == 4) return dynadj_bwd_mma_launch<3, 4>(q, st);
+  if (ks == 3 && wt == 5) return dynadj_bwd_mma_launch<3, 5>(q, st);
+  if (ks == 5 && wt == 3) return dynadj_bwd_mma_launch<5, 3>(q, st);
+  if (ks == 5 && wt == 4) return dynadj_bwd_mma_launch<5, 4>(q, st);
+  return dynadj_bwd_mma_launch<5, 5>(q, st);
 }
 
 }  // namespace dstd

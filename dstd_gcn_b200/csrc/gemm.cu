@@ -234,8 +234,8 @@ static void wgrad_dispatch_tn(const WgradParams& q, int tn, dim3 grid, cudaStrea
 }
 
 // partial must hold wgrad_splits(G) * M * Cd floats
-int launch_wgrad(WgradParams& q, cudaStream_t st) {
-  if (wgrad_tc_supported(q.M, q.Cd)) return launch_wgrad_tc(q, st);     // tcgen05 path (bgemm_tc.cu)
+int launch_wgrad(WgradParams& q, bool tc, cudaStream_t st) {
+  if (tc && wgrad_tc_supported(q.M, q.Cd)) return launch_wgrad_tc(q, st);     // tcgen05 path (bgemm_tc.cu)
   q.S = wgrad_splits(q.G);
   long long per = (q.G + q.S - 1) / q.S;
   q.cols_per_split = (per + 31) / 32 * 32;

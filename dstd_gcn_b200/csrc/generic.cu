@@ -5,8 +5,6 @@
 // (deterministic).  The pairwise tanh tensor D (2750 KB per sample at the stress shape) is produced and consumed in
 // (k', pair) tiles and never leaves the SM; the channel contraction of these shapes runs in bgemm / wgrad (gemm.cu).
 //   limits: P <= 128, K <= 128.
-#include <stdlib.h>
-
 #include "kernels.cuh"
 
 namespace dstd {
@@ -482,15 +480,9 @@ __global__ void __launch_bounds__(256) aggregate_fwd_gen_mma_kernel(AggParams q)
   }
 }
 
-static bool agg_gen_mma_on(int K) {
-  const char* e = getenv("DSTD_AGG_GEN_MMA");          // read per call (A/B in the tests)
-  const bool on = e ? atoi(e) != 0 : false;
-  return on && K >= 48;
-}
-
-int launch_aggregate_fwd_gen(const AggParams& q, cudaStream_t st) {
+int launch_aggregate_fwd_gen(const AggParams& q, bool mma, cudaStream_t st) {
   DSTD_REQUIRE(generic_supported(q.P, q.K), DSTD_ERR_UNSUPPORTED, "aggregate_fwd_gen: P=%d K=%d outside limits", q.P, q.K);
-  if (agg_gen_mma_on(q.K)) {
+  if (mma && q.K >= 48) {
     const int KP8 = (q.K + 7) & ~7, KLD = agm_kld(q.K);
     const size_t sm = (size_t)KP8 * KLD * sizeof(float);
     dim3 grid(q.P, q.N);

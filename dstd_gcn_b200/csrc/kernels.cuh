@@ -38,7 +38,7 @@ struct WgradParams {
   long long cols_per_split;
 };
 int wgrad_splits(long long G);
-int launch_wgrad(WgradParams& q, cudaStream_t st);   // fills q.S (number of partials actually written)
+int launch_wgrad(WgradParams& q, bool tc, cudaStream_t st);   // fills q.S (partials written); tc: tcgen05 allowed
 bool wgrad_tc_supported(int M, int Cd);
 int launch_wgrad_tc(WgradParams& q, cudaStream_t st);   // tcgen05 version (bgemm_tc.cu), same contract
 
@@ -134,7 +134,7 @@ int launch_dynadj_fwd_gen(const DynAdjFwdParams& q, cudaStream_t st);
 int dynadj_gen_tiles(int K);                                               // v tiles per (sample, branch)
 size_t dynadj_bwd_gen_ws_floats(int N, int nb, int P, int K);              // gm2 partials
 int launch_dynadj_bwd_gen(const DynAdjBwdParams& q, float* gm2_part, cudaStream_t st);   // q.S == N * tiles slots; part_adj: N slots
-int launch_aggregate_fwd_gen(const AggParams& q, cudaStream_t st);
+int launch_aggregate_fwd_gen(const AggParams& q, bool mma, cudaStream_t st);   // mma: mma.sync kernel for K >= 48
 int launch_aggregate_bwd_gen(const AggParams& q, cudaStream_t st);
 
 // ------------------------------------------------------------------ aggmix.cu
@@ -187,11 +187,9 @@ int aggmix_bwd_ctas(int N, int P, int K, int Cin, int Cout, int nb);
 bool unit_tc_supported(int Cin, int Cout, int P, int K, int nb);
 size_t unit_tc_ws_bytes(int nb);
 int unit_bwd_tc_ctas(int N, int Cin, int Cout, int P, int K, int nb);
-int launch_unit_fwd_tc(const AggMixParams& q, const PackParams& pk, void* ws, cudaStream_t st);
-int launch_unit_bwd_tc(const AggMixBwdParams& q, const PackParams& pk, void* ws, cudaStream_t st);
-
-// ------------------------------------------------------------------ bn_act.cu
-int bn_act_splits(int N, int C);
+// terms: split products per k-step (Switches::unit_terms)
+int launch_unit_fwd_tc(const AggMixParams& q, const PackParams& pk, void* ws, int terms, cudaStream_t st);
+int launch_unit_bwd_tc(const AggMixBwdParams& q, const PackParams& pk, void* ws, int terms, cudaStream_t st);
 
 // ------------------------------------------------------------------ misc.cu
 struct PackParams {

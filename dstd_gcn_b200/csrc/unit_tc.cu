@@ -22,8 +22,6 @@
 // kind::f16 contracts K = 16 per instruction).
 // All accumulators are M = 64 (channels on the TMEM lanes); results return through tcgen05.ld with thread = channel row,
 // which is exactly the order in which the next row image is written (16-byte stores, bank-conflict free).
-#include <stdlib.h>
-
 #include "kernels.cuh"
 #include "umma.cuh"
 
@@ -819,21 +817,14 @@ __global__ void pack_w16_kernel(PackParams q, unsigned char* wimg) {
 }
 
 // ------------------------------------------------------------------------------------------ geometry / launch
-// DSTD_PRECISION (secondary, stated-tolerance modes; the default "fp32" is the parity path): "bf16x2" keeps the products
-// hh + hm + mh (relative error ~2^-15), "bf16" only hh (plain bf16 operands, fp32 accumulate, ~2^-8).  Both run on these
-// kernels (there is no other reduced-precision implementation), so they imply DSTD_UNIT_TC=1.
-static int unit_terms() {
-  const char* p = getenv("DSTD_PRECISION");
-  if (p && p[0] == 'b' && p[1] == 'f' && p[2] == '1' && p[3] == '6') return (p[4] == 'x' && p[5] == '2') ? 3 : 1;
-  return 6;
-}
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
-// bwd: X0, G1 and scratch images; fwd: X0 and scratch.  The largest F (frames per item) that fits 227 KB wins.
-static bool unit_geom(int Cin, int Cout, int P, int K, int nb, bool bwd, UnitGeom& g) {
+// bwd: X0, G1 and scratch images; fwd: X0 and scratch.  The largest F (frames per item) that fits 227 KB wins.  The
+// product count `terms` does not change the geometry.
+static bool unit_geom(int Cin, int Cout, int P, int K, int nb, bool bwd, int terms, UnitGeom& g) {
   if (K < 1 || K > 40 || K * ((K + 1) / 2) > 2 * UT_NT || Cin < 1 || Cin > 64 || Cout < 1 || Cout > 64 || nb < 1 || nb > DSTD_MAX_BRANCH) return false;
   g.KQ = round_up(K, 8);
-  g.terms = unit_terms();
+  g.terms = terms;
   g.KW = round_up(K, 16);
   g.CinK = round_up(Cin, 16);
   g.CoutK = round_up(Cout, 16);
@@ -884,23 +875,20 @@ static bool unit_geom(int Cin, int Cout, int P, int K, int nb, bool bwd, UnitGeo
 // Opt-in (DSTD_UNIT_TC=1): measured on B200 at the H3.6M encoder shape, batch 256, the all-tcgen05 kernels are at parity
 // with the mma.sync / tcgen05-mix forward (unit forward 0.358 vs 0.353 ms) and 20 % behind the mma.sync backward
 // (0.82 vs 0.68 ms; 8.3 k vs 9.6 k samples/s for the whole step): the six-term bf16 chains re-read every operand from
-// shared memory per instruction and M = 64 accumulators run at half rate (DESIGN.md section 3).  Read per call: the
-// tests flip it to cover both paths.
-static bool unit_tc_enabled() {
-  const char* on = getenv("DSTD_UNIT_TC");
-  return (on && on[0] == '1') || unit_terms() != 6;
-}
-
+// shared memory per instruction and M = 64 accumulators run at half rate (DESIGN.md section 3).
+// DSTD_PRECISION (secondary, stated-tolerance modes; the default "fp32" is the parity path): "bf16x2" keeps the products
+// hh + hm + mh (relative error ~2^-15), "bf16" only hh (plain bf16 operands, fp32 accumulate, ~2^-8).  Both run on these
+// kernels (there is no other reduced-precision implementation), so they imply DSTD_UNIT_TC=1 (read_switches, api.cu).
 bool unit_tc_supported(int Cin, int Cout, int P, int K, int nb) {
   UnitGeom g;
-  return unit_tc_enabled() && unit_geom(Cin, Cout, P, K, nb, true, g) && unit_geom(Cin, Cout, P, K, nb, false, g);
+  return unit_geom(Cin, Cout, P, K, nb, true, 6, g) && unit_geom(Cin, Cout, P, K, nb, false, 6, g);
 }
 
 size_t unit_tc_ws_bytes(int nb) { return (size_t)nb * 3 * UT_WP_B + 256; }
 
 int unit_bwd_tc_ctas(int N, int Cin, int Cout, int P, int K, int nb) {
   UnitGeom g;
-  if (!unit_geom(Cin, Cout, P, K, nb, true, g)) return 0;
+  if (!unit_geom(Cin, Cout, P, K, nb, true, 6, g)) return 0;
   const long long items = (long long)N * cdiv(P, g.F);
   const int sms = num_sms();
   return (int)(items < sms ? items : sms);
@@ -913,9 +901,9 @@ static int pack_w16(const PackParams& pk, unsigned char* ws, int** err_flag, cud
   return check_launch("pack_w16");
 }
 
-int launch_unit_fwd_tc(const AggMixParams& a, const PackParams& pk, void* ws, cudaStream_t st) {
+int launch_unit_fwd_tc(const AggMixParams& a, const PackParams& pk, void* ws, int terms, cudaStream_t st) {
   UnitGeom g;
-  DSTD_REQUIRE(unit_geom(a.Cin, a.Cout, a.P, a.K, a.nb, false, g), DSTD_ERR_UNSUPPORTED, "unit_fwd_tc: shape outside limits");
+  DSTD_REQUIRE(unit_geom(a.Cin, a.Cout, a.P, a.K, a.nb, false, terms, g), DSTD_ERR_UNSUPPORTED, "unit_fwd_tc: shape outside limits");
   int* err_flag;
   int rc = pack_w16(pk, (unsigned char*)ws, &err_flag, st);
   if (rc) return rc;
@@ -936,9 +924,9 @@ int launch_unit_fwd_tc(const AggMixParams& a, const PackParams& pk, void* ws, cu
   return check_launch("unit_fwd_tc");
 }
 
-int launch_unit_bwd_tc(const AggMixBwdParams& a, const PackParams& pk, void* ws, cudaStream_t st) {
+int launch_unit_bwd_tc(const AggMixBwdParams& a, const PackParams& pk, void* ws, int terms, cudaStream_t st) {
   UnitGeom g;
-  DSTD_REQUIRE(unit_geom(a.Cin, a.Cout, a.P, a.K, a.nb, true, g), DSTD_ERR_UNSUPPORTED, "unit_bwd_tc: shape outside limits");
+  DSTD_REQUIRE(unit_geom(a.Cin, a.Cout, a.P, a.K, a.nb, true, terms, g), DSTD_ERR_UNSUPPORTED, "unit_bwd_tc: shape outside limits");
   int* err_flag;
   int rc = pack_w16(pk, (unsigned char*)ws, &err_flag, st);
   if (rc) return rc;
