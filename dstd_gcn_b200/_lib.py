@@ -95,6 +95,11 @@ SYMBOLS = {
     "dstd_bn_act_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
     "dstd_bn_act_forward": (C.c_int, [C.POINTER(BnFwdArgs), C.c_void_p]),
     "dstd_bn_act_backward": (C.c_int, [C.POINTER(BnBwdArgs), C.c_void_p]),
+    "dstd_bn_sync_buffer_doubles": (C.c_size_t, [C.c_int, C.c_int]),
+    "dstd_bn_act_forward_local": (C.c_int, [C.POINTER(BnFwdArgs), C.c_void_p, C.c_void_p]),
+    "dstd_bn_act_forward_global": (C.c_int, [C.POINTER(BnFwdArgs), C.c_void_p, C.c_int, C.c_void_p]),
+    "dstd_bn_act_backward_local": (C.c_int, [C.POINTER(BnBwdArgs), C.c_void_p, C.c_void_p]),
+    "dstd_bn_act_backward_global": (C.c_int, [C.POINTER(BnBwdArgs), C.c_void_p, C.c_int, C.c_void_p]),
     "dstd_chmix_bwd_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
     "dstd_chmix_forward": (C.c_int, [C.POINTER(ChmixFwdArgs), C.c_void_p]),
     "dstd_chmix_backward": (C.c_int, [C.POINTER(ChmixBwdArgs), C.c_void_p]),
@@ -274,14 +279,15 @@ class CudaBackend:
         return gx, galpha, grads
 
     # -- BN + residual + PReLU + mask
-    def bn_act_forward(self, y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask, vc_order, training,
-                       eps, momentum, out_like=None):
+    def _bn_fwd_args(self, y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask, vc_order, training, eps,
+                     momentum, out_like, with_ws=True):
+        """Fills dstd_bn_act_fwd_args; returns (args, out, save_mean, save_invstd, workspace or None)."""
         n, c, t, v = y.shape
         dev = y.device
         out = torch.empty_like(out_like if out_like is not None else y, device=dev)
         save_mean = torch.empty((c * v,), dtype=torch.float32, device=dev)
         save_invstd = torch.empty((c * v,), dtype=torch.float32, device=dev)
-        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), dev)
+        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), dev) if with_ws else None
         if nbt is not None:
             _check(nbt, "num_batches_tracked", torch.int64)
         a = BnFwdArgs()
@@ -293,20 +299,30 @@ class CudaBackend:
         a.num_batches_tracked = _ptr(nbt)
         a.prelu, a.mask = _cptr(prelu, "prelu"), _cptr(mask, "mask")
         a.save_mean, a.save_invstd = _ptr(save_mean), _ptr(save_invstd)
-        a.ws, a.ws_bytes = _ptr(ws), ws.numel()
+        a.ws, a.ws_bytes = _ptr(ws), (ws.numel() if ws is not None else 0)
+        return a, out, save_mean, save_invstd, ws
+
+    def bn_act_forward(self, y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask, vc_order, training,
+                       eps, momentum, out_like=None):
+        a, out, save_mean, save_invstd, ws = self._bn_fwd_args(y, r, gamma, beta, running_mean, running_var, nbt, prelu,
+                                                               mask, vc_order, training, eps, momentum, out_like)
         self._ok(self.lib.dstd_bn_act_forward(C.byref(a), _stream()), "dstd_bn_act_forward")
         return out, save_mean, save_invstd
 
-    def bn_act_backward(self, y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, training,
-                        need_gr=True, gr_add=None):
+    @staticmethod
+    def _bn_grad_bufs(y, r, prelu, need_gr):
+        """gy, gr (None unless r and need_gr), ggamma, gbeta, gprelu (None without PReLU): uninitialised."""
         n, c, t, v = y.shape
         dev = y.device
-        gy = torch.empty_like(y)
         gr = torch.empty_like(r) if (r is not None and need_gr) else None
-        ggamma = torch.empty((c * v,), dtype=torch.float32, device=dev)
-        gbeta = torch.empty((c * v,), dtype=torch.float32, device=dev)
         gprelu = torch.empty((1,), dtype=torch.float32, device=dev) if prelu is not None else None
-        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), dev)
+        return (torch.empty_like(y), gr, torch.empty((c * v,), dtype=torch.float32, device=dev),
+                torch.empty((c * v,), dtype=torch.float32, device=dev), gprelu)
+
+    def _bn_bwd_args(self, y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, training, gy, gr,
+                     gr_add, ggamma=None, gbeta=None, gprelu=None, ws=None):
+        """Fills dstd_bn_act_bwd_args with the given output buffers (None = not passed)."""
+        n, c, t, v = y.shape
         a = BnBwdArgs()
         a.N, a.C, a.T, a.V = n, c, t, v
         a.vc_order, a.training = int(vc_order), int(training)
@@ -317,9 +333,75 @@ class CudaBackend:
         a.prelu, a.mask = _cptr(prelu, "prelu"), _cptr(mask, "mask")
         a.save_mean, a.save_invstd = _cptr(save_mean, "save_mean"), _cptr(save_invstd, "save_invstd")
         a.ggamma, a.gbeta, a.gprelu = _ptr(ggamma), _ptr(gbeta), _ptr(gprelu)
-        a.ws, a.ws_bytes = _ptr(ws), ws.numel()
+        a.ws, a.ws_bytes = _ptr(ws), (ws.numel() if ws is not None else 0)
+        return a
+
+    def bn_act_backward(self, y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, training,
+                        need_gr=True, gr_add=None):
+        n, c, t, v = y.shape
+        gy, gr, ggamma, gbeta, gprelu = self._bn_grad_bufs(y, r, prelu, need_gr)
+        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), y.device)
+        a = self._bn_bwd_args(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, training, gy, gr,
+                              gr_add, ggamma, gbeta, gprelu, ws)
         self._ok(self.lib.dstd_bn_act_backward(C.byref(a), _stream()), "dstd_bn_act_backward")
         return gy, gr, ggamma, gbeta, gprelu
+
+    # -- synchronised BN: the two phases of each direction around an all-gather of fp64 rows (include/dstd_b200.h)
+    def _bn_rows(self, y, rows, what):
+        n, c, t, v = y.shape
+        _check(rows, what, torch.float64)
+        per = int(self.lib.dstd_bn_sync_buffer_doubles(c, v))
+        if not rows.is_contiguous() or rows.numel() % per:
+            raise RuntimeError(f"dstd_gcn_b200: `{what}` must be a contiguous multiple of {per} doubles")
+        return rows.numel() // per
+
+    def bn_act_forward_local(self, y, vc_order):
+        """This rank's exchange rows (count, mean, M2) [3*C*V] fp64 of a training-mode BN over y."""
+        n, c, t, v = y.shape
+        rows = torch.empty((int(self.lib.dstd_bn_sync_buffer_doubles(c, v)),), dtype=torch.float64, device=y.device)
+        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), y.device)
+        a = BnFwdArgs()
+        a.N, a.C, a.T, a.V = n, c, t, v
+        a.vc_order, a.training = int(vc_order), 1
+        a.y = _view(y, "y")
+        a.ws, a.ws_bytes = _ptr(ws), ws.numel()
+        self._ok(self.lib.dstd_bn_act_forward_local(C.byref(a), _ptr(rows), _stream()), "dstd_bn_act_forward_local")
+        return rows
+
+    def bn_act_forward_global(self, y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask, vc_order, eps,
+                              momentum, all_rows, out_like=None):
+        """Statistics merged from the gathered rows of every rank; same results as bn_act_forward."""
+        world = self._bn_rows(y, all_rows, "all_rows")
+        a, out, save_mean, save_invstd, _ = self._bn_fwd_args(y, r, gamma, beta, running_mean, running_var, nbt, prelu,
+                                                              mask, vc_order, True, eps, momentum, out_like,
+                                                              with_ws=False)
+        self._ok(self.lib.dstd_bn_act_forward_global(C.byref(a), _ptr(all_rows), world, _stream()),
+                 "dstd_bn_act_forward_global")
+        return out, save_mean, save_invstd
+
+    def bn_act_backward_local(self, y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order,
+                              need_gr=True, gr_add=None):
+        """This rank's parameter gradients and exchange rows (count, sum g', sum g' xhat) [3*C*V] fp64, plus the
+        (not yet written) gy / gr buffers for bn_act_backward_global: their layouts pick the kernels of both phases."""
+        n, c, t, v = y.shape
+        gy, gr, ggamma, gbeta, gprelu = self._bn_grad_bufs(y, r, prelu, need_gr)
+        ws = self._ws(self.lib.dstd_bn_act_workspace_bytes(n, c, t, v), y.device)
+        a = self._bn_bwd_args(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, True, gy, gr,
+                              gr_add, ggamma, gbeta, gprelu, ws)
+        rows = torch.empty((int(self.lib.dstd_bn_sync_buffer_doubles(c, v)),), dtype=torch.float64, device=y.device)
+        self._ok(self.lib.dstd_bn_act_backward_local(C.byref(a), _ptr(rows), _stream()), "dstd_bn_act_backward_local")
+        return ggamma, gbeta, gprelu, rows, gy, gr
+
+    def bn_act_backward_global(self, y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, all_rows,
+                               gy, gr=None, gr_add=None):
+        """Writes gy (and gr) of the global batch, from the gathered rows of every rank, into the buffers that
+        bn_act_backward_local returned; returns them."""
+        world = self._bn_rows(y, all_rows, "all_rows")
+        a = self._bn_bwd_args(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, True, gy, gr,
+                              gr_add)
+        self._ok(self.lib.dstd_bn_act_backward_global(C.byref(a), _ptr(all_rows), world, _stream()),
+                 "dstd_bn_act_backward_global")
+        return gy, gr
 
     # -- 1x1 channel mix
     def chmix_forward(self, xu, w, b):

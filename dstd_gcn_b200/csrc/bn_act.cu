@@ -684,8 +684,30 @@ __device__ __forceinline__ void bn_bwd_apply_consume(const BnBwdP& q, const floa
   }
 }
 
-template <int NJ, int U, bool ADD>
-__device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q) {
+// Synchronised BatchNorm (dstd_bn_act_backward_global): k1 = sum(g') / n and k2 = sum(g' xhat) / n over the global
+// batch, from the gathered exchange rows (count, sum g', sum g' xhat) of the `world` ranks, summed in rank order in
+// fp64.  tot[v] of channel c receives (k1, k2).
+__device__ __forceinline__ void sync_bwd_totals(const double* all, int world, int C, int V, int c, int vc_order,
+                                                double (*tot)[2]) {
+  const long long cv = (long long)C * V;
+  for (int v = threadIdx.x; v < V; v += blockDim.x) {
+    const int pi = bn_pidx(c, v, C, V, vc_order);
+    double n = 0., s1 = 0., s2 = 0.;
+    for (int r = 0; r < world; ++r) {
+      const double* row = all + 3 * cv * r + pi;
+      n += row[0];
+      s1 += row[cv];
+      s2 += row[2 * cv];
+    }
+    tot[v][0] = s1 / n;
+    tot[v][1] = s2 / n;
+  }
+}
+
+// SYNC: the global phase of the synchronised backward.  k1 / k2 come from the gathered rows (`all`, `world`) instead
+// of the split partials, and the parameter gradients are not written (the local phase wrote this rank's share).
+template <int NJ, int U, bool ADD, bool SYNC>
+__device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double* all, int world) {
   extern __shared__ float sh[];   // [2 stages][nst = 2 (gout, y), + r, + gr_add][U][T*V], then [U][T*V] for gr
   const int c = blockIdx.x, s = blockIdx.y, T = q.T, V = q.V, TV = T * V;
   const int n0 = (int)((long long)q.N * s / q.S), n1 = (int)((long long)q.N * (s + 1) / q.S), cnt = n1 - n0;
@@ -723,18 +745,23 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q) {
   // sums of pass 1 over the splits; the s == 0 CTA of the channel publishes the parameter gradients
   __shared__ double tot[32][2];
   __shared__ float red[32];
-  sum_partials(q.part, q.S, q.C, c, V, tot);
-  if (c == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
-    float a = 0.f;
-    for (int i = threadIdx.x; i < q.S * q.C; i += blockDim.x) a += q.part_p[i];
-    const float t = block_sum(a, red);
-    if (threadIdx.x == 0) q.gprelu[0] = t;
-  }
-  __syncthreads();
-  if (s == 0 && threadIdx.x < V) {
-    const int pi = bn_pidx(c, threadIdx.x, q.C, V, q.vc_order);
-    q.gbeta[pi] = (float)tot[threadIdx.x][0];
-    q.ggamma[pi] = (float)tot[threadIdx.x][1];
+  if (SYNC) {
+    sync_bwd_totals(all, world, q.C, V, c, q.vc_order, tot);
+    __syncthreads();
+  } else {
+    sum_partials(q.part, q.S, q.C, c, V, tot);
+    if (c == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
+      float a = 0.f;
+      for (int i = threadIdx.x; i < q.S * q.C; i += blockDim.x) a += q.part_p[i];
+      const float t = block_sum(a, red);
+      if (threadIdx.x == 0) q.gprelu[0] = t;
+    }
+    __syncthreads();
+    if (s == 0 && threadIdx.x < V) {
+      const int pi = bn_pidx(c, threadIdx.x, q.C, V, q.vc_order);
+      q.gbeta[pi] = (float)tot[threadIdx.x][0];
+      q.ggamma[pi] = (float)tot[threadIdx.x][1];
+    }
   }
   // per position: xhat = (y - mu) * is;  gy = gi * (gp - k1 - xhat * k2)
   float mu[NJ], is[NJ], g[NJ], b[NJ], gi[NJ], k1[NJ], k2[NJ];
@@ -758,7 +785,10 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q) {
         g[i] = __ldg(q.gamma + pi);
         b[i] = __ldg(q.beta + pi);
         gi[i] = g[i] * is[i];
-        if (q.training) {
+        if (SYNC) {
+          k1[i] = (float)tot[v][0];
+          k2[i] = (float)tot[v][1];
+        } else if (q.training) {
           k1[i] = (float)tot[v][0] * icnt;
           k2[i] = (float)tot[v][1] * icnt;
         }
@@ -826,13 +856,22 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q) {
 
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_kernel(BnBwdP q) {
-  bn_bwd_apply_body<NJ, U, false>(q);
+  bn_bwd_apply_body<NJ, U, false, false>(q, nullptr, 0);
 }
 // same with a fourth staged tensor, gr_add, summed into gr (separate instantiation: the plain kernel sits at the
 // 64-register cap and pays ~13 % for the extra slots)
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_kernel(BnBwdP q) {
-  bn_bwd_apply_body<NJ, U, true>(q);
+  bn_bwd_apply_body<NJ, U, true, false>(q, nullptr, 0);
+}
+// the global phase of the synchronised backward (k1, k2 from the gathered rows)
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_sync_kernel(BnBwdP q, const double* all, int world) {
+  bn_bwd_apply_body<NJ, U, false, true>(q, all, world);
+}
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_sync_kernel(BnBwdP q, const double* all, int world) {
+  bn_bwd_apply_body<NJ, U, true, true>(q, all, world);
 }
 
 // ================================================================================================ fast path
@@ -1143,8 +1182,9 @@ __device__ __forceinline__ void bnf_bwd_apply_consume(const float* st, const flo
   }
 }
 
-template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
-__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_kernel(BnBwdP q, int CH, int NP, int* err) {
+// SYNC: global phase of the synchronised backward, as in bn_bwd_apply_body
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG, bool SYNC>
+__device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int NP, int* err, const double* all, int world) {
   extern __shared__ __align__(16) float sh[];   // [2 stages][gout, y (, r) (, gr_add)][U][CH * T*V]
   __shared__ __align__(16) float4 ctab[BNF_MAXCH * 32];     // mean, invstd, gamma, beta
   __shared__ __align__(16) float4 ctab2[BNF_MAXCH * 32];    // gamma * invstd, k1, k2
@@ -1184,7 +1224,7 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
   };
   if (threadIdx.x == 0 && iters > 0) issue(0);
   // sums of pass 1 over the splits; the s == 0 CTA publishes the parameter gradients of its channels
-  if (blockIdx.x == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
+  if (!SYNC && blockIdx.x == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
     float a = 0.f;
     for (int i = threadIdx.x; i < NP; i += blockDim.x) a += q.part_p[i];
     const float t = block_sum(a, red);
@@ -1192,17 +1232,22 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
   }
   for (int ch = 0; ch < CH; ++ch) {
     const int c = c0 + ch;
-    sum_partials(q.part, q.S, q.C, c, V, tot);
+    if (SYNC) sync_bwd_totals(all, world, q.C, V, c, q.vc_order, tot);
+    else sum_partials(q.part, q.S, q.C, c, V, tot);
     __syncthreads();
     if (threadIdx.x < V) {
       const int v = threadIdx.x, pi = bn_pidx(c, v, q.C, V, q.vc_order);
       const float mu = __ldg(q.save_mean + pi), is = __ldg(q.save_invstd + pi), g = __ldg(q.gamma + pi);
       ctab[ch * 32 + v] = make_float4(mu, is, g, __ldg(q.beta + pi));
-      ctab2[ch * 32 + v] = make_float4(g * is, q.training ? (float)tot[v][0] * icnt : 0.f,
-                                       q.training ? (float)tot[v][1] * icnt : 0.f, 0.f);
-      if (s == 0) {
-        q.gbeta[pi] = (float)tot[v][0];
-        q.ggamma[pi] = (float)tot[v][1];
+      if (SYNC) {
+        ctab2[ch * 32 + v] = make_float4(g * is, (float)tot[v][0], (float)tot[v][1], 0.f);
+      } else {
+        ctab2[ch * 32 + v] = make_float4(g * is, q.training ? (float)tot[v][0] * icnt : 0.f,
+                                         q.training ? (float)tot[v][1] * icnt : 0.f, 0.f);
+        if (s == 0) {
+          q.gbeta[pi] = (float)tot[v][0];
+          q.ggamma[pi] = (float)tot[v][1];
+        }
       }
     }
     __syncthreads();
@@ -1241,6 +1286,95 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
     gyb += U * gysn;
     if (HAS_GR) grb += U * grsn;
     __syncthreads();
+  }
+}
+
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_kernel(BnBwdP q, int CH, int NP, int* err) {
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, false>(q, CH, NP, err, nullptr, 0);
+}
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_sync_kernel(BnBwdP q, int CH, int* err, const double* all, int world) {
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, true>(q, CH, 0, err, all, world);
+}
+
+// ---- synchronised BatchNorm: fold and merge kernels around the exchange of per-rank rows
+// Exchange rows of one rank, fp64, in BN parameter order: [3][C*V] = (count, mean, M2) in the forward,
+// (count, sum g', sum g' xhat) in the backward.  One CTA per channel (fold), one thread per parameter index (merge).
+
+// forward, local phase: this rank's split partials (shifted sums) -> (count, mean_r, M2_r)
+__global__ void bn_sync_fold_fwd_kernel(BnFwdP q, double* mine) {
+  __shared__ double tot[32][2];
+  const int c = blockIdx.x, V = q.V;
+  const long long cv = (long long)q.C * V;
+  sum_partials(q.part, q.S, q.C, c, V, tot);
+  __syncthreads();
+  if (threadIdx.x < V) {
+    const int v = threadIdx.x, pi = bn_pidx(c, v, q.C, V, q.vc_order);
+    const double cntd = (double)q.N * q.T;
+    const double shift = __ldg(q.y.p + vix(q.y, 0, c, 0, v));
+    const double dm = tot[v][0] / cntd;
+    double m2 = tot[v][1] - tot[v][0] * dm;
+    if (m2 < 0.) m2 = 0.;
+    mine[pi] = cntd;
+    mine[cv + pi] = shift + dm;
+    mine[2 * cv + pi] = m2;
+  }
+}
+
+// forward, global phase: Chan's merge of the `world` rows in rank order -> save_mean / save_invstd, running statistics
+// (global count, unbiased variance), num_batches_tracked
+__global__ void bn_sync_merge_fwd_kernel(BnFwdP q, const double* all, int world) {
+  const long long cv = (long long)q.C * q.V;
+  const int pi = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pi >= cv) return;
+  double n = 0., s = 0.;
+  for (int r = 0; r < world; ++r) {
+    const double nr = all[3 * cv * r + pi];
+    n += nr;
+    s += nr * all[3 * cv * r + cv + pi];
+  }
+  const double mean = s / n;
+  double m2 = 0.;
+  for (int r = 0; r < world; ++r) {
+    const double* row = all + 3 * cv * r + pi;
+    const double d = row[cv] - mean;
+    m2 += row[2 * cv] + row[0] * d * d;
+  }
+  const double var = m2 / n;
+  q.save_mean[pi] = (float)mean;
+  q.save_invstd[pi] = (float)(1.0 / sqrt(var + (double)q.eps));
+  if (q.running_mean) {
+    const double unb = n > 1. ? m2 / (n - 1.) : var;
+    q.running_mean[pi] = (float)((1.0 - q.momentum) * q.running_mean[pi] + q.momentum * mean);
+    q.running_var[pi] = (float)((1.0 - q.momentum) * q.running_var[pi] + q.momentum * unb);
+  }
+  if (pi == 0 && q.nbt) *q.nbt += 1;
+}
+
+// backward, local phase: this rank's parameter gradients (the sums and the order of bn_bwd_apply / bnf_bwd_apply:
+// launched with the block size of the apply kernel the plain call would run, over its NP slope partials) and its
+// exchange rows (count, sum g', sum g' xhat)
+__global__ void bn_sync_fold_bwd_kernel(BnBwdP q, int NP, double* mine) {
+  __shared__ double tot[32][2];
+  __shared__ float red[32];
+  const int c = blockIdx.x, V = q.V;
+  const long long cv = (long long)q.C * V;
+  sum_partials(q.part, q.S, q.C, c, V, tot);
+  if (c == 0 && q.gprelu) {
+    float a = 0.f;
+    for (int i = threadIdx.x; i < NP; i += blockDim.x) a += q.part_p[i];
+    const float t = block_sum(a, red);
+    if (threadIdx.x == 0) q.gprelu[0] = t;
+  }
+  __syncthreads();
+  if (threadIdx.x < V) {
+    const int v = threadIdx.x, pi = bn_pidx(c, v, q.C, V, q.vc_order);
+    q.gbeta[pi] = (float)tot[v][0];
+    q.ggamma[pi] = (float)tot[v][1];
+    mine[pi] = (double)q.N * q.T;
+    mine[cv + pi] = tot[v][0];
+    mine[2 * cv + pi] = tot[v][1];
   }
 }
 
@@ -1303,30 +1437,30 @@ static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false) {
   } while (0)
 
 // U (samples per pipeline stage) is a launch-time choice among the compiled instantiations
-#define DSTD_BN_CASE(kern, NJ_, u, grid, threads, smem, st, q)                       \
+#define DSTD_BN_CASE(kern, NJ_, u, grid, threads, smem, st, ...)                     \
   do {                                                                                \
     switch (u) {                                                                      \
       case 4:                                                                         \
         prefer_smem_carveout((const void*)kern<NJ_, 4>, true);                        \
-        kern<NJ_, 4><<<grid, threads, smem, st>>>(q);                                 \
+        kern<NJ_, 4><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
         break;                                                                        \
       case 2:                                                                         \
         prefer_smem_carveout((const void*)kern<NJ_, 2>, true);                        \
-        kern<NJ_, 2><<<grid, threads, smem, st>>>(q);                                 \
+        kern<NJ_, 2><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
         break;                                                                        \
       default:                                                                        \
         prefer_smem_carveout((const void*)kern<NJ_, 1>, true);                        \
-        kern<NJ_, 1><<<grid, threads, smem, st>>>(q);                                 \
+        kern<NJ_, 1><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
         break;                                                                        \
     }                                                                                 \
   } while (0)
-#define DSTD_BN_DISPATCH_U(kern, nj, u, grid, threads, smem, st, q)                  \
+#define DSTD_BN_DISPATCH_U(kern, nj, u, grid, threads, smem, st, ...)                \
   do {                                                                                \
     switch (nj) {                                                                     \
-      case 1: DSTD_BN_CASE(kern, 1, u, grid, threads, smem, st, q); break;            \
-      case 2: DSTD_BN_CASE(kern, 2, u, grid, threads, smem, st, q); break;            \
-      case 4: DSTD_BN_CASE(kern, 4, u, grid, threads, smem, st, q); break;            \
-      default: DSTD_BN_CASE(kern, 8, u, grid, threads, smem, st, q); break;           \
+      case 1: DSTD_BN_CASE(kern, 1, u, grid, threads, smem, st, __VA_ARGS__); break;  \
+      case 2: DSTD_BN_CASE(kern, 2, u, grid, threads, smem, st, __VA_ARGS__); break;  \
+      case 4: DSTD_BN_CASE(kern, 4, u, grid, threads, smem, st, __VA_ARGS__); break;  \
+      default: DSTD_BN_CASE(kern, 8, u, grid, threads, smem, st, __VA_ARGS__); break; \
     }                                                                                 \
   } while (0)
 
@@ -1351,21 +1485,24 @@ extern "C" size_t dstd_bn_act_workspace_bytes(int N, int C, int T, int V) {
   return arena_need({(size_t)S * C * V * 2 * sizeof(float), (size_t)S * C * sizeof(float)});
 }
 
-extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t stream) {
+// Which call an argument check serves: the plain one, or the local / global phase of a synchronised one.  The local
+// forward reads y only (and the workspace); the global phases read no workspace; the global backward writes no
+// parameter gradients.
+enum BnPhase { BN_PLAIN, BN_LOCAL, BN_GLOBAL };
+
+// ---- forward: argument checks and kernel parameters shared by the plain call and the two synchronised phases
+static int bn_fwd_setup(const dstd_bn_act_fwd_args* a, const Switches& sw, BnFwdP& q, BnPhase ph = BN_PLAIN) {
   DSTD_REQUIRE(a, DSTD_ERR_BAD_ARG, "bn_act_forward: null args");
   DSTD_REQUIRE(a->N > 0 && a->C > 0 && a->T > 0 && a->V > 0, DSTD_ERR_BAD_ARG, "bn_act_forward: bad dims");
-  DSTD_REQUIRE(a->y.ptr && a->out.ptr && a->gamma && a->beta && a->save_mean && a->save_invstd, DSTD_ERR_BAD_ARG,
-               "bn_act_forward: null tensor");
+  DSTD_REQUIRE(a->y.ptr && (ph == BN_LOCAL || (a->out.ptr && a->gamma && a->beta && a->save_mean && a->save_invstd)),
+               DSTD_ERR_BAD_ARG, "bn_act_forward: null tensor");
   DSTD_REQUIRE(a->T * a->V <= BN_MAXJ * BN_THREADS_MAX && a->V <= 32, DSTD_ERR_UNSUPPORTED,
                "bn_act: T*V=%d (max %d) or V=%d (max 32) outside the compiled limits", a->T * a->V,
                BN_MAXJ * BN_THREADS_MAX, a->V);
   DSTD_REQUIRE(a->training || (a->running_mean && a->running_var), DSTD_ERR_BAD_ARG,
                "bn_act_forward: eval mode needs running statistics");
-  DSTD_REQUIRE(a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws, DSTD_ERR_WORKSPACE,
-               "bn_act_forward: workspace too small");
-  const Switches sw = read_switches();
-  cudaStream_t st = (cudaStream_t)stream;
-  BnFwdP q;
+  DSTD_REQUIRE(ph == BN_GLOBAL || (a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws),
+               DSTD_ERR_WORKSPACE, "bn_act_forward: workspace too small");
   q.N = a->N; q.C = a->C; q.T = a->T; q.V = a->V;
   q.vc_order = a->vc_order; q.training = a->training;
   q.S = bn_act_splits(a->N, sw.bn_samples_per_cta);
@@ -1376,27 +1513,29 @@ extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t 
   q.nbt = a->num_batches_tracked;
   q.prelu = a->prelu; q.mask = a->mask;
   q.save_mean = a->save_mean; q.save_invstd = a->save_invstd;
-  Arena ar(a->ws, a->ws_bytes);
-  q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
-  BnGeom g = bn_geom(q.T, q.V);
-  const size_t tvb = (size_t)q.T * q.V * sizeof(float);
-  const size_t sm2 = 2 * tvb;
-  const int nst = q.r.p ? 2 : 1;                       // staged tensors: y (, r); two pipeline stages
-  const int u = bn_pick_u(tvb, 2 * nst, 4, BN_SMEM_BUDGET);
-  const size_t smu = (size_t)2 * nst * u * tvb;
-  const int cv = q.C * q.V;
-  if (q.training) {
-    DSTD_BN_DISPATCH(bn_stats_kernel, g.nj, dim3(q.C, q.S), g.threads, sm2, st, q);
-    count_launch();
-    DSTD_LAUNCH_CHECK("bn_stats");
-  } else {
-    bn_eval_stats_kernel<<<cdiv(cv, 128), 128, 0, st>>>(q);
-    count_launch();
-    DSTD_LAUNCH_CHECK("bn_eval_stats");
+  q.part = nullptr;
+  if (ph != BN_GLOBAL) {
+    Arena ar(a->ws, a->ws_bytes);
+    q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
   }
+  return DSTD_OK;
+}
+
+static int bn_fwd_stats(const BnFwdP& q, cudaStream_t st) {
+  const BnGeom g = bn_geom(q.T, q.V);
+  DSTD_BN_DISPATCH(bn_stats_kernel, g.nj, dim3(q.C, q.S), g.threads, 2 * (size_t)q.T * q.V * sizeof(float), st, q);
+  count_launch();
+  DSTD_LAUNCH_CHECK("bn_stats");
+  return DSTD_OK;
+}
+
+// the apply pass: bulk-copy staged kernel when the layouts allow it (see "fast path"), the generic one otherwise
+static int bn_fwd_apply(const BnFwdP& q, const Switches& sw, cudaStream_t st) {
+  const size_t tvb = (size_t)q.T * q.V * sizeof(float);
+  const int nst = q.r.p ? 2 : 1;                       // staged tensors: y (, r); two pipeline stages
   const BnFastPlan fp = bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.out});
   const int fu = fp.ok ? bnf_pick_u((size_t)fp.ch * tvb, nst, fp.big) : 0;
-  if (fu) {   // bulk-copy staged kernel (see "fast path")
+  if (fu) {
     const dim3 grid(q.C / fp.ch, q.S);
     const size_t smem = (size_t)2 * nst * fu * fp.ch * tvb;
     int* err = device_error_word();
@@ -1410,27 +1549,91 @@ extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t 
     DSTD_LAUNCH_CHECK("bnf_apply");
     return DSTD_OK;
   }
+  const BnGeom g = bn_geom(q.T, q.V);
+  const int u = bn_pick_u(tvb, 2 * nst, 4, BN_SMEM_BUDGET);
+  const size_t smu = (size_t)2 * nst * u * tvb;
   DSTD_BN_DISPATCH_U(bn_apply_kernel, g.nj, u, dim3(q.C, q.S), g.threads, smu, st, q);
   count_launch();
   DSTD_LAUNCH_CHECK("bn_apply");
   return DSTD_OK;
 }
 
-extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t stream) {
+extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t stream) {
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnFwdP q;
+  int rc = bn_fwd_setup(a, sw, q);
+  if (rc != DSTD_OK) return rc;
+  if (q.training) {
+    rc = bn_fwd_stats(q, st);
+    if (rc != DSTD_OK) return rc;
+  } else {
+    bn_eval_stats_kernel<<<cdiv(q.C * q.V, 128), 128, 0, st>>>(q);
+    count_launch();
+    DSTD_LAUNCH_CHECK("bn_eval_stats");
+  }
+  return bn_fwd_apply(q, sw, st);
+}
+
+extern "C" size_t dstd_bn_sync_buffer_doubles(int C, int V) { return (size_t)3 * C * V; }
+
+extern "C" int dstd_bn_act_forward_local(const dstd_bn_act_fwd_args* a, double* mine, dstd_stream_t stream) {
+  DSTD_REQUIRE(a && a->training == 1, DSTD_ERR_BAD_ARG, "bn_act_forward_local: needs training = 1");
+  DSTD_REQUIRE(mine, DSTD_ERR_BAD_ARG, "bn_act_forward_local: null exchange buffer");
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnFwdP q;
+  int rc = bn_fwd_setup(a, sw, q, BN_LOCAL);
+  if (rc != DSTD_OK) return rc;
+  rc = bn_fwd_stats(q, st);
+  if (rc != DSTD_OK) return rc;
+  bn_sync_fold_fwd_kernel<<<q.C, 256, 0, st>>>(q, mine);
+  count_launch();
+  DSTD_LAUNCH_CHECK("bn_sync_fold_fwd");
+  return DSTD_OK;
+}
+
+extern "C" int dstd_bn_act_forward_global(const dstd_bn_act_fwd_args* a, const double* all, int world,
+                                          dstd_stream_t stream) {
+  DSTD_REQUIRE(a && a->training == 1, DSTD_ERR_BAD_ARG, "bn_act_forward_global: needs training = 1");
+  DSTD_REQUIRE(all && world >= 1, DSTD_ERR_BAD_ARG, "bn_act_forward_global: null exchange buffer or world < 1");
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnFwdP q;
+  int rc = bn_fwd_setup(a, sw, q, BN_GLOBAL);
+  if (rc != DSTD_OK) return rc;
+  bn_sync_merge_fwd_kernel<<<cdiv(q.C * q.V, 128), 128, 0, st>>>(q, all, world);
+  count_launch();
+  DSTD_LAUNCH_CHECK("bn_sync_merge_fwd");
+  q.training = 0;          // the apply kernels' eval branch: normalise with save_mean / save_invstd as given
+  return bn_fwd_apply(q, sw, st);
+}
+
+// ---- backward: shared argument checks, kernel parameters and the kernel plan
+struct BnBwdPlan {
+  BnFastPlan fp;
+  int u1, u2;        // fast path: samples per stage of the reduce / apply pass (both nonzero = fast path taken)
+  int ub, ub2;       // generic path: the same
+  int nst, nst2;     // staged tensors of the reduce / apply pass
+  bool use_r, add;
+  BnGeom g;
+  bool fast() const { return u1 && u2; }
+};
+
+// (the local phase takes gy / gr as well: it does not write them, but their layouts pick the kernels, as in the plain
+// call)
+static int bn_bwd_setup(const dstd_bn_act_bwd_args* a, const Switches& sw, BnBwdP& q, BnPhase ph = BN_PLAIN) {
   DSTD_REQUIRE(a, DSTD_ERR_BAD_ARG, "bn_act_backward: null args");
   DSTD_REQUIRE(a->N > 0 && a->C > 0 && a->T > 0 && a->V > 0, DSTD_ERR_BAD_ARG, "bn_act_backward: bad dims");
   DSTD_REQUIRE(a->y.ptr && a->gout.ptr && a->gy.ptr && a->gamma && a->beta && a->save_mean && a->save_invstd &&
-                   a->ggamma && a->gbeta,
+                   (ph == BN_GLOBAL || (a->ggamma && a->gbeta)),
                DSTD_ERR_BAD_ARG, "bn_act_backward: null tensor");
   DSTD_REQUIRE(!a->gr.ptr || a->r.ptr, DSTD_ERR_BAD_ARG, "bn_act_backward: gr requested without r");
   DSTD_REQUIRE(!a->gr_add.ptr || a->gr.ptr, DSTD_ERR_BAD_ARG, "bn_act_backward: gr_add given without gr");
   DSTD_REQUIRE(a->T * a->V <= BN_MAXJ * BN_THREADS_MAX && a->V <= 32, DSTD_ERR_UNSUPPORTED,
                "bn_act: T*V=%d or V=%d outside the compiled limits", a->T * a->V, a->V);
-  DSTD_REQUIRE(a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws, DSTD_ERR_WORKSPACE,
-               "bn_act_backward: workspace too small");
-  const Switches sw = read_switches();
-  cudaStream_t st = (cudaStream_t)stream;
-  BnBwdP q;
+  DSTD_REQUIRE(ph == BN_GLOBAL || (a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws),
+               DSTD_ERR_WORKSPACE, "bn_act_backward: workspace too small");
   q.N = a->N; q.C = a->C; q.T = a->T; q.V = a->V;
   q.vc_order = a->vc_order; q.training = a->training;
   q.S = bn_act_splits(a->N, sw.bn_samples_per_cta);
@@ -1438,61 +1641,147 @@ extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t
   q.gamma = a->gamma; q.beta = a->beta; q.prelu = a->prelu; q.mask = a->mask;
   q.save_mean = a->save_mean; q.save_invstd = a->save_invstd;
   q.ggamma = a->ggamma; q.gbeta = a->gbeta; q.gprelu = a->prelu ? a->gprelu : nullptr;
-  Arena ar(a->ws, a->ws_bytes);
-  q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
-  q.part_p = ar.take<float>((size_t)q.S * q.C);
-  BnGeom g = bn_geom(q.T, q.V);
+  q.part = q.part_p = nullptr;
+  if (ph != BN_GLOBAL) {
+    Arena ar(a->ws, a->ws_bytes);
+    q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
+    q.part_p = ar.take<float>((size_t)q.S * q.C);
+  }
+  return DSTD_OK;
+}
+
+static BnBwdPlan bn_bwd_plan(const BnBwdP& q, const Switches& sw) {
+  BnBwdPlan p;
   const size_t tv = (size_t)q.T * q.V * sizeof(float);
-  const int nst = (q.r.p && q.prelu) ? 3 : 2;          // staged tensors: gout, y (, r); two pipeline stages
-  {
-    const bool use_r = q.r.p && q.prelu, has_gr = q.gr.p != nullptr, add = q.gadd.p != nullptr;
-    const bool combo = use_r ? has_gr : (!has_gr && !add);     // the instantiations the model uses
-    const bool gr_same = !has_gr || bnf_tfast(q.gr) == bnf_tfast(q.gy);
-    const BnFastPlan fp = (combo && gr_same) ? bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
-                                             : BnFastPlan{false, 0, 0, 0, false};
-    const int u1 = fp.ok ? bnf_pick_u((size_t)fp.ch * tv, nst, fp.big) : 0;
-    const int u2 = fp.ok ? bnf_pick_u((size_t)fp.ch * tv, nst + (add ? 1 : 0), fp.big) : 0;
-    if (u1 && u2) {
-      const dim3 grid(q.C / fp.ch, q.S);
-      int* err = device_error_word();
+  p.g = bn_geom(q.T, q.V);
+  p.use_r = q.r.p && q.prelu;
+  p.add = q.gadd.p != nullptr;
+  p.nst = p.use_r ? 3 : 2;                             // staged tensors: gout, y (, r); two pipeline stages
+  p.nst2 = p.nst + (p.add ? 1 : 0);                    // pass 2 also stages gr_add
+  const bool has_gr = q.gr.p != nullptr;
+  const bool combo = p.use_r ? has_gr : (!has_gr && !p.add);     // the instantiations the model uses
+  const bool gr_same = !has_gr || bnf_tfast(q.gr) == bnf_tfast(q.gy);
+  p.fp = (combo && gr_same) ? bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
+                            : BnFastPlan{false, 0, 0, 0, false};
+  p.u1 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst, p.fp.big) : 0;
+  p.u2 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst2, p.fp.big) : 0;
+  p.ub = bn_pick_u(tv, 2 * p.nst + 1, 4, BN_SMEM_BUDGET);
+  p.ub2 = bn_pick_u(tv, 2 * p.nst2 + 1, p.ub, BN_SMEM_BUDGET);
+  return p;
+}
+
+// pass 1 (per-split partial sums); the fast path's or the generic kernel, as planned
+static int bn_bwd_reduce(const BnBwdP& q, const BnBwdPlan& p, cudaStream_t st) {
+  const size_t tv = (size_t)q.T * q.V * sizeof(float);
+  if (p.fast()) {
+    const dim3 grid(q.C / p.fp.ch, q.S);
+    int* err = device_error_word();
 #define DSTD_K_RED_R(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, true, B_>
 #define DSTD_K_RED(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, false, B_>
-      if (use_r) DSTD_BNF(DSTD_K_RED_R, fp, u1, grid, fp.threads, (size_t)2 * nst * u1 * fp.ch * tv, st, q, fp.ch, err);
-      else DSTD_BNF(DSTD_K_RED, fp, u1, grid, fp.threads, (size_t)2 * nst * u1 * fp.ch * tv, st, q, fp.ch, err);
+    if (p.use_r) DSTD_BNF(DSTD_K_RED_R, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
+    else DSTD_BNF(DSTD_K_RED, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
 #undef DSTD_K_RED_R
 #undef DSTD_K_RED
-      count_launch();
-      DSTD_LAUNCH_CHECK("bnf_bwd_reduce");
-      const int np = (int)(grid.x * grid.y);
-      const size_t smem2 = (size_t)2 * (nst + (add ? 1 : 0)) * u2 * fp.ch * tv;
+    count_launch();
+    DSTD_LAUNCH_CHECK("bnf_bwd_reduce");
+    return DSTD_OK;
+  }
+  size_t sm_red = (size_t)2 * p.nst * p.ub * tv;
+  if (sm_red < 2 * tv) sm_red = 2 * tv;
+  DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, p.g.nj, p.ub, dim3(q.C, q.S), p.g.threads, sm_red, st, q);
+  count_launch();
+  DSTD_LAUNCH_CHECK("bn_bwd_reduce");
+  return DSTD_OK;
+}
+
+// pass 2 (gy, gr; the plain call also the parameter gradients).  all == nullptr: the plain kernels, k1 / k2 from this
+// call's own partial sums; otherwise the synchronised twins, k1 / k2 from the `world` gathered exchange rows.
+static int bn_bwd_apply(const BnBwdP& q, const BnBwdPlan& p, const double* all, int world, cudaStream_t st) {
+  const size_t tv = (size_t)q.T * q.V * sizeof(float);
+  if (p.fast()) {
+    const dim3 grid(q.C / p.fp.ch, q.S);
+    int* err = device_error_word();
+    const int np = (int)(grid.x * grid.y);
+    const size_t smem2 = (size_t)2 * p.nst2 * p.u2 * p.fp.ch * tv;
+    if (!all) {
 #define DSTD_K_APP_RA(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, true, B_>
 #define DSTD_K_APP_R(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, false, B_>
 #define DSTD_K_APP(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, false, false, false, B_>
-      if (use_r && add) DSTD_BNF(DSTD_K_APP_RA, fp, u2, grid, fp.threads, smem2, st, q, fp.ch, np, err);
-      else if (use_r) DSTD_BNF(DSTD_K_APP_R, fp, u2, grid, fp.threads, smem2, st, q, fp.ch, np, err);
-      else DSTD_BNF(DSTD_K_APP, fp, u2, grid, fp.threads, smem2, st, q, fp.ch, np, err);
+      if (p.use_r && p.add) DSTD_BNF(DSTD_K_APP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
+      else if (p.use_r) DSTD_BNF(DSTD_K_APP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
+      else DSTD_BNF(DSTD_K_APP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
 #undef DSTD_K_APP_RA
 #undef DSTD_K_APP_R
 #undef DSTD_K_APP
-      count_launch();
-      DSTD_LAUNCH_CHECK("bnf_bwd_apply");
-      return DSTD_OK;
+    } else {
+#define DSTD_K_SAPP_RA(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, true, B_>
+#define DSTD_K_SAPP_R(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, false, B_>
+#define DSTD_K_SAPP(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, false, false, false, B_>
+      if (p.use_r && p.add) DSTD_BNF(DSTD_K_SAPP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
+      else if (p.use_r) DSTD_BNF(DSTD_K_SAPP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
+      else DSTD_BNF(DSTD_K_SAPP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
+#undef DSTD_K_SAPP_RA
+#undef DSTD_K_SAPP_R
+#undef DSTD_K_SAPP
     }
+    count_launch();
+    DSTD_LAUNCH_CHECK("bnf_bwd_apply");
+    return DSTD_OK;
   }
-  const int ub = bn_pick_u(tv, 2 * nst + 1, 4, BN_SMEM_BUDGET);
-  size_t sm_red = (size_t)2 * nst * ub * tv;
-  if (sm_red < 2 * tv) sm_red = 2 * tv;
-  DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, g.nj, ub, dim3(q.C, q.S), g.threads, sm_red, st, q);
-  count_launch();
-  DSTD_LAUNCH_CHECK("bn_bwd_reduce");
-  const int nst2 = nst + (q.gadd.p ? 1 : 0);           // pass 2 also stages gr_add
-  const int ub2 = bn_pick_u(tv, 2 * nst2 + 1, ub, BN_SMEM_BUDGET);
-  if (q.gadd.p) {
-    DSTD_BN_DISPATCH_U(bn_bwd_apply_add_kernel, g.nj, ub2, dim3(q.C, q.S), g.threads, (size_t)(2 * nst2 + 1) * ub2 * tv, st, q);
+  const size_t sm2 = (size_t)(2 * p.nst2 + 1) * p.ub2 * tv;
+  const dim3 grid(q.C, q.S);
+  if (!all) {
+    if (q.gadd.p) DSTD_BN_DISPATCH_U(bn_bwd_apply_add_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
+    else DSTD_BN_DISPATCH_U(bn_bwd_apply_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
   } else {
-    DSTD_BN_DISPATCH_U(bn_bwd_apply_kernel, g.nj, ub2, dim3(q.C, q.S), g.threads, (size_t)(2 * nst2 + 1) * ub2 * tv, st, q);
+    if (q.gadd.p) DSTD_BN_DISPATCH_U(bn_bwd_apply_add_sync_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
+    else DSTD_BN_DISPATCH_U(bn_bwd_apply_sync_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
   }
   count_launch();
   DSTD_LAUNCH_CHECK("bn_bwd_apply");
   return DSTD_OK;
+}
+
+extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t stream) {
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnBwdP q;
+  int rc = bn_bwd_setup(a, sw, q);
+  if (rc != DSTD_OK) return rc;
+  const BnBwdPlan p = bn_bwd_plan(q, sw);
+  rc = bn_bwd_reduce(q, p, st);
+  if (rc != DSTD_OK) return rc;
+  return bn_bwd_apply(q, p, nullptr, 0, st);
+}
+
+extern "C" int dstd_bn_act_backward_local(const dstd_bn_act_bwd_args* a, double* mine, dstd_stream_t stream) {
+  DSTD_REQUIRE(a && a->training == 1, DSTD_ERR_BAD_ARG, "bn_act_backward_local: needs training = 1");
+  DSTD_REQUIRE(mine, DSTD_ERR_BAD_ARG, "bn_act_backward_local: null exchange buffer");
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnBwdP q;
+  int rc = bn_bwd_setup(a, sw, q, BN_LOCAL);
+  if (rc != DSTD_OK) return rc;
+  const BnBwdPlan p = bn_bwd_plan(q, sw);
+  rc = bn_bwd_reduce(q, p, st);
+  if (rc != DSTD_OK) return rc;
+  // the block size and slope-partial count of the apply kernel the plain call would run: same gprelu summation order
+  const int threads = p.fast() ? p.fp.threads : p.g.threads;
+  const int np = p.fast() ? (q.C / p.fp.ch) * q.S : q.S * q.C;
+  bn_sync_fold_bwd_kernel<<<q.C, threads, 0, st>>>(q, np, mine);
+  count_launch();
+  DSTD_LAUNCH_CHECK("bn_sync_fold_bwd");
+  return DSTD_OK;
+}
+
+extern "C" int dstd_bn_act_backward_global(const dstd_bn_act_bwd_args* a, const double* all, int world,
+                                           dstd_stream_t stream) {
+  DSTD_REQUIRE(a && a->training == 1, DSTD_ERR_BAD_ARG, "bn_act_backward_global: needs training = 1");
+  DSTD_REQUIRE(all && world >= 1, DSTD_ERR_BAD_ARG, "bn_act_backward_global: null exchange buffer or world < 1");
+  const Switches sw = read_switches();
+  cudaStream_t st = (cudaStream_t)stream;
+  BnBwdP q;
+  int rc = bn_bwd_setup(a, sw, q, BN_GLOBAL);
+  if (rc != DSTD_OK) return rc;
+  return bn_bwd_apply(q, bn_bwd_plan(q, sw), all, world, st);
 }

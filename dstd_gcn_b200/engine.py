@@ -14,7 +14,12 @@ with the differences that make it a B200 data-parallel step:
     (NCCL over NVLink), with the 1/world scaling folded into the fused Adam kernel;
   * the loss and its gradient come out of one kernel and the loss stays on the device (no per-step ``.item()`` sync,
     cf. prediction.py:264).
-BatchNorm statistics are per rank (DDP-without-SyncBN semantics).
+BatchNorm statistics are per rank by default (DDP-without-SyncBN semantics).  With ``TrainStep(sync_bn=True)`` and
+more than one rank every training-mode BatchNorm normalises with the statistics of the global batch and updates the
+running statistics from them, as ``torch.nn.SyncBatchNorm`` does (``ops.sync_batch_norm``): each BN call then
+all-gathers 3*C*V fp64 values per rank in its forward and again in its backward, both passes of the step run on one
+stream so every rank issues those collectives in the same order, and the step is not captured into a CUDA graph.  The
+running statistics stay bit-identical across ranks.
 """
 from __future__ import annotations
 
@@ -60,10 +65,13 @@ class TrainStep:
 
     ``inputs``, ``inputs_inv``, ``targets``: raw ``[N, T, 3V]`` fp32 batches already on the device (this rank's shard).
     Returns the (device, 0-dim) loss of this rank's shard.
+
+    ``sync_bn``: synchronised BatchNorm over the ranks of ``process_group`` (see the module docstring); with one rank
+    it changes nothing.
     """
 
     def __init__(self, model, lr=3e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, inverse=True, clip=-1.0,
-                 process_group: Optional[dist.ProcessGroup] = None):
+                 process_group: Optional[dist.ProcessGroup] = None, sync_bn: bool = False):
         self.model = model
         self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
         self.inverse, self.clip = bool(inverse), float(clip)
@@ -73,6 +81,7 @@ class TrainStep:
         self.step_count = 0
         self.pg = process_group
         self.world = dist.get_world_size(process_group) if dist.is_available() and dist.is_initialized() else 1
+        self.sync_bn = bool(sync_bn) and self.world > 1
         dev = self.flat.param.device
         # learning rate and step count also live on the device so that a captured CUDA graph of the step stays valid
         # across steps and StepLR updates (engine/prediction.py:193-196,310)
@@ -127,8 +136,15 @@ class TrainStep:
         v = vc // 3
         scale = 0.5 if self.inverse else 1.0
         self.flat.rebind_grads()
+        if self.sync_bn:
+            # both passes in order on the current stream: every rank issues the BN exchanges in the same order
+            with ops.sync_batch_norm(self.pg):
+                return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, vc, scale)
         if self.inverse and self._overlap and inputs.is_cuda:
             return self._loss_and_grads_two_streams(inputs, inputs_inv, targets, n, t, v, vc, scale)
+        return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, vc, scale)
+
+    def _loss_and_grads_one_stream(self, inputs, inputs_inv, targets, n, t, v, vc, scale):
         out = self.model(inputs.view(n, t, v, 3))
         loss = ops.mpjpe(out.reshape(n, t, vc), targets, scale)
         # the two passes share nothing but the parameters: back-propagate each as soon as its forward is done (the
@@ -172,7 +188,7 @@ class TrainStep:
         return loss.detach() + loss_i
 
     def _finish_step(self):
-        """All-reduce of the flat gradient bucket (the path's only collective), optional clip, fused Adam."""
+        """All-reduce of the flat gradient bucket (the only collective unless sync_bn), optional clip, fused Adam."""
         if self.world > 1:
             dist.all_reduce(self.flat.grad, op=dist.ReduceOp.SUM, group=self.pg)
         gscale = 1.0 / self.world
@@ -221,6 +237,10 @@ class TrainStep:
         """Capture one whole step (both forwards, backward, all-reduce, Adam: several hundred launches) into a CUDA
         graph bound to static input buffers.  The warm-up steps needed before capture are rolled back, so capturing
         does not change the training state.  Later calls with the same batch shape replay the graph."""
+        if self.sync_bn:
+            raise RuntimeError("TrainStep.capture: steps with synchronised BatchNorm (sync_bn=True, world > 1) run "
+                               "eagerly; their BatchNorm exchanges are collectives inside the passes, which are not "
+                               "captured")
         self._static = tuple(t.clone() for t in (inputs, inputs_inv, targets))
         snap = self._snapshot()
         side = torch.cuda.Stream()

@@ -14,6 +14,7 @@ from typing import List, Optional, Sequence, Tuple
 import os
 
 import torch
+import torch.distributed as dist
 from torch import Tensor
 
 from . import _lib
@@ -109,6 +110,60 @@ def bn_act_bwd(y: Tensor, r: Optional[Tensor], gout: Tensor, gamma: Tensor, beta
 def _(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, training, need_gr, gr_add=None):
     return [torch.empty_like(y), torch.empty_like(r) if (r is not None and need_gr) else y.new_empty((0,)),
             torch.empty_like(gamma), torch.empty_like(gamma), y.new_empty((1,) if prelu is not None else (0,))]
+
+
+# synchronised BatchNorm: each direction in two phases around an all-gather of fp64 rows (see sync_batch_norm)
+@torch.library.custom_op("dstd_b200::bn_act_fwd_local", mutates_args=())
+def bn_act_fwd_local(y: Tensor, vc_order: bool) -> Tensor:
+    """This rank's exchange rows (count, mean, M2) [3*C*V] fp64."""
+    return _lib.backend().bn_act_forward_local(y, vc_order)
+
+
+@bn_act_fwd_local.register_fake
+def _(y, vc_order):
+    return y.new_empty((3 * y.shape[1] * y.shape[3],), dtype=torch.float64)
+
+
+@torch.library.custom_op("dstd_b200::bn_act_fwd_global", mutates_args=("running_mean", "running_var", "nbt"))
+def bn_act_fwd_global(y: Tensor, r: Optional[Tensor], gamma: Tensor, beta: Tensor, running_mean: Optional[Tensor],
+                      running_var: Optional[Tensor], nbt: Optional[Tensor], prelu: Optional[Tensor],
+                      mask: Optional[Tensor], all_rows: Tensor, out_order: int, vc_order: bool, eps: float,
+                      momentum: float) -> Tuple[Tensor, Tensor, Tensor]:
+    return _lib.backend().bn_act_forward_global(y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask,
+                                                vc_order, eps, momentum, all_rows, _out_like(y, out_order))
+
+
+@bn_act_fwd_global.register_fake
+def _(y, r, gamma, beta, running_mean, running_var, nbt, prelu, mask, all_rows, out_order, vc_order, eps, momentum):
+    return torch.empty_like(_out_like(y, out_order)), torch.empty_like(gamma), torch.empty_like(gamma)
+
+
+@torch.library.custom_op("dstd_b200::bn_act_bwd_local", mutates_args=())
+def bn_act_bwd_local(y: Tensor, r: Optional[Tensor], gout: Tensor, gamma: Tensor, beta: Tensor,
+                     prelu: Optional[Tensor], mask: Optional[Tensor], save_mean: Tensor, save_invstd: Tensor,
+                     vc_order: bool, need_gr: bool, gr_add: Optional[Tensor] = None) -> List[Tensor]:
+    """[ggamma, gbeta, gprelu|empty, exchange rows (count, sum g', sum g' xhat) [3*C*V] fp64, gy, gr|empty]; gy and
+    gr are uninitialised buffers that bn_act_bwd_global fills."""
+    gg, gb, gp, rows, gy, gr = _lib.backend().bn_act_backward_local(y, r, gout, gamma, beta, prelu, mask, save_mean,
+                                                                    save_invstd, vc_order, need_gr, gr_add)
+    return [gg, gb, gp if gp is not None else y.new_empty((0,)), rows, gy, gr if gr is not None else y.new_empty((0,))]
+
+
+@bn_act_bwd_local.register_fake
+def _(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order, need_gr, gr_add=None):
+    return [torch.empty_like(gamma), torch.empty_like(gamma), y.new_empty((1,) if prelu is not None else (0,)),
+            y.new_empty((3 * gamma.numel(),), dtype=torch.float64), torch.empty_like(y),
+            torch.empty_like(r) if (r is not None and need_gr) else y.new_empty((0,))]
+
+
+@torch.library.custom_op("dstd_b200::bn_act_bwd_global", mutates_args=("gy", "gr"))
+def bn_act_bwd_global(y: Tensor, r: Optional[Tensor], gout: Tensor, gamma: Tensor, beta: Tensor,
+                      prelu: Optional[Tensor], mask: Optional[Tensor], save_mean: Tensor, save_invstd: Tensor,
+                      all_rows: Tensor, vc_order: bool, gy: Tensor, gr: Optional[Tensor],
+                      gr_add: Optional[Tensor] = None) -> None:
+    """Fills gy and gr (+ gr_add) (the buffers bn_act_bwd_local returned; gr None = not wanted)."""
+    _lib.backend().bn_act_backward_global(y, r, gout, gamma, beta, prelu, mask, save_mean, save_invstd, vc_order,
+                                          all_rows, gy, gr, gr_add)
 
 
 @torch.library.custom_op("dstd_b200::chmix_fwd", mutates_args=())
@@ -270,6 +325,7 @@ class defer_bn_updates:
 
     def __enter__(self):
         global _bn_defer
+        _refuse_sync_with_defer(_bn_sync)
         self._prev, _bn_defer = _bn_defer, self.items
         return self.items
 
@@ -304,22 +360,82 @@ def apply_deferred_bn_updates(items):
             torch._foreach_add_(nbts, 1)
 
 
+# When not None: the process group of the innermost active `sync_batch_norm` (a 1-tuple: the group may be None, the
+# default group).
+_bn_sync = None
+
+
+def _sync_world(sync):
+    return dist.get_world_size(sync[0]) if sync is not None and dist.is_available() and dist.is_initialized() else 1
+
+
+def _refuse_sync_with_defer(sync):
+    if _sync_world(sync) > 1:
+        raise RuntimeError("sync_batch_norm cannot be combined with defer_bn_updates: synchronised calls update the "
+                           "running statistics from the global batch inside the call; run the passes of a step in "
+                           "order on one stream instead of deferring the updates")
+
+
+class sync_batch_norm:
+    """Context manager: synchronised BatchNorm over the ranks of ``process_group`` (default: the default group).
+
+    Inside it, every training-mode ``bn_act`` call normalises with the statistics of the batches of all ranks together
+    and updates the running statistics from them, as ``torch.nn.SyncBatchNorm`` does; its backward uses the global
+    batch as well.  Each direction of a call runs a local phase, an all-gather of 3*C*V fp64 values per rank (rank
+    order), and a global phase, so the ranks must issue the same BN calls in the same order.  With a world size of 1,
+    and for eval-mode calls, nothing changes.  Not combinable with ``defer_bn_updates``."""
+
+    def __init__(self, process_group: Optional["dist.ProcessGroup"] = None):
+        self.group = process_group
+
+    def __enter__(self):
+        global _bn_sync
+        sync = (self.group,)
+        if _bn_defer is not None:
+            _refuse_sync_with_defer(sync)
+        self._prev, _bn_sync = _bn_sync, sync
+        return self
+
+    def __exit__(self, *exc):
+        global _bn_sync
+        _bn_sync = self._prev
+        return False
+
+
+def _all_gather_rows(rows, group):
+    """[world * 3*C*V] fp64: every rank's rows in rank order (list form: NCCL and gloo both provide it)."""
+    parts = [torch.empty_like(rows) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(parts, rows, group=group)
+    return torch.cat(parts)
+
+
 class _BnAct(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, y, r, gamma, beta, prelu, running_mean, running_var, nbt, mask, out_order, vc_order, training,
                 eps, momentum, pass_r):
-        deferred = _bn_defer is not None and training and running_mean is not None
-        if deferred:
-            n, _, t, _ = y.shape
-            entry = [running_mean, running_var, nbt, float(momentum), float(eps), float(n * t)]
-            running_mean = running_var = nbt = None
-        out, mean, invstd = torch.ops.dstd_b200.bn_act_fwd(y, r, gamma, beta, running_mean, running_var, nbt, prelu,
-                                                           mask, out_order, vc_order, training, eps, momentum)
-        if deferred:
-            _bn_defer.append(entry + [mean, invstd])
+        sync = _bn_sync if training and _sync_world(_bn_sync) > 1 else None
+        if sync is not None:
+            if _bn_defer is not None:
+                _refuse_sync_with_defer(sync)
+            rows = _all_gather_rows(torch.ops.dstd_b200.bn_act_fwd_local(y, vc_order), sync[0])
+            out, mean, invstd = torch.ops.dstd_b200.bn_act_fwd_global(y, r, gamma, beta, running_mean, running_var,
+                                                                      nbt, prelu, mask, rows, out_order, vc_order,
+                                                                      eps, momentum)
+        else:
+            deferred = _bn_defer is not None and training and running_mean is not None
+            if deferred:
+                n, _, t, _ = y.shape
+                entry = [running_mean, running_var, nbt, float(momentum), float(eps), float(n * t)]
+                running_mean = running_var = nbt = None
+            out, mean, invstd = torch.ops.dstd_b200.bn_act_fwd(y, r, gamma, beta, running_mean, running_var, nbt,
+                                                               prelu, mask, out_order, vc_order, training, eps,
+                                                               momentum)
+            if deferred:
+                _bn_defer.append(entry + [mean, invstd])
         ctx.save_for_backward(y, r, gamma, beta, prelu, mask, mean, invstd)
         ctx.vc_order, ctx.training, ctx.pass_r = vc_order, training, pass_r
+        ctx.sync = sync          # the backward performs its own exchange over the same group
         if pass_r:
             # second output = r itself: whatever else consumes r downstream (the layer skip) sends its gradient back
             # through this node, where the backward kernel adds it to d(pre-activation) in the same pass
@@ -330,9 +446,16 @@ class _BnAct(torch.autograd.Function):
     def backward(ctx, gout, g_thru=None):
         y, r, gamma, beta, prelu, mask, mean, invstd = ctx.saved_tensors
         need_gr = r is not None and ctx.needs_input_grad[1]
-        gy, gr, gg, gb, gp = torch.ops.dstd_b200.bn_act_bwd(y, r, gout, gamma, beta, prelu, mask, mean, invstd,
-                                                            ctx.vc_order, ctx.training, need_gr,
-                                                            g_thru if need_gr else None)
+        gr_add = g_thru if need_gr else None
+        if ctx.sync is not None:
+            gg, gb, gp, rows, gy, gr = torch.ops.dstd_b200.bn_act_bwd_local(y, r, gout, gamma, beta, prelu, mask,
+                                                                            mean, invstd, ctx.vc_order, need_gr, gr_add)
+            rows = _all_gather_rows(rows, ctx.sync[0])
+            torch.ops.dstd_b200.bn_act_bwd_global(y, r, gout, gamma, beta, prelu, mask, mean, invstd, rows,
+                                                  ctx.vc_order, gy, _opt(gr), gr_add)
+        else:
+            gy, gr, gg, gb, gp = torch.ops.dstd_b200.bn_act_bwd(y, r, gout, gamma, beta, prelu, mask, mean, invstd,
+                                                                ctx.vc_order, ctx.training, need_gr, gr_add)
         return (gy, _opt(gr), gg, gb, _opt(gp), None, None, None, None, None, None, None, None, None, None)
 
 

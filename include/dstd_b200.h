@@ -178,6 +178,28 @@ size_t dstd_bn_act_workspace_bytes(int N, int C, int T, int V);
 int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t stream);
 int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t stream);
 
+/* Synchronised BatchNorm (data parallel: statistics over the batches of all ranks).  Each direction of a
+ * training-mode call (training = 1, else DSTD_ERR_BAD_ARG) runs as two phases; between them the caller all-gathers
+ * one fp64 buffer of dstd_bn_sync_buffer_doubles(C, V) = 3*C*V doubles per rank, in rank order, into
+ * `all` = double[world][3][C*V] (BN parameter order c*V+v, or v*C+c when vc_order).
+ *   forward  local : writes `mine` = (count, mean, M2) of this rank's batch; no outputs (of the tensors only y and
+ *                    the workspace are used).
+ *   forward  global: merges the rows in rank order (Chan), writes save_mean / save_invstd, the running statistics
+ *                    (global count, unbiased variance), num_batches_tracked += 1, and `out`.
+ *   backward local : writes this rank's ggamma / gbeta / gprelu (sums over this rank's batch only: they are summed
+ *                    over ranks with the other parameter gradients) and `mine` = (count, sum g', sum g' xhat), where
+ *                    g' is the gradient of the pre-activation and save_mean / save_invstd hold the global statistics.
+ *   backward global: writes gy (and gr) from the rank-order fp64 sums of the gathered rows over the global count.
+ * The global phases use no workspace (ws may be NULL) and the global backward no ggamma / gbeta / gprelu (may be
+ * NULL).  The local backward does not write gy / gr but needs them (their layouts pick the same kernels as the plain
+ * call); the caller passes the buffers the global backward will write.  Identical `all` buffers give bit-identical
+ * results on every rank. */
+size_t dstd_bn_sync_buffer_doubles(int C, int V);
+int dstd_bn_act_forward_local(const dstd_bn_act_fwd_args* a, double* mine, dstd_stream_t stream);
+int dstd_bn_act_forward_global(const dstd_bn_act_fwd_args* a, const double* all, int world, dstd_stream_t stream);
+int dstd_bn_act_backward_local(const dstd_bn_act_bwd_args* a, double* mine, dstd_stream_t stream);
+int dstd_bn_act_backward_global(const dstd_bn_act_bwd_args* a, const double* all, int world, dstd_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------
  * 1x1 channel mix  out[n,o,p,k] = sum_c w[o,c] x[n,c,p,k] + b[o]
  * replaces DSTDGCB.residual[0] (nn.Conv2d 1x1, model/dstdgcn.py:118; nn.Linear in fast :183-186)
