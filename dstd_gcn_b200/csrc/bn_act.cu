@@ -10,6 +10,7 @@
 // Statistics use shifted sums (shift = y[0,c,0,v]) accumulated in fp32 per thread and combined in fp64, so the
 // E[x^2]-E[x]^2 cancellation does not bite on millimetre-scale poses.
 #include <initializer_list>
+#include <type_traits>
 
 #include "kernels.cuh"
 #include "umma.cuh"
@@ -18,6 +19,12 @@ namespace dstd {
 
 constexpr int BN_THREADS_MAX = 512;
 constexpr int BN_MAXJ = 8;       // positions per thread  -> T*V <= 4096
+// Joints.  The per-(c, v) shared tables of the kernels are sized for one warp of joints (V <= 32); the `_wide_`
+// instantiations size them for BN_MAXV and run V = 33 .. BN_MAXV, so the V <= 32 kernels are those of a 32-joint
+// build.  Every block of the generic kernels has at least min(T*V, 257) threads and the fast plan gives the wide
+// kernels at least V, so "one thread per v" loops need no stride.
+constexpr int BN_MAXV = 128;
+__host__ __device__ constexpr int bn_table_v(bool wide) { return wide ? BN_MAXV : 32; }
 // samples per pipeline stage: the largest of 4/2/1 not above `cap` whose `planes_per_u` staged planes fit `budget`
 static int bn_pick_u(size_t plane_bytes, int planes_per_u, int cap, size_t budget) {
   int u = 4;
@@ -230,7 +237,7 @@ __device__ __forceinline__ void stage_async_b(const Pos2<NJ>& ps, const View4& w
 
 // ------------------------------------------------------------------------------------------ forward: statistics
 template <int NJ>
-__global__ void __launch_bounds__(BN_THREADS_MAX) bn_stats_kernel(BnFwdP q) {
+__device__ __forceinline__ void bn_stats_body(const BnFwdP& q) {
   extern __shared__ float sh[];   // [2][T*V]
   constexpr int SU = 8;
   const int c = blockIdx.x, s = blockIdx.y, T = q.T, V = q.V, TV = T * V;
@@ -319,6 +326,15 @@ __global__ void __launch_bounds__(BN_THREADS_MAX) bn_stats_kernel(BnFwdP q) {
   }
 }
 
+template <int NJ>
+__global__ void __launch_bounds__(BN_THREADS_MAX) bn_stats_kernel(BnFwdP q) {
+  bn_stats_body<NJ>(q);
+}
+// planes of 4097 .. 8192 positions, whose apply and backward passes run the BIG fast kernels (V > 32 only)
+__global__ void __launch_bounds__(2 * BN_THREADS_MAX) bn_stats_big_kernel(BnFwdP q) {
+  bn_stats_body<BN_MAXJ>(q);
+}
+
 // Sum the per-split partial pairs of channel c for every v, in a fixed order (so that every CTA of the channel gets
 // bit-identical totals): 8 lanes per v, strided over the splits, combined with a butterfly.  Called by all threads;
 // the totals land in tot[v][0..1].  This replaces a separate "finalize" launch between the reduction and the apply
@@ -387,9 +403,10 @@ __device__ __forceinline__ void bn_apply_consume(const BnFwdP& q, const float* s
   }
 }
 
-template <int NJ, int U>
-__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_apply_kernel(BnFwdP q) {
+template <int NJ, int U, bool WIDE>
+__device__ __forceinline__ void bn_apply_body(const BnFwdP& q) {
   extern __shared__ float sh[];   // [2 stages][nst = 1 (y) or 2 (y, r)][U][T*V]
+  constexpr int VW = bn_table_v(WIDE);
   const int c = blockIdx.x, s = blockIdx.y, T = q.T, V = q.V, TV = T * V;
   const int n0 = (int)((long long)q.N * s / q.S), n1 = (int)((long long)q.N * (s + 1) / q.S), cnt = n1 - n0;
   const bool has_r = q.r.p != nullptr;
@@ -412,8 +429,8 @@ __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_apply_kernel(BnFwdP q) {
   };
   if (iters > 0) issue(0);
   cp_async_commit();
-  __shared__ double tot[32][2];
-  __shared__ float st_mean[32], st_is[32];
+  __shared__ double tot[VW][2];
+  __shared__ float st_mean[VW], st_is[VW];
   if (q.training) {   // batch statistics from the split partials; the s == 0 CTA of the channel publishes them
     sum_partials(q.part, q.S, q.C, c, V, tot);
     __syncthreads();
@@ -480,6 +497,15 @@ __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_apply_kernel(BnFwdP q) {
     else bn_apply_consume<NJ, U, false, false>(q, stage, op, sy, sr, me, c, n, left, sm, sc, sf, slope, has_r);
     __syncthreads();   // the buffer is refilled by the prefetch of the next iteration
   }
+}
+
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_apply_kernel(BnFwdP q) {
+  bn_apply_body<NJ, U, false>(q);
+}
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_apply_wide_kernel(BnFwdP q) {
+  bn_apply_body<NJ, U, true>(q);
 }
 
 // ------------------------------------------------------------------------------------------ backward
@@ -706,9 +732,10 @@ __device__ __forceinline__ void sync_bwd_totals(const double* all, int world, in
 
 // SYNC: the global phase of the synchronised backward.  k1 / k2 come from the gathered rows (`all`, `world`) instead
 // of the split partials, and the parameter gradients are not written (the local phase wrote this rank's share).
-template <int NJ, int U, bool ADD, bool SYNC>
+template <int NJ, int U, bool ADD, bool SYNC, bool WIDE>
 __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double* all, int world) {
   extern __shared__ float sh[];   // [2 stages][nst = 2 (gout, y), + r, + gr_add][U][T*V], then [U][T*V] for gr
+  constexpr int VW = bn_table_v(WIDE);
   const int c = blockIdx.x, s = blockIdx.y, T = q.T, V = q.V, TV = T * V;
   const int n0 = (int)((long long)q.N * s / q.S), n1 = (int)((long long)q.N * (s + 1) / q.S), cnt = n1 - n0;
   const bool has_prelu = q.prelu != nullptr;
@@ -743,7 +770,7 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double*
   if (iters > 0) issue(0);
   cp_async_commit();
   // sums of pass 1 over the splits; the s == 0 CTA of the channel publishes the parameter gradients
-  __shared__ double tot[32][2];
+  __shared__ double tot[VW][2];
   __shared__ float red[32];
   if (SYNC) {
     sync_bwd_totals(all, world, q.C, V, c, q.vc_order, tot);
@@ -856,22 +883,40 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double*
 
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_kernel(BnBwdP q) {
-  bn_bwd_apply_body<NJ, U, false, false>(q, nullptr, 0);
+  bn_bwd_apply_body<NJ, U, false, false, false>(q, nullptr, 0);
 }
 // same with a fourth staged tensor, gr_add, summed into gr (separate instantiation: the plain kernel sits at the
 // 64-register cap and pays ~13 % for the extra slots)
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_kernel(BnBwdP q) {
-  bn_bwd_apply_body<NJ, U, true, false>(q, nullptr, 0);
+  bn_bwd_apply_body<NJ, U, true, false, false>(q, nullptr, 0);
 }
 // the global phase of the synchronised backward (k1, k2 from the gathered rows)
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_sync_kernel(BnBwdP q, const double* all, int world) {
-  bn_bwd_apply_body<NJ, U, false, true>(q, all, world);
+  bn_bwd_apply_body<NJ, U, false, true, false>(q, all, world);
 }
 template <int NJ, int U>
 __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_sync_kernel(BnBwdP q, const double* all, int world) {
-  bn_bwd_apply_body<NJ, U, true, true>(q, all, world);
+  bn_bwd_apply_body<NJ, U, true, true, false>(q, all, world);
+}
+// V = 33 .. BN_MAXV
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_wide_kernel(BnBwdP q) {
+  bn_bwd_apply_body<NJ, U, false, false, true>(q, nullptr, 0);
+}
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_wide_kernel(BnBwdP q) {
+  bn_bwd_apply_body<NJ, U, true, false, true>(q, nullptr, 0);
+}
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_sync_wide_kernel(BnBwdP q, const double* all, int world) {
+  bn_bwd_apply_body<NJ, U, false, true, true>(q, all, world);
+}
+template <int NJ, int U>
+__global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_apply_add_sync_wide_kernel(BnBwdP q, const double* all,
+                                                                                       int world) {
+  bn_bwd_apply_body<NJ, U, true, true, true>(q, all, world);
 }
 
 // ================================================================================================ fast path
@@ -890,7 +935,14 @@ constexpr int BNF_MAXCH = 4;
 // BIG instantiations: slabs of 4097 .. 8192 positions (the stress configuration: two channels x T*V = 2750) with up to
 // 1024 threads, one CTA per SM, 13-bit slots (two channels at most, so the constant index still fits the word)
 constexpr int BNF_THREADS_BIG = 1024;
-template <bool BIG> struct BnfBits { static constexpr int SB = BIG ? 13 : 12; static constexpr uint32_t SM = (1u << SB) - 1u; };
+// Position word: the slots in the low 2 SB bits, the constant-table index ch * VW + v from bit KS.  The wide tables
+// (VW = BN_MAXV rows per channel) need a 64-bit word.
+template <bool BIG, bool WIDE = false> struct BnfBits {
+  static constexpr int SB = BIG ? 13 : 12;
+  static constexpr uint32_t SM = (1u << SB) - 1u;
+  static constexpr int VW = bn_table_v(WIDE), KS = WIDE ? 32 : 2 * SB;
+  using Pk = typename std::conditional<WIDE, unsigned long long, uint32_t>::type;
+};
 
 __device__ __forceinline__ void bnf_decode(bool tfast, int j, int T, int V, int TV, int& ch, int& t, int& v) {
   ch = j / TV;
@@ -908,17 +960,19 @@ __device__ __forceinline__ void bnf_timeout(int* err) {
 }
 
 // ---- forward apply: positions in out's memory order
-template <int NJ, int U, bool HAS_R, bool FULL, bool BIG>
-__device__ __forceinline__ void bnf_apply_consume(const float* st, const float4* ctab, const uint32_t (&pk)[NJ], float* ob,
+template <int NJ, int U, bool HAS_R, bool FULL, bool BIG, bool WIDE>
+__device__ __forceinline__ void bnf_apply_consume(const float* st, const float4* ctab,
+                                                  const typename BnfBits<BIG, WIDE>::Pk (&pk)[NJ], float* ob,
                                                   long long osn, int CHTV, int left, float slope) {
 #pragma unroll
   for (int i = 0; i < NJ; ++i) {
     if ((int)(threadIdx.x + i * blockDim.x) < CHTV) {
-      constexpr int SB = BnfBits<BIG>::SB;
-      constexpr uint32_t SM = BnfBits<BIG>::SM;
-      const float4 k = ctab[pk[i] >> (2 * SB)];
-      const float* py = st + (pk[i] & SM);
-      const float* pr = st + U * CHTV + ((pk[i] >> SB) & SM);
+      constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
+      constexpr uint32_t SM = BnfBits<BIG, WIDE>::SM;
+      const uint32_t lo = (uint32_t)pk[i];
+      const float4 k = ctab[(uint32_t)(pk[i] >> KS)];
+      const float* py = st + (lo & SM);
+      const float* pr = st + U * CHTV + ((lo >> SB) & SM);
       float* o = ob + i * blockDim.x;
 #pragma unroll
       for (int u = 0; u < U; ++u) {
@@ -932,11 +986,12 @@ __device__ __forceinline__ void bnf_apply_consume(const float* st, const float4*
   }
 }
 
-template <int NJ, int U, bool HAS_R, bool BIG>
-__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_apply_kernel(BnFwdP q, int CH, int* err) {
+template <int NJ, int U, bool HAS_R, bool BIG, bool WIDE>
+__device__ __forceinline__ void bnf_apply_body(const BnFwdP& q, int CH, int* err) {
+  constexpr int VW = BnfBits<BIG, WIDE>::VW;
   extern __shared__ __align__(16) float sh[];   // [2 stages][y (, r)][U][CH * T*V]
-  __shared__ __align__(16) float4 ctab[BNF_MAXCH * 32];     // per (ch, v): mean, gamma * invstd, beta
-  __shared__ double tot[32][2];
+  __shared__ __align__(16) float4 ctab[BNF_MAXCH * VW];     // per (ch, v): mean, gamma * invstd, beta
+  __shared__ double tot[VW][2];
   __shared__ __align__(8) uint64_t mbar[2];
   const int c0 = blockIdx.x * CH, s = blockIdx.y, T = q.T, V = q.V, TV = T * V, CHTV = CH * TV;
   const int n0 = (int)((long long)q.N * s / gridDim.y), n1 = (int)((long long)q.N * (s + 1) / gridDim.y), cnt = n1 - n0;
@@ -977,7 +1032,7 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
         const double mean = shift + dm;
         const float fm = (float)mean, fi = (float)(1.0 / sqrt(var + (double)q.eps));
         const int pi = bn_pidx(c, v, q.C, V, q.vc_order);
-        ctab[ch * 32 + v] = make_float4(fm, __ldg(q.gamma + pi) * fi, __ldg(q.beta + pi), 0.f);
+        ctab[ch * VW + v] = make_float4(fm, __ldg(q.gamma + pi) * fi, __ldg(q.beta + pi), 0.f);
         if (s == 0) {
           q.save_mean[pi] = fm;
           q.save_invstd[pi] = fi;
@@ -992,15 +1047,21 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
       __syncthreads();
     }
   } else {
-    if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
+    if (WIDE) {
+      for (int ix = threadIdx.x; ix < CH * VW; ix += blockDim.x)
+        if (ix % VW < V) {
+          const int pi = bn_pidx(c0 + ix / VW, ix % VW, q.C, V, q.vc_order);
+          ctab[ix] = make_float4(q.save_mean[pi], __ldg(q.gamma + pi) * q.save_invstd[pi], __ldg(q.beta + pi), 0.f);
+        }
+    } else if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
       const int pi = bn_pidx(c0 + (threadIdx.x >> 5), threadIdx.x & 31, q.C, V, q.vc_order);
       ctab[threadIdx.x] = make_float4(q.save_mean[pi], __ldg(q.gamma + pi) * q.save_invstd[pi], __ldg(q.beta + pi), 0.f);
     }
     __syncthreads();
   }
-  uint32_t pk[NJ];   // slot in y's slab | slot in r's slab << SB | (ch * 32 + v) << 2 SB   (valid iff j < CHTV)
+  typename BnfBits<BIG, WIDE>::Pk pk[NJ];   // slot in y's slab | slot in r's slab << SB | (ch * VW + v) << KS   (valid iff j < CHTV)
   {
-    constexpr int SB = BnfBits<BIG>::SB;
+    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_o = t_fastest(q.out), tf_y = t_fastest(q.y), tf_r = HAS_R && t_fastest(q.r);
 #pragma unroll
     for (int i = 0; i < NJ; ++i) {
@@ -1010,7 +1071,7 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
         int ch, t, v;
         bnf_decode(tf_o, j, T, V, TV, ch, t, v);
         pk[i] = (uint32_t)(ch * TV + slot_of(tf_y, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) << SB) |
-                ((uint32_t)(ch * 32 + v) << (2 * SB));
+                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
       }
     }
   }
@@ -1021,27 +1082,38 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
     if (!umma::mbar_wait(&mbar[it & 1], (uint32_t)(it >> 1) & 1u)) bnf_timeout(err);
     const float* st = sh + (it & 1) * stage_f;
     const int left = n1 - (n0 + it * U);
-    if (left >= U) bnf_apply_consume<NJ, U, HAS_R, true, BIG>(st, ctab, pk, ob, osn, CHTV, left, slope);
-    else bnf_apply_consume<NJ, U, HAS_R, false, BIG>(st, ctab, pk, ob, osn, CHTV, left, slope);
+    if (left >= U) bnf_apply_consume<NJ, U, HAS_R, true, BIG, WIDE>(st, ctab, pk, ob, osn, CHTV, left, slope);
+    else bnf_apply_consume<NJ, U, HAS_R, false, BIG, WIDE>(st, ctab, pk, ob, osn, CHTV, left, slope);
     ob += U * osn;
     __syncthreads();
   }
 }
 
+template <int NJ, int U, bool HAS_R, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_apply_kernel(BnFwdP q, int CH, int* err) {
+  bnf_apply_body<NJ, U, HAS_R, BIG, false>(q, CH, err);
+}
+template <int NJ, int U, bool HAS_R, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_apply_wide_kernel(BnFwdP q, int CH, int* err) {
+  bnf_apply_body<NJ, U, HAS_R, BIG, true>(q, CH, err);
+}
+
 // ---- backward pass 1: positions in y's memory order
-template <int NJ, int U, bool USE_R, bool FULL, bool BIG>
-__device__ __forceinline__ void bnf_reduce_consume(const float* st, const float4* ctab, const uint32_t (&pk)[NJ], int CHTV,
+template <int NJ, int U, bool USE_R, bool FULL, bool BIG, bool WIDE>
+__device__ __forceinline__ void bnf_reduce_consume(const float* st, const float4* ctab,
+                                                   const typename BnfBits<BIG, WIDE>::Pk (&pk)[NJ], int CHTV,
                                                    int left, float slope, bool has_prelu, float (&a1)[NJ],
                                                    float (&a2)[NJ], float& gsl) {
 #pragma unroll
   for (int i = 0; i < NJ; ++i) {
     if ((int)(threadIdx.x + i * blockDim.x) < CHTV) {
-      constexpr int SB = BnfBits<BIG>::SB;
-      constexpr uint32_t SM = BnfBits<BIG>::SM;
-      const float4 k = ctab[pk[i] >> (2 * SB)];
-      const float* pg = st + (pk[i] & SM);
+      constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
+      constexpr uint32_t SM = BnfBits<BIG, WIDE>::SM;
+      const uint32_t lo = (uint32_t)pk[i];
+      const float4 k = ctab[(uint32_t)(pk[i] >> KS)];
+      const float* pg = st + (lo & SM);
       const float* py = st + U * CHTV + threadIdx.x + i * blockDim.x;
-      const float* pr = st + 2 * U * CHTV + ((pk[i] >> SB) & SM);
+      const float* pr = st + 2 * U * CHTV + ((lo >> SB) & SM);
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         if (FULL || u < left) {
@@ -1057,10 +1129,11 @@ __device__ __forceinline__ void bnf_reduce_consume(const float* st, const float4
   }
 }
 
-template <int NJ, int U, bool USE_R, bool BIG>
-__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_reduce_kernel(BnBwdP q, int CH, int* err) {
+template <int NJ, int U, bool USE_R, bool BIG, bool WIDE>
+__device__ __forceinline__ void bnf_bwd_reduce_body(const BnBwdP& q, int CH, int* err) {
+  constexpr int VW = BnfBits<BIG, WIDE>::VW;
   extern __shared__ __align__(16) float sh[];   // [2 stages][gout, y (, r)][U][CH * T*V]
-  __shared__ __align__(16) float4 ctab[BNF_MAXCH * 32];     // per (ch, v): mean, invstd, gamma, beta
+  __shared__ __align__(16) float4 ctab[BNF_MAXCH * VW];     // per (ch, v): mean, invstd, gamma, beta
   __shared__ float red[32];
   __shared__ __align__(8) uint64_t mbar[2];
   const int c0 = blockIdx.x * CH, s = blockIdx.y, T = q.T, V = q.V, TV = T * V, CHTV = CH * TV;
@@ -1074,7 +1147,13 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
     umma::mbar_init(&mbar[1], 1);
     umma::mbar_init_fence();
   }
-  if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
+  if (WIDE) {
+    for (int ix = threadIdx.x; ix < CH * VW; ix += blockDim.x)
+      if (ix % VW < V) {
+        const int pi = bn_pidx(c0 + ix / VW, ix % VW, q.C, V, q.vc_order);
+        ctab[ix] = make_float4(__ldg(q.save_mean + pi), __ldg(q.save_invstd + pi), __ldg(q.gamma + pi), __ldg(q.beta + pi));
+      }
+  } else if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
     const int pi = bn_pidx(c0 + (threadIdx.x >> 5), threadIdx.x & 31, q.C, V, q.vc_order);
     ctab[threadIdx.x] = make_float4(__ldg(q.save_mean + pi), __ldg(q.save_invstd + pi), __ldg(q.gamma + pi), __ldg(q.beta + pi));
   }
@@ -1094,11 +1173,11 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
     }
   };
   if (threadIdx.x == 0 && iters > 0) issue(0);
-  uint32_t pk[NJ];   // slot in gout's slab | slot in r's slab << SB | (ch * 32 + v) << 2 SB;  y is read at j itself
+  typename BnfBits<BIG, WIDE>::Pk pk[NJ];   // slot in gout's slab | slot in r's slab << SB | (ch * VW + v) << KS;  y is read at j itself
   float a1[NJ], a2[NJ], gsl = 0.f;
   const bool tf_y = t_fastest(q.y);
   {
-    constexpr int SB = BnfBits<BIG>::SB;
+    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_g = t_fastest(q.gout), tf_r = USE_R && t_fastest(q.r);
 #pragma unroll
     for (int i = 0; i < NJ; ++i) {
@@ -1109,7 +1188,7 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
         int ch, t, v;
         bnf_decode(tf_y, j, T, V, TV, ch, t, v);
         pk[i] = (uint32_t)(ch * TV + slot_of(tf_g, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) << SB) |
-                ((uint32_t)(ch * 32 + v) << (2 * SB));
+                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
       }
     }
   }
@@ -1118,8 +1197,8 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
     if (!umma::mbar_wait(&mbar[it & 1], (uint32_t)(it >> 1) & 1u)) bnf_timeout(err);
     const float* st = sh + (it & 1) * stage_f;
     const int left = n1 - (n0 + it * U);
-    if (left >= U) bnf_reduce_consume<NJ, U, USE_R, true, BIG>(st, ctab, pk, CHTV, left, slope, has_prelu, a1, a2, gsl);
-    else bnf_reduce_consume<NJ, U, USE_R, false, BIG>(st, ctab, pk, CHTV, left, slope, has_prelu, a1, a2, gsl);
+    if (left >= U) bnf_reduce_consume<NJ, U, USE_R, true, BIG, WIDE>(st, ctab, pk, CHTV, left, slope, has_prelu, a1, a2, gsl);
+    else bnf_reduce_consume<NJ, U, USE_R, false, BIG, WIDE>(st, ctab, pk, CHTV, left, slope, has_prelu, a1, a2, gsl);
     __syncthreads();
   }
   // per-(c,v) totals: positions to their logical slot, then one thread per (ch, v) sums over t in order (fp64)
@@ -1149,21 +1228,32 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
   if (threadIdx.x == 0) q.part_p[(long long)s * gridDim.x + blockIdx.x] = totp;
 }
 
+template <int NJ, int U, bool USE_R, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_reduce_kernel(BnBwdP q, int CH, int* err) {
+  bnf_bwd_reduce_body<NJ, U, USE_R, BIG, false>(q, CH, err);
+}
+template <int NJ, int U, bool USE_R, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_reduce_wide_kernel(BnBwdP q, int CH, int* err) {
+  bnf_bwd_reduce_body<NJ, U, USE_R, BIG, true>(q, CH, err);
+}
+
 // ---- backward pass 2: positions in gy's memory order; gr (same order as gy) is stored straight from registers
-template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool FULL, bool BIG>
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool FULL, bool BIG, bool WIDE>
 __device__ __forceinline__ void bnf_bwd_apply_consume(const float* st, const float4* ctab, const float4* ctab2,
-                                                      const uint32_t (&pk)[NJ], const uint32_t (&pk2)[NJ], float* gyb, float* grb,
+                                                      const typename BnfBits<BIG, WIDE>::Pk (&pk)[NJ],
+                                                      const uint32_t (&pk2)[NJ], float* gyb, float* grb,
                                                       long long gysn, long long grsn, int CHTV, int left, float slope,
                                                       bool has_prelu) {
   constexpr int ADD_REGION = USE_R ? 3 : 2;
 #pragma unroll
   for (int i = 0; i < NJ; ++i) {
     if ((int)(threadIdx.x + i * blockDim.x) < CHTV) {
-      constexpr int SB = BnfBits<BIG>::SB;
-      constexpr uint32_t SM = BnfBits<BIG>::SM;
-      const float4 k = ctab[pk[i] >> (2 * SB)], k2 = ctab2[pk[i] >> (2 * SB)];
-      const float* pg = st + (pk[i] & SM);
-      const float* py = st + U * CHTV + ((pk[i] >> SB) & SM);
+      constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
+      constexpr uint32_t SM = BnfBits<BIG, WIDE>::SM;
+      const uint32_t lo = (uint32_t)pk[i];
+      const float4 k = ctab[(uint32_t)(pk[i] >> KS)], k2 = ctab2[(uint32_t)(pk[i] >> KS)];
+      const float* pg = st + (lo & SM);
+      const float* py = st + U * CHTV + ((lo >> SB) & SM);
       const float* pr = st + 2 * U * CHTV + (pk2[i] & SM);
       const float* pa = st + ADD_REGION * U * CHTV + ((pk2[i] >> SB) & SM);
       float* o = gyb + i * blockDim.x;
@@ -1183,12 +1273,13 @@ __device__ __forceinline__ void bnf_bwd_apply_consume(const float* st, const flo
 }
 
 // SYNC: global phase of the synchronised backward, as in bn_bwd_apply_body
-template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG, bool SYNC>
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG, bool SYNC, bool WIDE>
 __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int NP, int* err, const double* all, int world) {
+  constexpr int VW = BnfBits<BIG, WIDE>::VW;
   extern __shared__ __align__(16) float sh[];   // [2 stages][gout, y (, r) (, gr_add)][U][CH * T*V]
-  __shared__ __align__(16) float4 ctab[BNF_MAXCH * 32];     // mean, invstd, gamma, beta
-  __shared__ __align__(16) float4 ctab2[BNF_MAXCH * 32];    // gamma * invstd, k1, k2
-  __shared__ double tot[32][2];
+  __shared__ __align__(16) float4 ctab[BNF_MAXCH * VW];     // mean, invstd, gamma, beta
+  __shared__ __align__(16) float4 ctab2[BNF_MAXCH * VW];    // gamma * invstd, k1, k2
+  __shared__ double tot[VW][2];
   __shared__ float red[32];
   __shared__ __align__(8) uint64_t mbar[2];
   const int c0 = blockIdx.x * CH, s = blockIdx.y, T = q.T, V = q.V, TV = T * V, CHTV = CH * TV;
@@ -1238,11 +1329,11 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
     if (threadIdx.x < V) {
       const int v = threadIdx.x, pi = bn_pidx(c, v, q.C, V, q.vc_order);
       const float mu = __ldg(q.save_mean + pi), is = __ldg(q.save_invstd + pi), g = __ldg(q.gamma + pi);
-      ctab[ch * 32 + v] = make_float4(mu, is, g, __ldg(q.beta + pi));
+      ctab[ch * VW + v] = make_float4(mu, is, g, __ldg(q.beta + pi));
       if (SYNC) {
-        ctab2[ch * 32 + v] = make_float4(g * is, (float)tot[v][0], (float)tot[v][1], 0.f);
+        ctab2[ch * VW + v] = make_float4(g * is, (float)tot[v][0], (float)tot[v][1], 0.f);
       } else {
-        ctab2[ch * 32 + v] = make_float4(g * is, q.training ? (float)tot[v][0] * icnt : 0.f,
+        ctab2[ch * VW + v] = make_float4(g * is, q.training ? (float)tot[v][0] * icnt : 0.f,
                                          q.training ? (float)tot[v][1] * icnt : 0.f, 0.f);
         if (s == 0) {
           q.gbeta[pi] = (float)tot[v][0];
@@ -1252,9 +1343,10 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
     }
     __syncthreads();
   }
-  uint32_t pk[NJ], pk2[NJ];   // gout slot | y slot << SB | (ch*32+v) << 2 SB;   r slot | gr_add slot << SB
+  typename BnfBits<BIG, WIDE>::Pk pk[NJ];   // gout slot | y slot << SB | (ch * VW + v) << KS
+  uint32_t pk2[NJ];                         // r slot | gr_add slot << SB
   {
-    constexpr int SB = BnfBits<BIG>::SB;
+    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_o = t_fastest(q.gy), tf_g = t_fastest(q.gout), tf_y = t_fastest(q.y), tf_r = USE_R && t_fastest(q.r),
                tf_a = ADD && t_fastest(q.gadd);
 #pragma unroll
@@ -1266,7 +1358,7 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
         int ch, t, v;
         bnf_decode(tf_o, j, T, V, TV, ch, t, v);
         pk[i] = (uint32_t)(ch * TV + slot_of(tf_g, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_y, t, v, T, V)) << SB) |
-                ((uint32_t)(ch * 32 + v) << (2 * SB));
+                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
         pk2[i] = (uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_a, t, v, T, V)) << SB);
       }
     }
@@ -1280,9 +1372,9 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
     const float* st = sh + (it & 1) * stage_f;
     const int left = n1 - (n0 + it * U);
     if (left >= U)
-      bnf_bwd_apply_consume<NJ, U, USE_R, HAS_GR, ADD, true, BIG>(st, ctab, ctab2, pk, pk2, gyb, grb, gysn, grsn, CHTV, left, slope, has_prelu);
+      bnf_bwd_apply_consume<NJ, U, USE_R, HAS_GR, ADD, true, BIG, WIDE>(st, ctab, ctab2, pk, pk2, gyb, grb, gysn, grsn, CHTV, left, slope, has_prelu);
     else
-      bnf_bwd_apply_consume<NJ, U, USE_R, HAS_GR, ADD, false, BIG>(st, ctab, ctab2, pk, pk2, gyb, grb, gysn, grsn, CHTV, left, slope, has_prelu);
+      bnf_bwd_apply_consume<NJ, U, USE_R, HAS_GR, ADD, false, BIG, WIDE>(st, ctab, ctab2, pk, pk2, gyb, grb, gysn, grsn, CHTV, left, slope, has_prelu);
     gyb += U * gysn;
     if (HAS_GR) grb += U * grsn;
     __syncthreads();
@@ -1291,11 +1383,19 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
 
 template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
 __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_kernel(BnBwdP q, int CH, int NP, int* err) {
-  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, false>(q, CH, NP, err, nullptr, 0);
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, false, false>(q, CH, NP, err, nullptr, 0);
 }
 template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
 __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_sync_kernel(BnBwdP q, int CH, int* err, const double* all, int world) {
-  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, true>(q, CH, 0, err, all, world);
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, true, false>(q, CH, 0, err, all, world);
+}
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_wide_kernel(BnBwdP q, int CH, int NP, int* err) {
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, false, true>(q, CH, NP, err, nullptr, 0);
+}
+template <int NJ, int U, bool USE_R, bool HAS_GR, bool ADD, bool BIG>
+__global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 1 : 2) bnf_bwd_apply_sync_wide_kernel(BnBwdP q, int CH, int* err, const double* all, int world) {
+  bnf_bwd_apply_body<NJ, U, USE_R, HAS_GR, ADD, BIG, true, true>(q, CH, 0, err, all, world);
 }
 
 // ---- synchronised BatchNorm: fold and merge kernels around the exchange of per-rank rows
@@ -1303,8 +1403,9 @@ __global__ void __launch_bounds__(BIG ? BNF_THREADS_BIG : BN_THREADS_MAX, BIG ? 
 // (count, sum g', sum g' xhat) in the backward.  One CTA per channel (fold), one thread per parameter index (merge).
 
 // forward, local phase: this rank's split partials (shifted sums) -> (count, mean_r, M2_r)
-__global__ void bn_sync_fold_fwd_kernel(BnFwdP q, double* mine) {
-  __shared__ double tot[32][2];
+template <bool WIDE>
+__device__ __forceinline__ void bn_sync_fold_fwd_body(const BnFwdP& q, double* mine) {
+  __shared__ double tot[bn_table_v(WIDE)][2];
   const int c = blockIdx.x, V = q.V;
   const long long cv = (long long)q.C * V;
   sum_partials(q.part, q.S, q.C, c, V, tot);
@@ -1321,6 +1422,8 @@ __global__ void bn_sync_fold_fwd_kernel(BnFwdP q, double* mine) {
     mine[2 * cv + pi] = m2;
   }
 }
+__global__ void bn_sync_fold_fwd_kernel(BnFwdP q, double* mine) { bn_sync_fold_fwd_body<false>(q, mine); }
+__global__ void bn_sync_fold_fwd_wide_kernel(BnFwdP q, double* mine) { bn_sync_fold_fwd_body<true>(q, mine); }
 
 // forward, global phase: Chan's merge of the `world` rows in rank order -> save_mean / save_invstd, running statistics
 // (global count, unbiased variance), num_batches_tracked
@@ -1355,8 +1458,9 @@ __global__ void bn_sync_merge_fwd_kernel(BnFwdP q, const double* all, int world)
 // backward, local phase: this rank's parameter gradients (the sums and the order of bn_bwd_apply / bnf_bwd_apply:
 // launched with the block size of the apply kernel the plain call would run, over its NP slope partials) and its
 // exchange rows (count, sum g', sum g' xhat)
-__global__ void bn_sync_fold_bwd_kernel(BnBwdP q, int NP, double* mine) {
-  __shared__ double tot[32][2];
+template <bool WIDE>
+__device__ __forceinline__ void bn_sync_fold_bwd_body(const BnBwdP& q, int NP, double* mine) {
+  __shared__ double tot[bn_table_v(WIDE)][2];
   __shared__ float red[32];
   const int c = blockIdx.x, V = q.V;
   const long long cv = (long long)q.C * V;
@@ -1377,12 +1481,15 @@ __global__ void bn_sync_fold_bwd_kernel(BnBwdP q, int NP, double* mine) {
     mine[2 * cv + pi] = tot[v][1];
   }
 }
+__global__ void bn_sync_fold_bwd_kernel(BnBwdP q, int NP, double* mine) { bn_sync_fold_bwd_body<false>(q, NP, mine); }
+__global__ void bn_sync_fold_bwd_wide_kernel(BnBwdP q, int NP, double* mine) { bn_sync_fold_bwd_body<true>(q, NP, mine); }
 
 // host side of the fast path
 struct BnFastPlan {
   bool ok;
   int ch, nj, threads;
   bool big;     // slab of 4097 .. 8192 positions: BIG instantiations (<= 1024 threads, one CTA per SM)
+  bool wide;    // V > 32: the _wide_ instantiations
 };
 static bool bnf_tfast(const View4& w) { return !(w.sk == 1 || w.sp != 1); }
 static bool bnf_slab_ok(const View4& w, int T, int V) {
@@ -1391,8 +1498,8 @@ static bool bnf_slab_ok(const View4& w, int T, int V) {
   return dense && w.sc == (long long)T * V && (reinterpret_cast<unsigned long long>(w.p) & 15ull) == 0 && (w.sn & 3ll) == 0;
 }
 static BnFastPlan bnf_plan(bool fast, int C, int T, int V, const float* mask, std::initializer_list<const View4*> ws) {
-  BnFastPlan pl{false, 0, 0, 0, false};
-  if (!fast || mask || V > 32) return pl;
+  BnFastPlan pl{false, 0, 0, 0, false, V > 32};
+  if (!fast || mask || V > BN_MAXV) return pl;
   const int TV = T * V;
   pl.ch = (TV % 4 == 0) ? 1 : (TV % 2 == 0) ? 2 : 4;
   const int chtv = pl.ch * TV;
@@ -1402,12 +1509,16 @@ static BnFastPlan bnf_plan(bool fast, int C, int T, int V, const float* mask, st
     if (!bnf_slab_ok(*w, T, V)) return pl;
   pl.nj = chtv <= 4 * BN_THREADS_MAX ? 4 : 8;
   pl.threads = cdiv(cdiv(chtv, pl.nj), 32) * 32;
+  if (pl.wide && pl.threads < V) pl.threads = cdiv(V, 32) * 32;   // one thread per v in the per-channel steps
   pl.ok = true;
   return pl;
 }
+// The per-(c, v) tables of the wide fast kernels take up to 13.5 KB more static shared memory (bnf_bwd_apply: two
+// float4 tables of BNF_MAXCH * BN_MAXV rows and the fp64 totals) than the 32-joint ones; it comes off the budget.
+constexpr size_t BNF_WIDE_TABLES = (size_t)(2 * BNF_MAXCH * 16 + 16) * (BN_MAXV - 32);
 // samples per stage: the largest of 4/2/1 whose two stages of `nst` slabs fit two CTAs per SM; 0 = none
-static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false) {
-  const size_t budget = big ? (size_t)220 * 1024 : BN_SMEM_BUDGET;   // BIG: one CTA per SM
+static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false, bool wide = false) {
+  const size_t budget = (big ? (size_t)220 * 1024 : BN_SMEM_BUDGET) - (wide ? BNF_WIDE_TABLES : 0);   // BIG: one CTA per SM
   for (int u = big ? 2 : 4; u >= 1; u >>= 1)
     if ((size_t)2 * nst * u * slab_bytes <= budget) return u;
   return 0;
@@ -1427,13 +1538,19 @@ static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false) {
     }                                                                                                 \
   } while (0)
 // plan: {nj, big}; BIG slabs always run 8 positions per thread, 2 or 1 samples per stage
-#define DSTD_BNF(KERN, plan, u, grid, threads, smem, st, ...)                                         \
+#define DSTD_BNF_NJ(KERN, plan, u, grid, threads, smem, st, ...)                                      \
   do {                                                                                                \
     if ((plan).big) {                                                                                 \
       if ((u) == 2) DSTD_BNF_ONE(KERN, 8, 2, true, grid, threads, smem, st, __VA_ARGS__);             \
       else DSTD_BNF_ONE(KERN, 8, 1, true, grid, threads, smem, st, __VA_ARGS__);                      \
     } else if ((plan).nj == 4) DSTD_BNF_U(KERN, 4, u, grid, threads, smem, st, __VA_ARGS__);          \
     else DSTD_BNF_U(KERN, 8, u, grid, threads, smem, st, __VA_ARGS__);                                \
+  } while (0)
+// plan.wide picks KERN##_W, the macro naming the kernel's _wide_ twin
+#define DSTD_BNF(KERN, plan, u, grid, threads, smem, st, ...)                                         \
+  do {                                                                                                \
+    if ((plan).wide) DSTD_BNF_NJ(KERN##_W, plan, u, grid, threads, smem, st, __VA_ARGS__);            \
+    else DSTD_BNF_NJ(KERN, plan, u, grid, threads, smem, st, __VA_ARGS__);                            \
   } while (0)
 
 // U (samples per pipeline stage) is a launch-time choice among the compiled instantiations
@@ -1464,6 +1581,13 @@ static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false) {
     }                                                                                 \
   } while (0)
 
+// V > 32: the kernel's _wide_ twin
+#define DSTD_BN_DISPATCH_UW(kern, wide, nj, u, grid, threads, smem, st, ...)         \
+  do {                                                                                \
+    if (wide) DSTD_BN_DISPATCH_U(kern##_wide_kernel, nj, u, grid, threads, smem, st, __VA_ARGS__); \
+    else DSTD_BN_DISPATCH_U(kern##_kernel, nj, u, grid, threads, smem, st, __VA_ARGS__);           \
+  } while (0)
+
 #define DSTD_BN_DISPATCH(kern, nj, grid, threads, smem, st, q)          \
   do {                                                                  \
     switch (nj) {                                                       \
@@ -1490,15 +1614,30 @@ extern "C" size_t dstd_bn_act_workspace_bytes(int N, int C, int T, int V) {
 // parameter gradients.
 enum BnPhase { BN_PLAIN, BN_LOCAL, BN_GLOBAL };
 
+// T*V above BN_MAXJ * BN_THREADS_MAX: only V > 32 on the fast path (`fast`: it takes every pass of the call)
+static int bn_check_positions(int T, int V, bool fast) {
+  DSTD_REQUIRE(T * V <= BN_MAXJ * BN_THREADS_MAX || (V > 32 && fast), DSTD_ERR_UNSUPPORTED,
+               "bn_act: T*V=%d outside the compiled limits: the generic kernels (dropout mask, layouts the fast path "
+               "does not take, V <= 32) run up to %d positions, the fast path for V > 32 slabs of up to %d",
+               T * V, BN_MAXJ * BN_THREADS_MAX, 8 * BNF_THREADS_BIG);
+  return DSTD_OK;
+}
+
+// fast-path samples per stage of the forward apply pass; 0 = the generic kernel
+static int bn_fwd_fast_u(const BnFwdP& q, const Switches& sw, BnFastPlan* out = nullptr) {
+  const BnFastPlan fp = bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.out});
+  if (out) *out = fp;
+  return fp.ok ? bnf_pick_u((size_t)fp.ch * q.T * q.V * sizeof(float), q.r.p ? 2 : 1, fp.big, fp.wide) : 0;
+}
+
 // ---- forward: argument checks and kernel parameters shared by the plain call and the two synchronised phases
 static int bn_fwd_setup(const dstd_bn_act_fwd_args* a, const Switches& sw, BnFwdP& q, BnPhase ph = BN_PLAIN) {
   DSTD_REQUIRE(a, DSTD_ERR_BAD_ARG, "bn_act_forward: null args");
   DSTD_REQUIRE(a->N > 0 && a->C > 0 && a->T > 0 && a->V > 0, DSTD_ERR_BAD_ARG, "bn_act_forward: bad dims");
   DSTD_REQUIRE(a->y.ptr && (ph == BN_LOCAL || (a->out.ptr && a->gamma && a->beta && a->save_mean && a->save_invstd)),
                DSTD_ERR_BAD_ARG, "bn_act_forward: null tensor");
-  DSTD_REQUIRE(a->T * a->V <= BN_MAXJ * BN_THREADS_MAX && a->V <= 32, DSTD_ERR_UNSUPPORTED,
-               "bn_act: T*V=%d (max %d) or V=%d (max 32) outside the compiled limits", a->T * a->V,
-               BN_MAXJ * BN_THREADS_MAX, a->V);
+  DSTD_REQUIRE(a->V <= BN_MAXV, DSTD_ERR_UNSUPPORTED, "bn_act: V=%d joints (max %d) outside the compiled limits",
+               a->V, BN_MAXV);
   DSTD_REQUIRE(a->training || (a->running_mean && a->running_var), DSTD_ERR_BAD_ARG,
                "bn_act_forward: eval mode needs running statistics");
   DSTD_REQUIRE(ph == BN_GLOBAL || (a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws),
@@ -1518,12 +1657,18 @@ static int bn_fwd_setup(const dstd_bn_act_fwd_args* a, const Switches& sw, BnFwd
     Arena ar(a->ws, a->ws_bytes);
     q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
   }
-  return DSTD_OK;
+  return bn_check_positions(q.T, q.V, q.T * q.V <= BN_MAXJ * BN_THREADS_MAX || bn_fwd_fast_u(q, sw) > 0);
 }
 
 static int bn_fwd_stats(const BnFwdP& q, cudaStream_t st) {
   const BnGeom g = bn_geom(q.T, q.V);
-  DSTD_BN_DISPATCH(bn_stats_kernel, g.nj, dim3(q.C, q.S), g.threads, 2 * (size_t)q.T * q.V * sizeof(float), st, q);
+  const size_t smem = 2 * (size_t)q.T * q.V * sizeof(float);
+  if (q.T * q.V > BN_MAXJ * BN_THREADS_MAX) {
+    prefer_smem_carveout((const void*)bn_stats_big_kernel, true);
+    bn_stats_big_kernel<<<dim3(q.C, q.S), g.threads, smem, st>>>(q);
+  } else {
+    DSTD_BN_DISPATCH(bn_stats_kernel, g.nj, dim3(q.C, q.S), g.threads, smem, st, q);
+  }
   count_launch();
   DSTD_LAUNCH_CHECK("bn_stats");
   return DSTD_OK;
@@ -1533,18 +1678,22 @@ static int bn_fwd_stats(const BnFwdP& q, cudaStream_t st) {
 static int bn_fwd_apply(const BnFwdP& q, const Switches& sw, cudaStream_t st) {
   const size_t tvb = (size_t)q.T * q.V * sizeof(float);
   const int nst = q.r.p ? 2 : 1;                       // staged tensors: y (, r); two pipeline stages
-  const BnFastPlan fp = bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.out});
-  const int fu = fp.ok ? bnf_pick_u((size_t)fp.ch * tvb, nst, fp.big) : 0;
+  BnFastPlan fp;
+  const int fu = bn_fwd_fast_u(q, sw, &fp);
   if (fu) {
     const dim3 grid(q.C / fp.ch, q.S);
     const size_t smem = (size_t)2 * nst * fu * fp.ch * tvb;
     int* err = device_error_word();
 #define DSTD_K_APPLY_R(NJ_, U_, B_) bnf_apply_kernel<NJ_, U_, true, B_>
 #define DSTD_K_APPLY(NJ_, U_, B_) bnf_apply_kernel<NJ_, U_, false, B_>
+#define DSTD_K_APPLY_R_W(NJ_, U_, B_) bnf_apply_wide_kernel<NJ_, U_, true, B_>
+#define DSTD_K_APPLY_W(NJ_, U_, B_) bnf_apply_wide_kernel<NJ_, U_, false, B_>
     if (q.r.p) DSTD_BNF(DSTD_K_APPLY_R, fp, fu, grid, fp.threads, smem, st, q, fp.ch, err);
     else DSTD_BNF(DSTD_K_APPLY, fp, fu, grid, fp.threads, smem, st, q, fp.ch, err);
 #undef DSTD_K_APPLY_R
 #undef DSTD_K_APPLY
+#undef DSTD_K_APPLY_R_W
+#undef DSTD_K_APPLY_W
     count_launch();
     DSTD_LAUNCH_CHECK("bnf_apply");
     return DSTD_OK;
@@ -1552,7 +1701,7 @@ static int bn_fwd_apply(const BnFwdP& q, const Switches& sw, cudaStream_t st) {
   const BnGeom g = bn_geom(q.T, q.V);
   const int u = bn_pick_u(tvb, 2 * nst, 4, BN_SMEM_BUDGET);
   const size_t smu = (size_t)2 * nst * u * tvb;
-  DSTD_BN_DISPATCH_U(bn_apply_kernel, g.nj, u, dim3(q.C, q.S), g.threads, smu, st, q);
+  DSTD_BN_DISPATCH_UW(bn_apply, q.V > 32, g.nj, u, dim3(q.C, q.S), g.threads, smu, st, q);
   count_launch();
   DSTD_LAUNCH_CHECK("bn_apply");
   return DSTD_OK;
@@ -1587,7 +1736,8 @@ extern "C" int dstd_bn_act_forward_local(const dstd_bn_act_fwd_args* a, double* 
   if (rc != DSTD_OK) return rc;
   rc = bn_fwd_stats(q, st);
   if (rc != DSTD_OK) return rc;
-  bn_sync_fold_fwd_kernel<<<q.C, 256, 0, st>>>(q, mine);
+  if (q.V > 32) bn_sync_fold_fwd_wide_kernel<<<q.C, 256, 0, st>>>(q, mine);
+  else bn_sync_fold_fwd_kernel<<<q.C, 256, 0, st>>>(q, mine);
   count_launch();
   DSTD_LAUNCH_CHECK("bn_sync_fold_fwd");
   return DSTD_OK;
@@ -1620,6 +1770,8 @@ struct BnBwdPlan {
   bool fast() const { return u1 && u2; }
 };
 
+static BnBwdPlan bn_bwd_plan(const BnBwdP& q, const Switches& sw);
+
 // (the local phase takes gy / gr as well: it does not write them, but their layouts pick the kernels, as in the plain
 // call)
 static int bn_bwd_setup(const dstd_bn_act_bwd_args* a, const Switches& sw, BnBwdP& q, BnPhase ph = BN_PLAIN) {
@@ -1630,8 +1782,8 @@ static int bn_bwd_setup(const dstd_bn_act_bwd_args* a, const Switches& sw, BnBwd
                DSTD_ERR_BAD_ARG, "bn_act_backward: null tensor");
   DSTD_REQUIRE(!a->gr.ptr || a->r.ptr, DSTD_ERR_BAD_ARG, "bn_act_backward: gr requested without r");
   DSTD_REQUIRE(!a->gr_add.ptr || a->gr.ptr, DSTD_ERR_BAD_ARG, "bn_act_backward: gr_add given without gr");
-  DSTD_REQUIRE(a->T * a->V <= BN_MAXJ * BN_THREADS_MAX && a->V <= 32, DSTD_ERR_UNSUPPORTED,
-               "bn_act: T*V=%d or V=%d outside the compiled limits", a->T * a->V, a->V);
+  DSTD_REQUIRE(a->V <= BN_MAXV, DSTD_ERR_UNSUPPORTED, "bn_act: V=%d joints (max %d) outside the compiled limits",
+               a->V, BN_MAXV);
   DSTD_REQUIRE(ph == BN_GLOBAL || (a->ws_bytes >= dstd_bn_act_workspace_bytes(a->N, a->C, a->T, a->V) && a->ws),
                DSTD_ERR_WORKSPACE, "bn_act_backward: workspace too small");
   q.N = a->N; q.C = a->C; q.T = a->T; q.V = a->V;
@@ -1647,7 +1799,7 @@ static int bn_bwd_setup(const dstd_bn_act_bwd_args* a, const Switches& sw, BnBwd
     q.part = ar.take<float>((size_t)q.S * q.C * q.V * 2);
     q.part_p = ar.take<float>((size_t)q.S * q.C);
   }
-  return DSTD_OK;
+  return bn_check_positions(q.T, q.V, q.T * q.V <= BN_MAXJ * BN_THREADS_MAX || bn_bwd_plan(q, sw).fast());
 }
 
 static BnBwdPlan bn_bwd_plan(const BnBwdP& q, const Switches& sw) {
@@ -1662,9 +1814,9 @@ static BnBwdPlan bn_bwd_plan(const BnBwdP& q, const Switches& sw) {
   const bool combo = p.use_r ? has_gr : (!has_gr && !p.add);     // the instantiations the model uses
   const bool gr_same = !has_gr || bnf_tfast(q.gr) == bnf_tfast(q.gy);
   p.fp = (combo && gr_same) ? bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
-                            : BnFastPlan{false, 0, 0, 0, false};
-  p.u1 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst, p.fp.big) : 0;
-  p.u2 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst2, p.fp.big) : 0;
+                            : BnFastPlan{false, 0, 0, 0, false, false};
+  p.u1 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst, p.fp.big, p.fp.wide) : 0;
+  p.u2 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst2, p.fp.big, p.fp.wide) : 0;
   p.ub = bn_pick_u(tv, 2 * p.nst + 1, 4, BN_SMEM_BUDGET);
   p.ub2 = bn_pick_u(tv, 2 * p.nst2 + 1, p.ub, BN_SMEM_BUDGET);
   return p;
@@ -1678,17 +1830,21 @@ static int bn_bwd_reduce(const BnBwdP& q, const BnBwdPlan& p, cudaStream_t st) {
     int* err = device_error_word();
 #define DSTD_K_RED_R(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, true, B_>
 #define DSTD_K_RED(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, false, B_>
+#define DSTD_K_RED_R_W(NJ_, U_, B_) bnf_bwd_reduce_wide_kernel<NJ_, U_, true, B_>
+#define DSTD_K_RED_W(NJ_, U_, B_) bnf_bwd_reduce_wide_kernel<NJ_, U_, false, B_>
     if (p.use_r) DSTD_BNF(DSTD_K_RED_R, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
     else DSTD_BNF(DSTD_K_RED, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
 #undef DSTD_K_RED_R
 #undef DSTD_K_RED
+#undef DSTD_K_RED_R_W
+#undef DSTD_K_RED_W
     count_launch();
     DSTD_LAUNCH_CHECK("bnf_bwd_reduce");
     return DSTD_OK;
   }
   size_t sm_red = (size_t)2 * p.nst * p.ub * tv;
   if (sm_red < 2 * tv) sm_red = 2 * tv;
-  DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, p.g.nj, p.ub, dim3(q.C, q.S), p.g.threads, sm_red, st, q);
+  DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, p.g.nj, p.ub, dim3(q.C, q.S), p.g.threads, sm_red, st, q);   // any V
   count_launch();
   DSTD_LAUNCH_CHECK("bn_bwd_reduce");
   return DSTD_OK;
@@ -1707,22 +1863,34 @@ static int bn_bwd_apply(const BnBwdP& q, const BnBwdPlan& p, const double* all, 
 #define DSTD_K_APP_RA(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, true, B_>
 #define DSTD_K_APP_R(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, false, B_>
 #define DSTD_K_APP(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, false, false, false, B_>
+#define DSTD_K_APP_RA_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, true, true, true, B_>
+#define DSTD_K_APP_R_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, true, true, false, B_>
+#define DSTD_K_APP_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, false, false, false, B_>
       if (p.use_r && p.add) DSTD_BNF(DSTD_K_APP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
       else if (p.use_r) DSTD_BNF(DSTD_K_APP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
       else DSTD_BNF(DSTD_K_APP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
 #undef DSTD_K_APP_RA
 #undef DSTD_K_APP_R
 #undef DSTD_K_APP
+#undef DSTD_K_APP_RA_W
+#undef DSTD_K_APP_R_W
+#undef DSTD_K_APP_W
     } else {
 #define DSTD_K_SAPP_RA(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, true, B_>
 #define DSTD_K_SAPP_R(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, false, B_>
 #define DSTD_K_SAPP(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, false, false, false, B_>
+#define DSTD_K_SAPP_RA_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, true, true, true, B_>
+#define DSTD_K_SAPP_R_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, true, true, false, B_>
+#define DSTD_K_SAPP_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, false, false, false, B_>
       if (p.use_r && p.add) DSTD_BNF(DSTD_K_SAPP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
       else if (p.use_r) DSTD_BNF(DSTD_K_SAPP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
       else DSTD_BNF(DSTD_K_SAPP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
 #undef DSTD_K_SAPP_RA
 #undef DSTD_K_SAPP_R
 #undef DSTD_K_SAPP
+#undef DSTD_K_SAPP_RA_W
+#undef DSTD_K_SAPP_R_W
+#undef DSTD_K_SAPP_W
     }
     count_launch();
     DSTD_LAUNCH_CHECK("bnf_bwd_apply");
@@ -1730,12 +1898,13 @@ static int bn_bwd_apply(const BnBwdP& q, const BnBwdPlan& p, const double* all, 
   }
   const size_t sm2 = (size_t)(2 * p.nst2 + 1) * p.ub2 * tv;
   const dim3 grid(q.C, q.S);
+  const bool wide = q.V > 32;
   if (!all) {
-    if (q.gadd.p) DSTD_BN_DISPATCH_U(bn_bwd_apply_add_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
-    else DSTD_BN_DISPATCH_U(bn_bwd_apply_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
+    if (q.gadd.p) DSTD_BN_DISPATCH_UW(bn_bwd_apply_add, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
+    else DSTD_BN_DISPATCH_UW(bn_bwd_apply, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
   } else {
-    if (q.gadd.p) DSTD_BN_DISPATCH_U(bn_bwd_apply_add_sync_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
-    else DSTD_BN_DISPATCH_U(bn_bwd_apply_sync_kernel, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
+    if (q.gadd.p) DSTD_BN_DISPATCH_UW(bn_bwd_apply_add_sync, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
+    else DSTD_BN_DISPATCH_UW(bn_bwd_apply_sync, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
   }
   count_launch();
   DSTD_LAUNCH_CHECK("bn_bwd_apply");
@@ -1768,7 +1937,8 @@ extern "C" int dstd_bn_act_backward_local(const dstd_bn_act_bwd_args* a, double*
   // the block size and slope-partial count of the apply kernel the plain call would run: same gprelu summation order
   const int threads = p.fast() ? p.fp.threads : p.g.threads;
   const int np = p.fast() ? (q.C / p.fp.ch) * q.S : q.S * q.C;
-  bn_sync_fold_bwd_kernel<<<q.C, threads, 0, st>>>(q, np, mine);
+  if (q.V > 32) bn_sync_fold_bwd_wide_kernel<<<q.C, threads, 0, st>>>(q, np, mine);
+  else bn_sync_fold_bwd_kernel<<<q.C, threads, 0, st>>>(q, np, mine);
   count_launch();
   DSTD_LAUNCH_CHECK("bn_sync_fold_bwd");
   return DSTD_OK;

@@ -53,11 +53,19 @@ _MIRROR = {
 }
 
 
+def _registered_mirror(layout: str):
+    from .model.layers import graph
+    lists = graph.mirror_lists(layout)      # KeyError for an unknown layout, as for the built-in table
+    if lists is None:
+        raise ValueError(f"layout {layout!r} was registered without mirror lists (register_layout(..., mirror=(right, left)))")
+    return lists
+
+
 def mirror(all_seqs: torch.Tensor, layout: str) -> torch.Tensor:
     """Left/right mirrored copy of raw windows ``[N, T, 3J]`` (``get_mirror`` of dataset/h36m.py:100-116,
     dataset/cmu.py:93-105, dataset/pw3d.py:116-128): `m[right] = src[left]`, then `m[left] = src[right]`, then negate x.
-    Runs on the tensor's device."""
-    right, left = _MIRROR[layout]
+    Runs on the tensor's device.  A layout added with ``graph.register_layout`` uses the lists registered with it."""
+    right, left = _MIRROR[layout] if layout in _MIRROR else _registered_mirror(layout)
     n, t, vc = all_seqs.shape
     src = all_seqs.view(n, t, vc // 3, 3)
     dev = all_seqs.device

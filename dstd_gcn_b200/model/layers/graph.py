@@ -11,6 +11,11 @@ The reference builds the matrices from raw-skeleton joint ids and a
 compact index space the model sees (0..V-1), which is the only form the hot
 path ever consumes.  ``tests/test_layers.py`` checks every matrix against the
 golden copies dumped from the reference (``tests/golden/adjacency.npz``).
+
+Other skeletons (up to ``MAX_JOINTS`` joints) are added to the same table with
+``register_layout``; every consumer of a layout name (``Graph``, the models'
+``layout=`` argument, ``data.mirror``, ``DevicePrefetcher(mirror_layout=)``)
+then accepts the new name.
 """
 import numpy as np
 
@@ -40,12 +45,72 @@ _EDGES = {
 }
 
 
+# the BatchNorm kernels hold the per-joint constants of a channel in one table of this many rows
+MAX_JOINTS = 128
+
+
 def _parse(spec):
     return [tuple(int(t) for t in e.split("-")) for e in spec.split()]
 
 
+def _int(x, what):
+    if isinstance(x, (bool, np.bool_)) or not isinstance(x, (int, np.integer)):
+        raise TypeError(f"{what} must be an int, got {x!r}")
+    return int(x)
+
+
+def _edge_list(pairs, joints, what):
+    out, seen = [], set()
+    for e in pairs:
+        if len(e) != 2:
+            raise ValueError(f"{what}: {e!r} is not a pair of joint indices")
+        i, j = _int(e[0], what), _int(e[1], what)
+        if i == j:
+            raise ValueError(f"{what}: self loop {i}-{j} (the identity is added by the graph itself)")
+        if not 0 <= i < j < joints:
+            raise ValueError(f"{what}: edge {i}-{j} must satisfy 0 <= i < j < joints = {joints}")
+        if (i, j) in seen:
+            raise ValueError(f"{what}: duplicate edge {i}-{j}")
+        seen.add((i, j))
+        out.append(f"{i}-{j}")
+    return " ".join(out)
+
+
+def register_layout(name, joints, bones, parts, mirror=None):
+    """Add a skeleton layout under ``name``: ``joints`` joints (1 .. ``MAX_JOINTS``), the ``bones`` of the ``connect``
+    adjacency and the semantic ``parts`` pairs, each a sequence of ``(i, j)`` with ``0 <= i < j < joints`` and no
+    duplicates.  ``mirror`` is an optional ``(right, left)`` pair of equal-length, disjoint joint-index lists of the
+    raw windows that ``data.mirror`` swaps; without it, mirroring the layout raises.  A name can be registered once
+    and the built-in layouts cannot be replaced."""
+    if not isinstance(name, str) or not name:
+        raise ValueError(f"layout name must be a non-empty string, got {name!r}")
+    if name in _EDGES:
+        raise ValueError(f"layout {name!r} is already registered")
+    joints = _int(joints, "joints")
+    if not 1 <= joints <= MAX_JOINTS:
+        raise ValueError(f"joints = {joints} outside 1 .. {MAX_JOINTS}")
+    spec = dict(joints=joints, bones=_edge_list(bones, joints, "bones"), parts=_edge_list(parts, joints, "parts"))
+    if mirror is not None:
+        if len(mirror) != 2:
+            raise ValueError("mirror must be a (right, left) pair of joint-index lists")
+        right, left = ([_int(k, "mirror") for k in side] for side in mirror)
+        if len(right) != len(left):
+            raise ValueError(f"mirror: right has {len(right)} joints, left {len(left)}")
+        if min(right + left, default=0) < 0:
+            raise ValueError("mirror: negative joint index")
+        if len(set(right)) != len(right) or len(set(left)) != len(left) or set(right) & set(left):
+            raise ValueError("mirror: right and left must be disjoint lists of distinct joints")
+        spec["mirror"] = (right, left)
+    _EDGES[name] = spec
+
+
+def mirror_lists(layout):
+    """``(right, left)`` lists given to ``register_layout`` for ``layout``, or None if it was registered without."""
+    return _EDGES[layout].get("mirror")
+
+
 class Graph:
-    """Skeleton graph of one dataset layout (``h36m`` 22 joints, ``cmu`` 25, ``3dpw`` 23)."""
+    """Skeleton graph of one dataset layout (``h36m`` 22 joints, ``cmu`` 25, ``3dpw`` 23, or a registered one)."""
 
     def __init__(self, layout="h36m"):
         if layout not in _EDGES:

@@ -131,6 +131,10 @@ int dstd_gc_backward(const dstd_gc_bwd_args* a, dstd_stream_t stream);
  * Views are addressed (n,c,t,v) -> (n,c,p,k).  BN parameter index is c*V+v, or v*C+c when vc_order.
  * training: batch statistics (biased variance), running stats updated with `momentum`
  * (unbiased variance), *num_batches_tracked += 1.  eval: running statistics.
+ * Shapes: V <= 128 joints and T*V <= 4096 positions.  Planes of 4097 .. 8192 positions run only
+ * when V > 32 and the bulk-copy kernels take the call: no mask, dense 16-byte aligned channel
+ * slabs, the channel count a multiple of the slab's (1, 2 or 4 channels, at most 2 above 4096
+ * positions), DSTD_BN_FAST not 0.  Otherwise DSTD_ERR_UNSUPPORTED.
  * ------------------------------------------------------------------------------------------- */
 typedef struct {
   int N, C, T, V;
