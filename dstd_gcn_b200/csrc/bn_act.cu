@@ -1,11 +1,21 @@
 // Fused BatchNorm(C*V channels, statistics over N,T) + residual + PReLU + dropout mask, forward and backward
 // (model/dstdgcn.py:44-50 BatchNorm.forward, :152-154 `x = bn(x); x += r; x = prelu(x)`, :306-308, :283-284).
 //
-// Work decomposition shared by all four kernels: CTA = (channel c, batch split s); a thread owns up to MAXJ fixed
-// (t,v) positions of the T x V plane and walks the samples of its split, so the per-(c,v) BN parameters are
-// per-thread constants and every access to a [T x V] plane is one contiguous, coalesced sweep.  When the producer and
-// the consumer keep the plane in different memory orders (T-major vs V-major: this op is where the block switches
-// between the spatial and the temporal unit layout) the plane is transposed through shared memory.
+// Kernel families:
+//  * generic (bn_stats, bn_apply, bn_bwd_reduce, bn_bwd_apply): any strides, dropout mask.  CTA = (channel c, batch
+//    split s); a thread owns up to BN_MAXJ fixed (t,v) positions of the T x V plane and walks the samples of its
+//    split, so the per-(c,v) BN parameters are per-thread constants and every access to a [T x V] plane is one
+//    contiguous, coalesced sweep.  When the producer and the consumer keep the plane in different memory orders
+//    (T-major vs V-major: this op is where the block switches between the spatial and the temporal unit layout) the
+//    plane is transposed through shared memory.
+//  * fast (bnf_apply, bnf_bwd_reduce, bnf_bwd_apply): dense CH-channel slabs staged by bulk copies ("fast path"
+//    below); bit-identical to the generic kernels.
+//  * synchronised BatchNorm: bn_sync_fold_fwd / bn_sync_fold_bwd (this rank's exchange rows) and bn_sync_merge_fwd
+//    (the ranks' rows merged) around the all-gather.
+// Twins of a kernel carry the same body with a compile-time flag and are named by suffix, in this order:
+// `_add` stages gr_add and sums it into gr, `_sync` is the global phase of the synchronised backward (k1, k2 from the
+// gathered rows), `_wide` sizes the per-(c, v) shared tables for V = 33 .. BN_MAXV.  Every V <= 32 kernel is the
+// kernel of a 32-joint build.
 //
 // Statistics use shifted sums (shift = y[0,c,0,v]) accumulated in fp32 per thread and combined in fp64, so the
 // E[x^2]-E[x]^2 cancellation does not bite on millimetre-scale poses.
@@ -55,7 +65,7 @@ static BnGeom bn_geom(int T, int V) {
 }
 
 // position j (0..TV) in the memory order of view `v` -> logical (t, v)
-__device__ __forceinline__ bool t_fastest(const View4& vw) { return !(vw.sk == 1 || vw.sp != 1); }
+__host__ __device__ __forceinline__ bool t_fastest(const View4& vw) { return !(vw.sk == 1 || vw.sp != 1); }
 __device__ __forceinline__ void decode_pos(const View4& vw, int j, int T, int V, int& t, int& v) {
   if (!t_fastest(vw)) {   // V fastest (or generic): j = t*V + v
     t = j / V;
@@ -147,10 +157,13 @@ __device__ __forceinline__ void cp_async4_s(unsigned sdst, const float* gsrc) {
 __device__ __forceinline__ void cp_async8_s(unsigned sdst, const float* gsrc) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sdst), "l"(gsrc) : "memory");
 }
+// the [T x V] planes of `w` are dense in w's memory order
+__host__ __device__ __forceinline__ bool plane_dense(const View4& w, int T, int V) {
+  return t_fastest(w) ? (w.sp == 1 && w.sk == T) : (w.sk == 1 && w.sp == V);
+}
 // how a [T x V] plane of `w` can be copied: 2 = dense and every plane 8-byte aligned, 1 = dense, 0 = generic strides
 __device__ __forceinline__ int plane_mode(const View4& w, int T, int V) {
-  const bool dense = t_fastest(w) ? (w.sp == 1 && w.sk == T) : (w.sk == 1 && w.sp == V);
-  if (!dense) return 0;
+  if (!plane_dense(w, T, V)) return 0;
   const bool al8 = ((reinterpret_cast<unsigned long long>(w.p) & 7ull) == 0) && !((w.sn | w.sc) & 1ll) && !((T * V) & 1);
   return al8 ? 2 : 1;
 }
@@ -158,14 +171,18 @@ __device__ __forceinline__ int plane_mode(const View4& w, int T, int V) {
 __device__ __forceinline__ int slot_of(bool tfast, int t, int v, int T, int V) { return tfast ? v * T + t : t * V + v; }
 
 // cp.async samples n .. n+U-1 (`left` of them exist) of channel plane c of `w` into the [U][T*V] region at shared
-// address `sdst`, each plane in w's own memory order
-template <int NJ, int U, bool FULL>
+// address `sdst`, each plane in w's own memory order.
+// The forward passes `mode` = plane_mode(w, T, V), hoisted out of its sample loop, and, since the launch geometry
+// gives NJ * blockDim >= T*V, leaves the pair loop after one pair for NJ <= 2.  BWD: the backward kernels' form, which
+// derives `mode` here at every call (the argument is ignored) and has no single-pair break: they sit at the
+// 64-register cap and measured slower with the hoisted mode / single-pair form.
+template <int NJ, int U, bool FULL, bool BWD>
 __device__ __forceinline__ void stage_async(const Pos2<NJ>& ps, const View4& w, int mode, int c, int n, int left,
                                             unsigned sdst, int T, int V) {
   const int TV = T * V;
+  if (BWD) mode = plane_mode(w, T, V);
   const float* base = w.p + (long long)n * w.sn + (long long)c * w.sc;
   if (mode == 2) {
-    // the launch geometry gives NJ * blockDim >= T*V, so for NJ <= 2 a thread owns at most one pair of positions
     for (int j = 2 * threadIdx.x; j < TV; j += 2 * blockDim.x) {
       const float* p = base + j;
       unsigned d = sdst + (unsigned)j * 4u;
@@ -175,7 +192,7 @@ __device__ __forceinline__ void stage_async(const Pos2<NJ>& ps, const View4& w, 
         p += w.sn;
         d += (unsigned)TV * 4u;
       }
-      if (NJ <= 2) break;
+      if (!BWD && NJ <= 2) break;
     }
   } else {
     const bool tfast = t_fastest(w);
@@ -197,41 +214,19 @@ __device__ __forceinline__ void stage_async(const Pos2<NJ>& ps, const View4& w, 
   }
 }
 
-// backward kernels: same copy, plane mode derived at the call (they sit at the 64-register cap and measured slower
-// with the hoisted mode / single-pair form of the forward)
-template <int NJ, int U, bool FULL>
-__device__ __forceinline__ void stage_async_b(const Pos2<NJ>& ps, const View4& w, int c, int n, int left, unsigned sdst,
-                                              int T, int V) {
-  const int TV = T * V, mode = plane_mode(w, T, V);
-  const float* base = w.p + (long long)n * w.sn + (long long)c * w.sc;
-  if (mode == 2) {
-    for (int j = 2 * threadIdx.x; j < TV; j += 2 * blockDim.x) {
-      const float* p = base + j;
-      unsigned d = sdst + (unsigned)j * 4u;
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        if (FULL || u < left) cp_async8_s(d, p);
-        p += w.sn;
-        d += (unsigned)TV * 4u;
-      }
+// Split s's partial pair of channel c for every v: the per-position sums in sh[0 .. T*V) and sh[T*V .. 2*T*V)
+// (logical slots t*V+v) summed over t in order, in fp64, into part[s][c][v][0..1]
+__device__ __forceinline__ void bn_store_partials(const float* sh, float* part, int s, int C, int c, int T, int V) {
+  if (threadIdx.x < V) {
+    const int v = threadIdx.x, TV = T * V;
+    double s1 = 0., s2 = 0.;
+    for (int t = 0; t < T; ++t) {
+      s1 += sh[t * V + v];
+      s2 += sh[TV + t * V + v];
     }
-  } else {
-    const bool tfast = t_fastest(w);
-#pragma unroll
-    for (int i = 0; i < NJ; ++i) {
-      const int pk = tfast ? ps.tf[i] : ps.vf[i];
-      if (pk >= 0) {
-        const int j = threadIdx.x + i * blockDim.x;
-        const float* p = base + (mode ? (long long)j : (long long)(pk >> 8) * w.sp + (long long)(pk & 255) * w.sk);
-        unsigned d = sdst + (unsigned)j * 4u;
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          if (FULL || u < left) cp_async4_s(d, p);
-          p += w.sn;
-          d += (unsigned)TV * 4u;
-        }
-      }
-    }
+    float* dst = part + (((long long)s * C + c) * V + v) * 2;
+    dst[0] = (float)s1;
+    dst[1] = (float)s2;
   }
 }
 
@@ -313,17 +308,7 @@ __device__ __forceinline__ void bn_stats_body(const BnFwdP& q) {
       }
   }
   __syncthreads();
-  if (threadIdx.x < V) {
-    int v = threadIdx.x;
-    double s1 = 0., s2 = 0.;
-    for (int t = 0; t < T; ++t) {
-      s1 += sh[t * V + v];
-      s2 += sh[TV + t * V + v];
-    }
-    float* dst = q.part + (((long long)s * q.C + c) * V + v) * 2;
-    dst[0] = (float)s1;
-    dst[1] = (float)s2;
-  }
+  bn_store_partials(sh, q.part, s, q.C, c, T, V);
 }
 
 template <int NJ>
@@ -420,11 +405,11 @@ __device__ __forceinline__ void bn_apply_body(const BnFwdP& q) {
     const unsigned d = sbase + (unsigned)((it & 1) * stage_f) * 4u;
     const int n = n0 + it * U, left = n1 - n;
     if (left >= U) {
-      stage_async<NJ, U, true>(ps, q.y, mode_y, c, n, left, d, T, V);
-      if (has_r) stage_async<NJ, U, true>(ps, q.r, mode_r, c, n, left, d + (unsigned)(U * TV) * 4u, T, V);
+      stage_async<NJ, U, true, false>(ps, q.y, mode_y, c, n, left, d, T, V);
+      if (has_r) stage_async<NJ, U, true, false>(ps, q.r, mode_r, c, n, left, d + (unsigned)(U * TV) * 4u, T, V);
     } else {
-      stage_async<NJ, U, false>(ps, q.y, mode_y, c, n, left, d, T, V);
-      if (has_r) stage_async<NJ, U, false>(ps, q.r, mode_r, c, n, left, d + (unsigned)(U * TV) * 4u, T, V);
+      stage_async<NJ, U, false, false>(ps, q.y, mode_y, c, n, left, d, T, V);
+      if (has_r) stage_async<NJ, U, false, false>(ps, q.r, mode_r, c, n, left, d + (unsigned)(U * TV) * 4u, T, V);
     }
   };
   if (iters > 0) issue(0);
@@ -518,6 +503,14 @@ struct BnBwdP {
   float* part_p;  // [S][C]
 };
 
+// gprelu = the np slope partials of pass 1 summed in a fixed order; called by all threads of one CTA
+__device__ __forceinline__ void bn_sum_slope_partials(const BnBwdP& q, int np, float* red) {
+  float a = 0.f;
+  for (int i = threadIdx.x; i < np; i += blockDim.x) a += q.part_p[i];
+  const float t = block_sum(a, red);
+  if (threadIdx.x == 0) q.gprelu[0] = t;
+}
+
 // d(pre-activation) at one element; also returns xhat and the PReLU-slope contribution
 __device__ __forceinline__ float bn_gpre(bool has_prelu, float yv, float rv, float gv, float mv, float mu, float is,
                                          float g, float b, float slope, float& xhat, float& gslope) {
@@ -586,13 +579,13 @@ __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_reduce_kernel(BnBwdP
     const unsigned d = sbase + (unsigned)((it & 1) * stage_f) * 4u, du = (unsigned)(U * TV) * 4u;
     const int n = n0 + it * U, left = n1 - n;
     if (left >= U) {
-      stage_async_b<NJ, U, true>(ps, q.gout, c, n, left, d, T, V);
-      stage_async_b<NJ, U, true>(ps, q.y, c, n, left, d + du, T, V);
-      if (use_r) stage_async_b<NJ, U, true>(ps, q.r, c, n, left, d + 2 * du, T, V);
+      stage_async<NJ, U, true, true>(ps, q.gout, 0, c, n, left, d, T, V);
+      stage_async<NJ, U, true, true>(ps, q.y, 0, c, n, left, d + du, T, V);
+      if (use_r) stage_async<NJ, U, true, true>(ps, q.r, 0, c, n, left, d + 2 * du, T, V);
     } else {
-      stage_async_b<NJ, U, false>(ps, q.gout, c, n, left, d, T, V);
-      stage_async_b<NJ, U, false>(ps, q.y, c, n, left, d + du, T, V);
-      if (use_r) stage_async_b<NJ, U, false>(ps, q.r, c, n, left, d + 2 * du, T, V);
+      stage_async<NJ, U, false, true>(ps, q.gout, 0, c, n, left, d, T, V);
+      stage_async<NJ, U, false, true>(ps, q.y, 0, c, n, left, d + du, T, V);
+      if (use_r) stage_async<NJ, U, false, true>(ps, q.r, 0, c, n, left, d + 2 * du, T, V);
     }
   };
   if (iters > 0) issue(0);
@@ -650,17 +643,7 @@ __global__ void __launch_bounds__(BN_THREADS_MAX, 2) bn_bwd_reduce_kernel(BnBwdP
     }
   }
   __syncthreads();
-  if (threadIdx.x < V) {
-    int v = threadIdx.x;
-    double s1 = 0., s2 = 0.;
-    for (int t = 0; t < T; ++t) {
-      s1 += sh[t * V + v];
-      s2 += sh[TV + t * V + v];
-    }
-    float* dst = q.part + (((long long)s * q.C + c) * V + v) * 2;
-    dst[0] = (float)s1;
-    dst[1] = (float)s2;
-  }
+  bn_store_partials(sh, q.part, s, q.C, c, T, V);
   float tot = block_sum(gsl, red);
   if (threadIdx.x == 0) q.part_p[(long long)s * q.C + c] = tot;
 }
@@ -744,7 +727,7 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double*
   const float slope = has_prelu ? __ldg(q.prelu) : 1.f;
   const float icnt = 1.0f / ((float)q.N * (float)T);
   const bool has_add = ADD;       // the host launches the ADD instantiation only with gr and gr_add present
-  const int add_region = has_add ? (use_r ? 3 : 2) : -1;          // staged planes: gout, y, (r), (gr_add)
+  const int add_region = has_add ? (use_r ? 3 : 2) : 0;           // staged planes: gout, y, (r), (gr_add); 0: unused
   const int stage_f = ((use_r ? 3 : 2) + (has_add ? 1 : 0)) * U * TV, iters = (cnt + U - 1) / U;
   const unsigned sbase = (unsigned)__cvta_generic_to_shared(sh);
   float* sho = sh + 2 * stage_f;                       // gr hand-over, each plane in gr's memory order
@@ -756,15 +739,15 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double*
     const unsigned d = sbase + (unsigned)((it & 1) * stage_f) * 4u, du = (unsigned)(U * TV) * 4u;
     const int n = n0 + it * U, left = n1 - n;
     if (left >= U) {
-      stage_async_b<NJ, U, true>(ps, q.gout, c, n, left, d, T, V);
-      stage_async_b<NJ, U, true>(ps, q.y, c, n, left, d + du, T, V);
-      if (use_r) stage_async_b<NJ, U, true>(ps, q.r, c, n, left, d + 2 * du, T, V);
-      if (has_add) stage_async_b<NJ, U, true>(ps, q.gadd, c, n, left, d + add_region * du, T, V);
+      stage_async<NJ, U, true, true>(ps, q.gout, 0, c, n, left, d, T, V);
+      stage_async<NJ, U, true, true>(ps, q.y, 0, c, n, left, d + du, T, V);
+      if (use_r) stage_async<NJ, U, true, true>(ps, q.r, 0, c, n, left, d + 2 * du, T, V);
+      if (has_add) stage_async<NJ, U, true, true>(ps, q.gadd, 0, c, n, left, d + add_region * du, T, V);
     } else {
-      stage_async_b<NJ, U, false>(ps, q.gout, c, n, left, d, T, V);
-      stage_async_b<NJ, U, false>(ps, q.y, c, n, left, d + du, T, V);
-      if (use_r) stage_async_b<NJ, U, false>(ps, q.r, c, n, left, d + 2 * du, T, V);
-      if (has_add) stage_async_b<NJ, U, false>(ps, q.gadd, c, n, left, d + add_region * du, T, V);
+      stage_async<NJ, U, false, true>(ps, q.gout, 0, c, n, left, d, T, V);
+      stage_async<NJ, U, false, true>(ps, q.y, 0, c, n, left, d + du, T, V);
+      if (use_r) stage_async<NJ, U, false, true>(ps, q.r, 0, c, n, left, d + 2 * du, T, V);
+      if (has_add) stage_async<NJ, U, false, true>(ps, q.gadd, 0, c, n, left, d + add_region * du, T, V);
     }
   };
   if (iters > 0) issue(0);
@@ -777,12 +760,7 @@ __device__ __forceinline__ void bn_bwd_apply_body(const BnBwdP& q, const double*
     __syncthreads();
   } else {
     sum_partials(q.part, q.S, q.C, c, V, tot);
-    if (c == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
-      float a = 0.f;
-      for (int i = threadIdx.x; i < q.S * q.C; i += blockDim.x) a += q.part_p[i];
-      const float t = block_sum(a, red);
-      if (threadIdx.x == 0) q.gprelu[0] = t;
-    }
+    if (c == 0 && s == 0 && q.gprelu) bn_sum_slope_partials(q, q.S * q.C, red);
     __syncthreads();
     if (s == 0 && threadIdx.x < V) {
       const int pi = bn_pidx(c, threadIdx.x, q.C, V, q.vc_order);
@@ -942,6 +920,14 @@ template <bool BIG, bool WIDE = false> struct BnfBits {
   static constexpr uint32_t SM = (1u << SB) - 1u;
   static constexpr int VW = bn_table_v(WIDE), KS = WIDE ? 32 : 2 * SB;
   using Pk = typename std::conditional<WIDE, unsigned long long, uint32_t>::type;
+  // slot of slab position (ch, t, v) in a slab staged in memory order tf_a | the same in order tf_b << SB
+  __device__ __forceinline__ static uint32_t slots(int ch, int t, int v, int T, int V, int TV, bool tf_a, bool tf_b) {
+    return (uint32_t)(ch * TV + slot_of(tf_a, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_b, t, v, T, V)) << SB);
+  }
+  // the position word: slots(...) | (ch * VW + v) << KS
+  __device__ __forceinline__ static Pk pack(int ch, int t, int v, int T, int V, int TV, bool tf_a, bool tf_b) {
+    return slots(ch, t, v, T, V, TV, tf_a, tf_b) | ((Pk)(ch * VW + v) << KS);
+  }
 };
 
 __device__ __forceinline__ void bnf_decode(bool tfast, int j, int T, int V, int TV, int& ch, int& t, int& v) {
@@ -957,6 +943,26 @@ __device__ __forceinline__ void bnf_decode(bool tfast, int j, int T, int V, int 
 }
 __device__ __forceinline__ void bnf_timeout(int* err) {
   if (err) *(volatile int*)err = 2;
+}
+// the two stage mbarriers, initialised by thread 0 (the caller synchronises the block before their first use)
+__device__ __forceinline__ void bnf_mbar_init(uint64_t* mbar) {
+  if (threadIdx.x == 0) {
+    umma::mbar_init(&mbar[0], 1);
+    umma::mbar_init(&mbar[1], 1);
+    umma::mbar_init_fence();
+  }
+}
+// the per-(ch, v) constant table of the CH channels at c0 from the BN parameters: ctab[ch * VW + v] = f(pi), pi the
+// parameter index of (c0 + ch, v)
+template <bool WIDE, class F>
+__device__ __forceinline__ void bnf_fill_ctab(float4* ctab, int CH, int c0, int C, int V, int vc_order, F f) {
+  constexpr int VW = bn_table_v(WIDE);
+  if (WIDE) {
+    for (int ix = threadIdx.x; ix < CH * VW; ix += blockDim.x)
+      if (ix % VW < V) ctab[ix] = f(bn_pidx(c0 + ix / VW, ix % VW, C, V, vc_order));
+  } else if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
+    ctab[threadIdx.x] = f(bn_pidx(c0 + (threadIdx.x >> 5), threadIdx.x & 31, C, V, vc_order));
+  }
 }
 
 // ---- forward apply: positions in out's memory order
@@ -998,11 +1004,7 @@ __device__ __forceinline__ void bnf_apply_body(const BnFwdP& q, int CH, int* err
   constexpr int NST = HAS_R ? 2 : 1;
   const int stage_f = NST * U * CHTV, iters = (cnt + U - 1) / U;
   const float slope = q.prelu ? __ldg(q.prelu) : 1.f;
-  if (threadIdx.x == 0) {
-    umma::mbar_init(&mbar[0], 1);
-    umma::mbar_init(&mbar[1], 1);
-    umma::mbar_init_fence();
-  }
+  bnf_mbar_init(mbar);
   __syncthreads();
   auto issue = [&](int it) {   // thread 0: one bulk copy per sample and tensor
     const int n = n0 + it * U, cu = min(U, n1 - n);
@@ -1047,21 +1049,13 @@ __device__ __forceinline__ void bnf_apply_body(const BnFwdP& q, int CH, int* err
       __syncthreads();
     }
   } else {
-    if (WIDE) {
-      for (int ix = threadIdx.x; ix < CH * VW; ix += blockDim.x)
-        if (ix % VW < V) {
-          const int pi = bn_pidx(c0 + ix / VW, ix % VW, q.C, V, q.vc_order);
-          ctab[ix] = make_float4(q.save_mean[pi], __ldg(q.gamma + pi) * q.save_invstd[pi], __ldg(q.beta + pi), 0.f);
-        }
-    } else if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
-      const int pi = bn_pidx(c0 + (threadIdx.x >> 5), threadIdx.x & 31, q.C, V, q.vc_order);
-      ctab[threadIdx.x] = make_float4(q.save_mean[pi], __ldg(q.gamma + pi) * q.save_invstd[pi], __ldg(q.beta + pi), 0.f);
-    }
+    bnf_fill_ctab<WIDE>(ctab, CH, c0, q.C, V, q.vc_order, [&](int pi) {
+      return make_float4(q.save_mean[pi], __ldg(q.gamma + pi) * q.save_invstd[pi], __ldg(q.beta + pi), 0.f);
+    });
     __syncthreads();
   }
   typename BnfBits<BIG, WIDE>::Pk pk[NJ];   // slot in y's slab | slot in r's slab << SB | (ch * VW + v) << KS   (valid iff j < CHTV)
   {
-    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_o = t_fastest(q.out), tf_y = t_fastest(q.y), tf_r = HAS_R && t_fastest(q.r);
 #pragma unroll
     for (int i = 0; i < NJ; ++i) {
@@ -1070,8 +1064,7 @@ __device__ __forceinline__ void bnf_apply_body(const BnFwdP& q, int CH, int* err
       if (j < CHTV) {
         int ch, t, v;
         bnf_decode(tf_o, j, T, V, TV, ch, t, v);
-        pk[i] = (uint32_t)(ch * TV + slot_of(tf_y, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) << SB) |
-                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
+        pk[i] = BnfBits<BIG, WIDE>::pack(ch, t, v, T, V, TV, tf_y, tf_r);
       }
     }
   }
@@ -1142,21 +1135,10 @@ __device__ __forceinline__ void bnf_bwd_reduce_body(const BnBwdP& q, int CH, int
   const int stage_f = NST * U * CHTV, iters = (cnt + U - 1) / U;
   const bool has_prelu = q.prelu != nullptr;
   const float slope = has_prelu ? __ldg(q.prelu) : 1.f;
-  if (threadIdx.x == 0) {
-    umma::mbar_init(&mbar[0], 1);
-    umma::mbar_init(&mbar[1], 1);
-    umma::mbar_init_fence();
-  }
-  if (WIDE) {
-    for (int ix = threadIdx.x; ix < CH * VW; ix += blockDim.x)
-      if (ix % VW < V) {
-        const int pi = bn_pidx(c0 + ix / VW, ix % VW, q.C, V, q.vc_order);
-        ctab[ix] = make_float4(__ldg(q.save_mean + pi), __ldg(q.save_invstd + pi), __ldg(q.gamma + pi), __ldg(q.beta + pi));
-      }
-  } else if (threadIdx.x < CH * 32 && (threadIdx.x & 31) < V) {
-    const int pi = bn_pidx(c0 + (threadIdx.x >> 5), threadIdx.x & 31, q.C, V, q.vc_order);
-    ctab[threadIdx.x] = make_float4(__ldg(q.save_mean + pi), __ldg(q.save_invstd + pi), __ldg(q.gamma + pi), __ldg(q.beta + pi));
-  }
+  bnf_mbar_init(mbar);
+  bnf_fill_ctab<WIDE>(ctab, CH, c0, q.C, V, q.vc_order, [&](int pi) {
+    return make_float4(__ldg(q.save_mean + pi), __ldg(q.save_invstd + pi), __ldg(q.gamma + pi), __ldg(q.beta + pi));
+  });
   __syncthreads();
   auto issue = [&](int it) {
     const int n = n0 + it * U, cu = min(U, n1 - n);
@@ -1177,7 +1159,6 @@ __device__ __forceinline__ void bnf_bwd_reduce_body(const BnBwdP& q, int CH, int
   float a1[NJ], a2[NJ], gsl = 0.f;
   const bool tf_y = t_fastest(q.y);
   {
-    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_g = t_fastest(q.gout), tf_r = USE_R && t_fastest(q.r);
 #pragma unroll
     for (int i = 0; i < NJ; ++i) {
@@ -1187,8 +1168,7 @@ __device__ __forceinline__ void bnf_bwd_reduce_body(const BnBwdP& q, int CH, int
       if (j < CHTV) {
         int ch, t, v;
         bnf_decode(tf_y, j, T, V, TV, ch, t, v);
-        pk[i] = (uint32_t)(ch * TV + slot_of(tf_g, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) << SB) |
-                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
+        pk[i] = BnfBits<BIG, WIDE>::pack(ch, t, v, T, V, TV, tf_g, tf_r);
       }
     }
   }
@@ -1289,11 +1269,7 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
   const bool has_prelu = q.prelu != nullptr;
   const float slope = has_prelu ? __ldg(q.prelu) : 1.f;
   const float icnt = 1.0f / ((float)q.N * (float)T);
-  if (threadIdx.x == 0) {
-    umma::mbar_init(&mbar[0], 1);
-    umma::mbar_init(&mbar[1], 1);
-    umma::mbar_init_fence();
-  }
+  bnf_mbar_init(mbar);
   __syncthreads();
   auto issue = [&](int it) {
     const int n = n0 + it * U, cu = min(U, n1 - n);
@@ -1315,12 +1291,7 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
   };
   if (threadIdx.x == 0 && iters > 0) issue(0);
   // sums of pass 1 over the splits; the s == 0 CTA publishes the parameter gradients of its channels
-  if (!SYNC && blockIdx.x == 0 && s == 0 && q.gprelu) {   // fixed-order sum of the slope partials
-    float a = 0.f;
-    for (int i = threadIdx.x; i < NP; i += blockDim.x) a += q.part_p[i];
-    const float t = block_sum(a, red);
-    if (threadIdx.x == 0) q.gprelu[0] = t;
-  }
+  if (!SYNC && blockIdx.x == 0 && s == 0 && q.gprelu) bn_sum_slope_partials(q, NP, red);
   for (int ch = 0; ch < CH; ++ch) {
     const int c = c0 + ch;
     if (SYNC) sync_bwd_totals(all, world, q.C, V, c, q.vc_order, tot);
@@ -1346,7 +1317,6 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
   typename BnfBits<BIG, WIDE>::Pk pk[NJ];   // gout slot | y slot << SB | (ch * VW + v) << KS
   uint32_t pk2[NJ];                         // r slot | gr_add slot << SB
   {
-    constexpr int SB = BnfBits<BIG, WIDE>::SB, KS = BnfBits<BIG, WIDE>::KS;
     const bool tf_o = t_fastest(q.gy), tf_g = t_fastest(q.gout), tf_y = t_fastest(q.y), tf_r = USE_R && t_fastest(q.r),
                tf_a = ADD && t_fastest(q.gadd);
 #pragma unroll
@@ -1357,9 +1327,8 @@ __device__ __forceinline__ void bnf_bwd_apply_body(const BnBwdP& q, int CH, int 
       if (j < CHTV) {
         int ch, t, v;
         bnf_decode(tf_o, j, T, V, TV, ch, t, v);
-        pk[i] = (uint32_t)(ch * TV + slot_of(tf_g, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_y, t, v, T, V)) << SB) |
-                ((typename BnfBits<BIG, WIDE>::Pk)(ch * VW + v) << KS);
-        pk2[i] = (uint32_t)(ch * TV + slot_of(tf_r, t, v, T, V)) | ((uint32_t)(ch * TV + slot_of(tf_a, t, v, T, V)) << SB);
+        pk[i] = BnfBits<BIG, WIDE>::pack(ch, t, v, T, V, TV, tf_g, tf_y);
+        pk2[i] = BnfBits<BIG, WIDE>::slots(ch, t, v, T, V, TV, tf_r, tf_a);
       }
     }
   }
@@ -1465,12 +1434,7 @@ __device__ __forceinline__ void bn_sync_fold_bwd_body(const BnBwdP& q, int NP, d
   const int c = blockIdx.x, V = q.V;
   const long long cv = (long long)q.C * V;
   sum_partials(q.part, q.S, q.C, c, V, tot);
-  if (c == 0 && q.gprelu) {
-    float a = 0.f;
-    for (int i = threadIdx.x; i < NP; i += blockDim.x) a += q.part_p[i];
-    const float t = block_sum(a, red);
-    if (threadIdx.x == 0) q.gprelu[0] = t;
-  }
+  if (c == 0 && q.gprelu) bn_sum_slope_partials(q, NP, red);
   __syncthreads();
   if (threadIdx.x < V) {
     const int v = threadIdx.x, pi = bn_pidx(c, v, q.C, V, q.vc_order);
@@ -1491,11 +1455,10 @@ struct BnFastPlan {
   bool big;     // slab of 4097 .. 8192 positions: BIG instantiations (<= 1024 threads, one CTA per SM)
   bool wide;    // V > 32: the _wide_ instantiations
 };
-static bool bnf_tfast(const View4& w) { return !(w.sk == 1 || w.sp != 1); }
 static bool bnf_slab_ok(const View4& w, int T, int V) {
   if (!w.p) return true;
-  const bool dense = bnf_tfast(w) ? (w.sp == 1 && w.sk == T) : (w.sk == 1 && w.sp == V);
-  return dense && w.sc == (long long)T * V && (reinterpret_cast<unsigned long long>(w.p) & 15ull) == 0 && (w.sn & 3ll) == 0;
+  return plane_dense(w, T, V) && w.sc == (long long)T * V && (reinterpret_cast<unsigned long long>(w.p) & 15ull) == 0 &&
+         (w.sn & 3ll) == 0;
 }
 static BnFastPlan bnf_plan(bool fast, int C, int T, int V, const float* mask, std::initializer_list<const View4*> ws) {
   BnFastPlan pl{false, 0, 0, 0, false, V > 32};
@@ -1524,79 +1487,40 @@ static int bnf_pick_u(size_t slab_bytes, int nst, bool big = false, bool wide = 
   return 0;
 }
 
-#define DSTD_BNF_ONE(KERN, NJ_, U_, BIG_, grid, threads, smem, st, ...)                               \
-  do {                                                                                                \
-    prefer_smem_carveout((const void*)KERN(NJ_, U_, BIG_), true);                                     \
-    KERN(NJ_, U_, BIG_)<<<grid, threads, smem, st>>>(__VA_ARGS__);                                    \
-  } while (0)
-#define DSTD_BNF_U(KERN, NJ_, u, grid, threads, smem, st, ...)                                        \
-  do {                                                                                                \
-    switch (u) {                                                                                      \
-      case 4: DSTD_BNF_ONE(KERN, NJ_, 4, false, grid, threads, smem, st, __VA_ARGS__); break;         \
-      case 2: DSTD_BNF_ONE(KERN, NJ_, 2, false, grid, threads, smem, st, __VA_ARGS__); break;         \
-      default: DSTD_BNF_ONE(KERN, NJ_, 1, false, grid, threads, smem, st, __VA_ARGS__); break;        \
-    }                                                                                                 \
-  } while (0)
-// plan: {nj, big}; BIG slabs always run 8 positions per thread, 2 or 1 samples per stage
-#define DSTD_BNF_NJ(KERN, plan, u, grid, threads, smem, st, ...)                                      \
-  do {                                                                                                \
-    if ((plan).big) {                                                                                 \
-      if ((u) == 2) DSTD_BNF_ONE(KERN, 8, 2, true, grid, threads, smem, st, __VA_ARGS__);             \
-      else DSTD_BNF_ONE(KERN, 8, 1, true, grid, threads, smem, st, __VA_ARGS__);                      \
-    } else if ((plan).nj == 4) DSTD_BNF_U(KERN, 4, u, grid, threads, smem, st, __VA_ARGS__);          \
-    else DSTD_BNF_U(KERN, 8, u, grid, threads, smem, st, __VA_ARGS__);                                \
-  } while (0)
-// plan.wide picks KERN##_W, the macro naming the kernel's _wide_ twin
-#define DSTD_BNF(KERN, plan, u, grid, threads, smem, st, ...)                                         \
-  do {                                                                                                \
-    if ((plan).wide) DSTD_BNF_NJ(KERN##_W, plan, u, grid, threads, smem, st, __VA_ARGS__);            \
-    else DSTD_BNF_NJ(KERN, plan, u, grid, threads, smem, st, __VA_ARGS__);                            \
-  } while (0)
+// Kernel dispatch: call f with std::integral_constant arguments naming a compiled instantiation.
+template <int K> using IntC = std::integral_constant<int, K>;
+// samples per pipeline stage: 4, 2, or 1 for any other value
+template <class F> static int with_u(int u, F&& f) {
+  if (u == 4) return f(IntC<4>{});
+  if (u == 2) return f(IntC<2>{});
+  return f(IntC<1>{});
+}
+// positions per thread of the generic kernels: 1, 2, 4, or 8 for any other value
+template <class F> static int with_nj(int nj, F&& f) {
+  if (nj == 1) return f(IntC<1>{});
+  if (nj == 2) return f(IntC<2>{});
+  if (nj == 4) return f(IntC<4>{});
+  return f(IntC<8>{});
+}
+// fast path f(NJ, U, BIG): BIG slabs run 8 positions per thread and 2 or 1 samples per stage, the others NJ = plan.nj
+// (4, or 8 for any other value) and U as with_u
+template <class F> static int with_bnf(const BnFastPlan& plan, int u, F&& f) {
+  if (plan.big) return u == 2 ? f(IntC<8>{}, IntC<2>{}, std::true_type{}) : f(IntC<8>{}, IntC<1>{}, std::true_type{});
+  return with_u(u, [&](auto U) {
+    return plan.nj == 4 ? f(IntC<4>{}, U, std::false_type{}) : f(IntC<8>{}, U, std::false_type{});
+  });
+}
 
-// U (samples per pipeline stage) is a launch-time choice among the compiled instantiations
-#define DSTD_BN_CASE(kern, NJ_, u, grid, threads, smem, st, ...)                     \
-  do {                                                                                \
-    switch (u) {                                                                      \
-      case 4:                                                                         \
-        prefer_smem_carveout((const void*)kern<NJ_, 4>, true);                        \
-        kern<NJ_, 4><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
-        break;                                                                        \
-      case 2:                                                                         \
-        prefer_smem_carveout((const void*)kern<NJ_, 2>, true);                        \
-        kern<NJ_, 2><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
-        break;                                                                        \
-      default:                                                                        \
-        prefer_smem_carveout((const void*)kern<NJ_, 1>, true);                        \
-        kern<NJ_, 1><<<grid, threads, smem, st>>>(__VA_ARGS__);                       \
-        break;                                                                        \
-    }                                                                                 \
-  } while (0)
-#define DSTD_BN_DISPATCH_U(kern, nj, u, grid, threads, smem, st, ...)                \
-  do {                                                                                \
-    switch (nj) {                                                                     \
-      case 1: DSTD_BN_CASE(kern, 1, u, grid, threads, smem, st, __VA_ARGS__); break;  \
-      case 2: DSTD_BN_CASE(kern, 2, u, grid, threads, smem, st, __VA_ARGS__); break;  \
-      case 4: DSTD_BN_CASE(kern, 4, u, grid, threads, smem, st, __VA_ARGS__); break;  \
-      default: DSTD_BN_CASE(kern, 8, u, grid, threads, smem, st, __VA_ARGS__); break; \
-    }                                                                                 \
-  } while (0)
-
-// V > 32: the kernel's _wide_ twin
-#define DSTD_BN_DISPATCH_UW(kern, wide, nj, u, grid, threads, smem, st, ...)         \
-  do {                                                                                \
-    if (wide) DSTD_BN_DISPATCH_U(kern##_wide_kernel, nj, u, grid, threads, smem, st, __VA_ARGS__); \
-    else DSTD_BN_DISPATCH_U(kern##_kernel, nj, u, grid, threads, smem, st, __VA_ARGS__);           \
-  } while (0)
-
-#define DSTD_BN_DISPATCH(kern, nj, grid, threads, smem, st, q)          \
-  do {                                                                  \
-    switch (nj) {                                                       \
-      case 1: kern<1><<<grid, threads, smem, st>>>(q); break;           \
-      case 2: kern<2><<<grid, threads, smem, st>>>(q); break;           \
-      case 4: kern<4><<<grid, threads, smem, st>>>(q); break;           \
-      default: kern<8><<<grid, threads, smem, st>>>(q); break;          \
-    }                                                                   \
-  } while (0)
+// one launch of a streaming pass: the largest shared-memory carve-out for the kernel, then the launch
+template <class... P, class... A>
+static int bn_launch(void (*kernel)(P...), dim3 grid, int threads, size_t smem, cudaStream_t st, const char* name,
+                     const A&... args) {
+  prefer_smem_carveout((const void*)kernel, true);
+  kernel<<<grid, threads, smem, st>>>(args...);
+  count_launch();
+  DSTD_LAUNCH_CHECK(name);
+  return DSTD_OK;
+}
 
 }  // namespace dstd
 
@@ -1663,12 +1587,12 @@ static int bn_fwd_setup(const dstd_bn_act_fwd_args* a, const Switches& sw, BnFwd
 static int bn_fwd_stats(const BnFwdP& q, cudaStream_t st) {
   const BnGeom g = bn_geom(q.T, q.V);
   const size_t smem = 2 * (size_t)q.T * q.V * sizeof(float);
-  if (q.T * q.V > BN_MAXJ * BN_THREADS_MAX) {
-    prefer_smem_carveout((const void*)bn_stats_big_kernel, true);
-    bn_stats_big_kernel<<<dim3(q.C, q.S), g.threads, smem, st>>>(q);
-  } else {
-    DSTD_BN_DISPATCH(bn_stats_kernel, g.nj, dim3(q.C, q.S), g.threads, smem, st, q);
-  }
+  if (q.T * q.V > BN_MAXJ * BN_THREADS_MAX)
+    return bn_launch(bn_stats_big_kernel, dim3(q.C, q.S), g.threads, smem, st, "bn_stats", q);
+  with_nj(g.nj, [&](auto NJ) {
+    bn_stats_kernel<NJ><<<dim3(q.C, q.S), g.threads, smem, st>>>(q);
+    return 0;
+  });
   count_launch();
   DSTD_LAUNCH_CHECK("bn_stats");
   return DSTD_OK;
@@ -1684,27 +1608,21 @@ static int bn_fwd_apply(const BnFwdP& q, const Switches& sw, cudaStream_t st) {
     const dim3 grid(q.C / fp.ch, q.S);
     const size_t smem = (size_t)2 * nst * fu * fp.ch * tvb;
     int* err = device_error_word();
-#define DSTD_K_APPLY_R(NJ_, U_, B_) bnf_apply_kernel<NJ_, U_, true, B_>
-#define DSTD_K_APPLY(NJ_, U_, B_) bnf_apply_kernel<NJ_, U_, false, B_>
-#define DSTD_K_APPLY_R_W(NJ_, U_, B_) bnf_apply_wide_kernel<NJ_, U_, true, B_>
-#define DSTD_K_APPLY_W(NJ_, U_, B_) bnf_apply_wide_kernel<NJ_, U_, false, B_>
-    if (q.r.p) DSTD_BNF(DSTD_K_APPLY_R, fp, fu, grid, fp.threads, smem, st, q, fp.ch, err);
-    else DSTD_BNF(DSTD_K_APPLY, fp, fu, grid, fp.threads, smem, st, q, fp.ch, err);
-#undef DSTD_K_APPLY_R
-#undef DSTD_K_APPLY
-#undef DSTD_K_APPLY_R_W
-#undef DSTD_K_APPLY_W
-    count_launch();
-    DSTD_LAUNCH_CHECK("bnf_apply");
-    return DSTD_OK;
+    return with_bnf(fp, fu, [&](auto NJ, auto U, auto BIG) {
+      const auto k = q.r.p ? (fp.wide ? bnf_apply_wide_kernel<NJ, U, true, BIG> : bnf_apply_kernel<NJ, U, true, BIG>)
+                           : (fp.wide ? bnf_apply_wide_kernel<NJ, U, false, BIG> : bnf_apply_kernel<NJ, U, false, BIG>);
+      return bn_launch(k, grid, fp.threads, smem, st, "bnf_apply", q, fp.ch, err);
+    });
   }
   const BnGeom g = bn_geom(q.T, q.V);
   const int u = bn_pick_u(tvb, 2 * nst, 4, BN_SMEM_BUDGET);
   const size_t smu = (size_t)2 * nst * u * tvb;
-  DSTD_BN_DISPATCH_UW(bn_apply, q.V > 32, g.nj, u, dim3(q.C, q.S), g.threads, smu, st, q);
-  count_launch();
-  DSTD_LAUNCH_CHECK("bn_apply");
-  return DSTD_OK;
+  return with_nj(g.nj, [&](auto NJ) {
+    return with_u(u, [&](auto U) {
+      const auto k = q.V > 32 ? bn_apply_wide_kernel<NJ, U> : bn_apply_kernel<NJ, U>;
+      return bn_launch(k, dim3(q.C, q.S), g.threads, smu, st, "bn_apply", q);
+    });
+  });
 }
 
 extern "C" int dstd_bn_act_forward(const dstd_bn_act_fwd_args* a, dstd_stream_t stream) {
@@ -1812,7 +1730,7 @@ static BnBwdPlan bn_bwd_plan(const BnBwdP& q, const Switches& sw) {
   p.nst2 = p.nst + (p.add ? 1 : 0);                    // pass 2 also stages gr_add
   const bool has_gr = q.gr.p != nullptr;
   const bool combo = p.use_r ? has_gr : (!has_gr && !p.add);     // the instantiations the model uses
-  const bool gr_same = !has_gr || bnf_tfast(q.gr) == bnf_tfast(q.gy);
+  const bool gr_same = !has_gr || t_fastest(q.gr) == t_fastest(q.gy);
   p.fp = (combo && gr_same) ? bnf_plan(sw.bn_fast, q.C, q.T, q.V, q.mask, {&q.y, &q.r, &q.gout, &q.gy, &q.gr, &q.gadd})
                             : BnFastPlan{false, 0, 0, 0, false, false};
   p.u1 = p.fp.ok ? bnf_pick_u((size_t)p.fp.ch * tv, p.nst, p.fp.big, p.fp.wide) : 0;
@@ -1828,26 +1746,20 @@ static int bn_bwd_reduce(const BnBwdP& q, const BnBwdPlan& p, cudaStream_t st) {
   if (p.fast()) {
     const dim3 grid(q.C / p.fp.ch, q.S);
     int* err = device_error_word();
-#define DSTD_K_RED_R(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, true, B_>
-#define DSTD_K_RED(NJ_, U_, B_) bnf_bwd_reduce_kernel<NJ_, U_, false, B_>
-#define DSTD_K_RED_R_W(NJ_, U_, B_) bnf_bwd_reduce_wide_kernel<NJ_, U_, true, B_>
-#define DSTD_K_RED_W(NJ_, U_, B_) bnf_bwd_reduce_wide_kernel<NJ_, U_, false, B_>
-    if (p.use_r) DSTD_BNF(DSTD_K_RED_R, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
-    else DSTD_BNF(DSTD_K_RED, p.fp, p.u1, grid, p.fp.threads, (size_t)2 * p.nst * p.u1 * p.fp.ch * tv, st, q, p.fp.ch, err);
-#undef DSTD_K_RED_R
-#undef DSTD_K_RED
-#undef DSTD_K_RED_R_W
-#undef DSTD_K_RED_W
-    count_launch();
-    DSTD_LAUNCH_CHECK("bnf_bwd_reduce");
-    return DSTD_OK;
+    const size_t smem = (size_t)2 * p.nst * p.u1 * p.fp.ch * tv;
+    return with_bnf(p.fp, p.u1, [&](auto NJ, auto U, auto BIG) {
+      const auto k = p.use_r ? (p.fp.wide ? bnf_bwd_reduce_wide_kernel<NJ, U, true, BIG> : bnf_bwd_reduce_kernel<NJ, U, true, BIG>)
+                             : (p.fp.wide ? bnf_bwd_reduce_wide_kernel<NJ, U, false, BIG> : bnf_bwd_reduce_kernel<NJ, U, false, BIG>);
+      return bn_launch(k, grid, p.fp.threads, smem, st, "bnf_bwd_reduce", q, p.fp.ch, err);
+    });
   }
   size_t sm_red = (size_t)2 * p.nst * p.ub * tv;
   if (sm_red < 2 * tv) sm_red = 2 * tv;
-  DSTD_BN_DISPATCH_U(bn_bwd_reduce_kernel, p.g.nj, p.ub, dim3(q.C, q.S), p.g.threads, sm_red, st, q);   // any V
-  count_launch();
-  DSTD_LAUNCH_CHECK("bn_bwd_reduce");
-  return DSTD_OK;
+  return with_nj(p.g.nj, [&](auto NJ) {   // any V
+    return with_u(p.ub, [&](auto U) {
+      return bn_launch(bn_bwd_reduce_kernel<NJ, U>, dim3(q.C, q.S), p.g.threads, sm_red, st, "bn_bwd_reduce", q);
+    });
+  });
 }
 
 // pass 2 (gy, gr; the plain call also the parameter gradients).  all == nullptr: the plain kernels, k1 / k2 from this
@@ -1859,56 +1771,41 @@ static int bn_bwd_apply(const BnBwdP& q, const BnBwdPlan& p, const double* all, 
     int* err = device_error_word();
     const int np = (int)(grid.x * grid.y);
     const size_t smem2 = (size_t)2 * p.nst2 * p.u2 * p.fp.ch * tv;
-    if (!all) {
-#define DSTD_K_APP_RA(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, true, B_>
-#define DSTD_K_APP_R(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, true, true, false, B_>
-#define DSTD_K_APP(NJ_, U_, B_) bnf_bwd_apply_kernel<NJ_, U_, false, false, false, B_>
-#define DSTD_K_APP_RA_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, true, true, true, B_>
-#define DSTD_K_APP_R_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, true, true, false, B_>
-#define DSTD_K_APP_W(NJ_, U_, B_) bnf_bwd_apply_wide_kernel<NJ_, U_, false, false, false, B_>
-      if (p.use_r && p.add) DSTD_BNF(DSTD_K_APP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
-      else if (p.use_r) DSTD_BNF(DSTD_K_APP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
-      else DSTD_BNF(DSTD_K_APP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, np, err);
-#undef DSTD_K_APP_RA
-#undef DSTD_K_APP_R
-#undef DSTD_K_APP
-#undef DSTD_K_APP_RA_W
-#undef DSTD_K_APP_R_W
-#undef DSTD_K_APP_W
-    } else {
-#define DSTD_K_SAPP_RA(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, true, B_>
-#define DSTD_K_SAPP_R(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, true, true, false, B_>
-#define DSTD_K_SAPP(NJ_, U_, B_) bnf_bwd_apply_sync_kernel<NJ_, U_, false, false, false, B_>
-#define DSTD_K_SAPP_RA_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, true, true, true, B_>
-#define DSTD_K_SAPP_R_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, true, true, false, B_>
-#define DSTD_K_SAPP_W(NJ_, U_, B_) bnf_bwd_apply_sync_wide_kernel<NJ_, U_, false, false, false, B_>
-      if (p.use_r && p.add) DSTD_BNF(DSTD_K_SAPP_RA, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
-      else if (p.use_r) DSTD_BNF(DSTD_K_SAPP_R, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
-      else DSTD_BNF(DSTD_K_SAPP, p.fp, p.u2, grid, p.fp.threads, smem2, st, q, p.fp.ch, err, all, world);
-#undef DSTD_K_SAPP_RA
-#undef DSTD_K_SAPP_R
-#undef DSTD_K_SAPP
-#undef DSTD_K_SAPP_RA_W
-#undef DSTD_K_SAPP_R_W
-#undef DSTD_K_SAPP_W
-    }
-    count_launch();
-    DSTD_LAUNCH_CHECK("bnf_bwd_apply");
-    return DSTD_OK;
+    // the instantiations the model uses: (USE_R, HAS_GR, ADD) = (1, 1, 1), (1, 1, 0) or (0, 0, 0)
+    return with_bnf(p.fp, p.u2, [&](auto NJ, auto U, auto BIG) {
+      if (!all) {
+        const auto k = p.use_r && p.add ? (p.fp.wide ? bnf_bwd_apply_wide_kernel<NJ, U, true, true, true, BIG>
+                                                     : bnf_bwd_apply_kernel<NJ, U, true, true, true, BIG>)
+                       : p.use_r        ? (p.fp.wide ? bnf_bwd_apply_wide_kernel<NJ, U, true, true, false, BIG>
+                                                     : bnf_bwd_apply_kernel<NJ, U, true, true, false, BIG>)
+                                        : (p.fp.wide ? bnf_bwd_apply_wide_kernel<NJ, U, false, false, false, BIG>
+                                                     : bnf_bwd_apply_kernel<NJ, U, false, false, false, BIG>);
+        return bn_launch(k, grid, p.fp.threads, smem2, st, "bnf_bwd_apply", q, p.fp.ch, np, err);
+      }
+      const auto k = p.use_r && p.add ? (p.fp.wide ? bnf_bwd_apply_sync_wide_kernel<NJ, U, true, true, true, BIG>
+                                                   : bnf_bwd_apply_sync_kernel<NJ, U, true, true, true, BIG>)
+                     : p.use_r        ? (p.fp.wide ? bnf_bwd_apply_sync_wide_kernel<NJ, U, true, true, false, BIG>
+                                                   : bnf_bwd_apply_sync_kernel<NJ, U, true, true, false, BIG>)
+                                      : (p.fp.wide ? bnf_bwd_apply_sync_wide_kernel<NJ, U, false, false, false, BIG>
+                                                   : bnf_bwd_apply_sync_kernel<NJ, U, false, false, false, BIG>);
+      return bn_launch(k, grid, p.fp.threads, smem2, st, "bnf_bwd_apply", q, p.fp.ch, err, all, world);
+    });
   }
   const size_t sm2 = (size_t)(2 * p.nst2 + 1) * p.ub2 * tv;
   const dim3 grid(q.C, q.S);
-  const bool wide = q.V > 32;
-  if (!all) {
-    if (q.gadd.p) DSTD_BN_DISPATCH_UW(bn_bwd_apply_add, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
-    else DSTD_BN_DISPATCH_UW(bn_bwd_apply, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q);
-  } else {
-    if (q.gadd.p) DSTD_BN_DISPATCH_UW(bn_bwd_apply_add_sync, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
-    else DSTD_BN_DISPATCH_UW(bn_bwd_apply_sync, wide, p.g.nj, p.ub2, grid, p.g.threads, sm2, st, q, all, world);
-  }
-  count_launch();
-  DSTD_LAUNCH_CHECK("bn_bwd_apply");
-  return DSTD_OK;
+  const bool wide = q.V > 32, add = q.gadd.p != nullptr;
+  return with_nj(p.g.nj, [&](auto NJ) {
+    return with_u(p.ub2, [&](auto U) {
+      if (!all) {
+        const auto k = add ? (wide ? bn_bwd_apply_add_wide_kernel<NJ, U> : bn_bwd_apply_add_kernel<NJ, U>)
+                           : (wide ? bn_bwd_apply_wide_kernel<NJ, U> : bn_bwd_apply_kernel<NJ, U>);
+        return bn_launch(k, grid, p.g.threads, sm2, st, "bn_bwd_apply", q);
+      }
+      const auto k = add ? (wide ? bn_bwd_apply_add_sync_wide_kernel<NJ, U> : bn_bwd_apply_add_sync_kernel<NJ, U>)
+                         : (wide ? bn_bwd_apply_sync_wide_kernel<NJ, U> : bn_bwd_apply_sync_kernel<NJ, U>);
+      return bn_launch(k, grid, p.g.threads, sm2, st, "bn_bwd_apply", q, all, world);
+    });
+  });
 }
 
 extern "C" int dstd_bn_act_backward(const dstd_bn_act_bwd_args* a, dstd_stream_t stream) {

@@ -5,10 +5,12 @@ parity tests and a (P, K) sweep across the 40-wide specialised tiles, under the 
 switch setting (set in-process: the library reads them per call).  The sizes and the xa decision do not depend on the
 switches, so a caller that sized its buffers before flipping one still hands over enough workspace.
 
-On the GPU: the kernels one forward + backward launches, per shape and switch setting.
+On the GPU: the kernels one forward + backward launches, per shape and switch setting; and the BatchNorm kernels
+(with template arguments, grid, block and dynamic shared memory) of the BN parity cases, with the fast path on and off.
 
-TABLE and KERNELS hold what the library did before these decisions were moved into one plan (api.cu gc_plan); a change
-to either is a change of what the library computes, allocates or launches."""
+TABLE and KERNELS hold what the library did before these decisions were moved into one plan (api.cu gc_plan), and
+BN_LAUNCHES what it did before the BatchNorm dispatch macros became templates (bn_act.cu with_u / with_nj / with_bnf);
+a change to any of them is a change of what the library computes, allocates or launches."""
 import pytest
 import torch
 
@@ -273,3 +275,974 @@ def test_kernel_paths(setting, monkeypatch):
     for i, case in enumerate(KERNEL_CASES):
         dflt, over = KERNELS[i]
         assert launched_kernels(case) == over.get(setting, dflt), (case, setting)
+
+
+# ---- GPU: the BatchNorm kernels each bn_act call launches, with their template arguments and launch geometry.  The
+# parity tests pass whichever compiled U or twin a dispatch picks; this table does not.
+def _bn_cases():
+    from tests import test_custom_skeleton as cs
+    cases = {}
+    for src, rows, full in (("parity", gp.BN_CASES, True), ("parity_fast", gp.BN_FAST_CASES, False),
+                            ("skeleton", cs.BN_CASES, True), ("skeleton_fast", cs.BN_FAST_CASES, False)):
+        for i, row in enumerate(rows):
+            if not full:   # n, c, t, v, y_order, r_order, out_order, prelu, training -> the full form
+                n, c, t, v, yo, ro, oo, use_prelu, training = row
+                row = (n, c, t, v, yo, ro, oo, False, use_prelu, False, training)
+            cases[f"{src}/{i}"] = row
+    return cases
+
+
+BN_CASES = _bn_cases()
+BN_SYNC_CASES = ("parity/0", "skeleton/2")   # generic and fast (DSTD_BN_FAST=0 / 1), V <= 32 and V > 32
+
+
+def _bn_launch_log(fn):
+    """Library kernels `fn` launches, in order: 'name<template args> grid block smem', names without 'dstd::'."""
+    import json
+    import tempfile
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    with tempfile.TemporaryDirectory() as d:
+        path = f"{d}/trace.json"
+        prof.export_chrome_trace(path)
+        with open(path) as f:
+            evs = json.load(f)["traceEvents"]
+    evs = sorted((e for e in evs if e.get("cat") == "kernel" and "dstd::" in e["name"]), key=lambda e: e["ts"])
+    out = []
+    for e in evs:
+        a = e.get("args", {})
+        geom = "x".join(map(str, a.get("grid", ()))), "x".join(map(str, a.get("block", ()))), a.get("shared memory")
+        out.append(e["name"].removeprefix("void ").removeprefix("dstd::").split("(")[0] + " %s %s %s" % geom)
+    return out
+
+
+def _bn_inputs(case):
+    from dstd_gcn_b200.ops import _out_like
+    n, c, t, v, yo, ro, out_order, vc, use_prelu, use_mask, training = case
+    g = torch.Generator().manual_seed(n * 13 + c + v)
+    d = dict(y=gp.to_dev(gp._ordered(g, n, c, t, v, yo) * 2.0 + 3.0),
+             r=gp.to_dev(gp._ordered(g, n, c, t, v, ro)) if ro else None,
+             gamma=gp.to_dev(gp.rnd((c * v,), g, 0.5) + 1.0), beta=gp.to_dev(gp.rnd((c * v,), g, 0.5)),
+             rm=torch.zeros(c * v, device=gp.DEV), rv=torch.ones(c * v, device=gp.DEV),
+             nbt=torch.zeros((), dtype=torch.int64, device=gp.DEV),
+             prelu=gp.to_dev(torch.tensor([0.25], dtype=torch.float64)) if use_prelu else None,
+             mask=gp.to_dev((torch.rand((n, c, t, v), generator=g) > 0.1).double() / 0.9) if use_mask else None)
+    d["out_like"] = _out_like(d["y"], out_order) if out_order else None
+    return d
+
+
+def bn_launches(case):
+    """Kernels of one forward, one backward and, with a residual, one backward with gr_add."""
+    n, c, t, v, yo, ro, out_order, vc, use_prelu, use_mask, training = case
+    be, d = gp.cuda_backend(), _bn_inputs(case)
+    y, r, prelu, mask = d["y"], d["r"], d["prelu"], d["mask"]
+    fwd = lambda: be.bn_act_forward(y, r, d["gamma"], d["beta"], d["rm"], d["rv"], d["nbt"] if training else None,
+                                    prelu, mask, vc, training, 1e-5, 0.1, d["out_like"])
+    out, mean, istd = fwd()
+    gout = torch.randn_like(out)
+    bwd = lambda gadd=None: be.bn_act_backward(y, r, gout, d["gamma"], d["beta"], prelu, mask, mean, istd, vc,
+                                               training, r is not None, gadd)
+    log = {"fwd": _bn_launch_log(fwd), "bwd": _bn_launch_log(bwd)}
+    if r is not None:
+        gadd = torch.randn_like(out)
+        log["bwd_add"] = _bn_launch_log(lambda: bwd(gadd))
+    return log
+
+
+def bn_sync_launches(case):
+    """Kernels of the four phases of a synchronised BN call on one rank."""
+    n, c, t, v, yo, ro, out_order, vc, use_prelu, use_mask, training = case
+    be, d = gp.cuda_backend(), _bn_inputs(case)
+    y, r, prelu, mask = d["y"], d["r"], d["prelu"], d["mask"]
+    res = {}
+    log = {"fwd_local": _bn_launch_log(lambda: res.update(rows=be.bn_act_forward_local(y, vc)))}
+    log["fwd_global"] = _bn_launch_log(lambda: res.update(fwd=be.bn_act_forward_global(
+        y, r, d["gamma"], d["beta"], d["rm"], d["rv"], d["nbt"], prelu, mask, vc, 1e-5, 0.1, res["rows"],
+        d["out_like"])))
+    out, mean, istd = res["fwd"]
+    gout = torch.randn_like(out)
+    log["bwd_local"] = _bn_launch_log(lambda: res.update(bwd=be.bn_act_backward_local(
+        y, r, gout, d["gamma"], d["beta"], prelu, mask, mean, istd, vc, r is not None)))
+    rows, gy, gr = res["bwd"][3:]
+    log["bwd_global"] = _bn_launch_log(lambda: be.bn_act_backward_global(
+        y, r, gout, d["gamma"], d["beta"], prelu, mask, mean, istd, vc, rows, gy, gr))
+    return log
+
+
+REFUSED = "refused"   # T*V above the generic kernels' limit with the fast path off: the call raises
+
+# case id (BN_CASES, or sync/<id> of BN_SYNC_CASES): {'1': the launches of each call with DSTD_BN_FAST=1, '0': the
+# same with DSTD_BN_FAST=0 where they differ}.  A launch: 'kernel<template args> grid block shared-memory-bytes' (static
+# + dynamic, as the profiler reports it).
+BN_LAUNCHES = {
+    'parity/0': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 16x1x1 416x1x1 6160',
+                'bnf_apply_kernel<4, 4, true, false> 8x1x1 416x1x1 101136',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 2, true, false> 8x1x1 416x1x1 76112',
+                'bnf_bwd_apply_kernel<4, 2, true, true, false, false> 8x1x1 416x1x1 78672',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<4, 2, true, false> 8x1x1 416x1x1 76112',
+                'bnf_bwd_apply_kernel<4, 2, true, true, true, false> 8x1x1 416x1x1 103312',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 16x1x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 16x1x1 416x1x1 50048',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 16x1x1 416x1x1 74048',
+                'bn_bwd_apply_kernel<2, 4> 16x1x1 416x1x1 86880',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 16x1x1 416x1x1 74048',
+                'bn_bwd_apply_add_kernel<2, 4> 16x1x1 416x1x1 111520',
+            ],
+        },
+    },
+    'parity/1': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 16x1x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 16x1x1 416x1x1 25408',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 16x1x1 416x1x1 49408',
+                'bn_bwd_apply_kernel<2, 4> 16x1x1 416x1x1 62240',
+            ],
+        },
+    },
+    'parity/2': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<1> 8x1x1 256x1x1 2000',
+                'bnf_apply_kernel<4, 4, false, false> 4x1x1 128x1x1 18576',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, false, false> 4x1x1 128x1x1 34192',
+                'bnf_bwd_apply_kernel<4, 4, false, false, false, false> 4x1x1 128x1x1 36752',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<1> 8x1x1 256x1x1 2000',
+                'bn_apply_kernel<1, 4> 8x1x1 256x1x1 8768',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<1, 4> 8x1x1 256x1x1 16128',
+                'bn_bwd_apply_kernel<1, 4> 8x1x1 256x1x1 20640',
+            ],
+        },
+    },
+    'parity/3': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bnf_apply_kernel<4, 4, true, false> 8x1x1 256x1x1 61456',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, true, false> 8x1x1 256x1x1 90512',
+                'bnf_bwd_apply_kernel<4, 4, true, true, false, false> 8x1x1 256x1x1 93072',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<4, 4, true, false> 8x1x1 256x1x1 90512',
+                'bnf_bwd_apply_kernel<4, 2, true, true, true, false> 8x1x1 256x1x1 63632',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bn_apply_kernel<2, 4> 8x1x1 480x1x1 59648',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 480x1x1 88448',
+                'bn_bwd_apply_kernel<2, 4> 8x1x1 480x1x1 103680',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 480x1x1 88448',
+                'bn_bwd_apply_add_kernel<2, 2> 8x1x1 480x1x1 66880',
+            ],
+        },
+    },
+    'parity/4': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 64x2x1 416x1x1 6160',
+                'bnf_apply_kernel<4, 4, false, false> 32x2x1 416x1x1 51856',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, false, false> 32x2x1 416x1x1 100752',
+                'bnf_bwd_apply_kernel<4, 4, false, false, false, false> 32x2x1 416x1x1 103312',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 64x2x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 64x2x1 416x1x1 25408',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 64x2x1 416x1x1 49408',
+                'bn_bwd_apply_kernel<2, 4> 64x2x1 416x1x1 62240',
+            ],
+        },
+    },
+    'parity/5': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 3x1x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 3x1x1 416x1x1 50048',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 3x1x1 416x1x1 74048',
+                'bn_bwd_apply_kernel<2, 4> 3x1x1 416x1x1 86880',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 3x1x1 416x1x1 74048',
+                'bn_bwd_apply_add_kernel<2, 4> 3x1x1 416x1x1 111520',
+            ],
+        },
+    },
+    'parity_fast/0': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x2x1 416x1x1 6160',
+                'bnf_apply_kernel<4, 4, true, false> 4x2x1 416x1x1 101136',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 2, true, false> 4x2x1 416x1x1 76112',
+                'bnf_bwd_apply_kernel<4, 2, true, true, false, false> 4x2x1 416x1x1 78672',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<4, 2, true, false> 4x2x1 416x1x1 76112',
+                'bnf_bwd_apply_kernel<4, 2, true, true, true, false> 4x2x1 416x1x1 103312',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x2x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 8x2x1 416x1x1 50048',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 8x2x1 416x1x1 74048',
+                'bn_bwd_apply_kernel<2, 4> 8x2x1 416x1x1 86880',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 8x2x1 416x1x1 74048',
+                'bn_bwd_apply_add_kernel<2, 4> 8x2x1 416x1x1 111520',
+            ],
+        },
+    },
+    'parity_fast/1': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x1x1 416x1x1 6160',
+                'bnf_apply_kernel<4, 4, false, false> 4x1x1 416x1x1 51856',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, false, false> 4x1x1 416x1x1 100752',
+                'bnf_bwd_apply_kernel<4, 4, false, false, false, false> 4x1x1 416x1x1 103312',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x1x1 416x1x1 6160',
+                'bn_apply_kernel<2, 4> 8x1x1 416x1x1 25408',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 416x1x1 49408',
+                'bn_bwd_apply_kernel<2, 4> 8x1x1 416x1x1 62240',
+            ],
+        },
+    },
+    'parity_fast/2': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 4x1x1 480x1x1 7360',
+                'bnf_apply_kernel<4, 4, true, false> 4x1x1 256x1x1 61456',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, true, false> 4x1x1 256x1x1 90512',
+                'bnf_bwd_apply_kernel<4, 4, true, true, false, false> 4x1x1 256x1x1 93072',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<4, 4, true, false> 4x1x1 256x1x1 90512',
+                'bnf_bwd_apply_kernel<4, 2, true, true, true, false> 4x1x1 256x1x1 63632',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 4x1x1 480x1x1 7360',
+                'bn_apply_kernel<2, 4> 4x1x1 480x1x1 59648',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 4x1x1 480x1x1 88448',
+                'bn_bwd_apply_kernel<2, 4> 4x1x1 480x1x1 103680',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 4x1x1 480x1x1 88448',
+                'bn_bwd_apply_add_kernel<2, 2> 4x1x1 480x1x1 66880',
+            ],
+        },
+    },
+    'parity_fast/3': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x1x1 448x1x1 7000',
+                'bnf_apply_kernel<8, 2, true, false> 2x1x1 448x1x1 114576',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<8, 1, true, false> 2x1x1 448x1x1 86192',
+                'bnf_bwd_apply_kernel<8, 1, true, true, false, false> 2x1x1 448x1x1 88752',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<8, 1, true, false> 2x1x1 448x1x1 86192',
+                'bnf_bwd_apply_kernel<8, 1, true, true, true, false> 2x1x1 448x1x1 116752',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<2> 8x1x1 448x1x1 7000',
+                'bn_apply_kernel<2, 4> 8x1x1 448x1x1 56768',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 448x1x1 84128',
+                'bn_bwd_apply_kernel<2, 4> 8x1x1 448x1x1 98640',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 448x1x1 84128',
+                'bn_bwd_apply_add_kernel<2, 2> 8x1x1 448x1x1 63640',
+            ],
+        },
+    },
+    'parity_fast/4': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bnf_apply_kernel<8, 4, false, false> 2x1x1 448x1x1 114576',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<8, 2, false, false> 2x1x1 448x1x1 114192',
+                'bnf_bwd_apply_kernel<8, 2, false, false, false, false> 2x1x1 448x1x1 116752',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bn_apply_kernel<2, 4> 8x1x1 448x1x1 28768',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<2, 4> 8x1x1 448x1x1 56128',
+                'bn_bwd_apply_kernel<2, 4> 8x1x1 448x1x1 70640',
+            ],
+        },
+    },
+    'parity_fast/5': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<1> 4x1x1 224x1x1 1760',
+                'bnf_apply_kernel<4, 4, false, false> 4x1x1 64x1x1 9616',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<4, 4, false, false> 4x1x1 64x1x1 16272',
+                'bnf_bwd_apply_kernel<4, 4, false, false, false, false> 4x1x1 64x1x1 18832',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<1> 4x1x1 224x1x1 1760',
+                'bn_apply_kernel<1, 4> 4x1x1 224x1x1 7808',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<1, 4> 4x1x1 224x1x1 14208',
+                'bn_bwd_apply_kernel<1, 4> 4x1x1 224x1x1 18240',
+            ],
+        },
+    },
+    'parity_fast/6': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 352x1x1 22000',
+                'bnf_apply_kernel<8, 2, true, true> 2x1x1 704x1x1 178576',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<8, 1, true, true> 2x1x1 704x1x1 134192',
+                'bnf_bwd_apply_kernel<8, 1, true, true, false, true> 2x1x1 704x1x1 136752',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_kernel<8, 1, true, true> 2x1x1 704x1x1 134192',
+                'bnf_bwd_apply_kernel<8, 1, true, true, true, true> 2x1x1 704x1x1 180752',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 352x1x1 22000',
+                'bn_apply_kernel<8, 2> 4x1x1 352x1x1 88768',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 352x1x1 66128',
+                'bn_bwd_apply_kernel<8, 1> 4x1x1 352x1x1 77640',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 352x1x1 66128',
+                'bn_bwd_apply_add_kernel<8, 1> 4x1x1 352x1x1 99640',
+            ],
+        },
+    },
+    'parity_fast/7': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 352x1x1 22000',
+                'bnf_apply_kernel<8, 2, false, true> 2x1x1 704x1x1 90576',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_kernel<8, 2, false, true> 2x1x1 704x1x1 178192',
+                'bnf_bwd_apply_kernel<8, 2, false, false, false, true> 2x1x1 704x1x1 180752',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 352x1x1 22000',
+                'bn_apply_kernel<8, 4> 4x1x1 352x1x1 88768',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 2> 4x1x1 352x1x1 88128',
+                'bn_bwd_apply_kernel<8, 2> 4x1x1 352x1x1 110640',
+            ],
+        },
+    },
+    'skeleton/0': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 320x1x1 9240',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 320x1x1 76992',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 320x1x1 55568',
+                'bn_bwd_apply_wide_kernel<4, 2> 8x1x1 320x1x1 66856',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 320x1x1 55568',
+                'bn_bwd_apply_add_wide_kernel<4, 2> 8x1x1 320x1x1 85336',
+            ],
+        },
+    },
+    'skeleton/1': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 352x1x1 45632',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 4> 8x1x1 352x1x1 85248',
+                'bn_bwd_apply_wide_kernel<4, 4> 8x1x1 352x1x1 108576',
+            ],
+        },
+    },
+    'skeleton/2': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bnf_apply_wide_kernel<8, 2, true, false> 4x1x1 352x1x1 95376',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 352x1x1 72176',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, false> 4x1x1 352x1x1 82416',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 352x1x1 72176',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, false> 4x1x1 352x1x1 103696',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 352x1x1 88192',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 352x1x1 63968',
+                'bn_bwd_apply_wide_kernel<4, 2> 8x1x1 352x1x1 76656',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 352x1x1 63968',
+                'bn_bwd_apply_add_wide_kernel<4, 2> 8x1x1 352x1x1 97936',
+            ],
+        },
+    },
+    'skeleton/3': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 16x2x1 352x1x1 10640',
+                'bnf_apply_wide_kernel<8, 4, false, false> 8x2x1 352x1x1 95376',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 2, false, false> 8x2x1 352x1x1 93456',
+                'bnf_bwd_apply_wide_kernel<8, 2, false, false, false, false> 8x2x1 352x1x1 103696',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<4> 16x2x1 352x1x1 10640',
+                'bn_apply_wide_kernel<4, 4> 16x2x1 352x1x1 45632',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 4> 16x2x1 352x1x1 85248',
+                'bn_bwd_apply_wide_kernel<4, 4> 16x2x1 352x1x1 108576',
+            ],
+        },
+    },
+    'skeleton/4': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 4x1x1 128x1x1 0',
+                'bn_apply_wide_kernel<4, 2> 8x1x1 512x1x1 64672',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 512x1x1 92528',
+                'bn_bwd_apply_wide_kernel<4, 2> 8x1x1 512x1x1 109976',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 512x1x1 92528',
+                'bn_bwd_apply_add_wide_kernel<4, 1> 8x1x1 512x1x1 71476',
+            ],
+        },
+    },
+    'skeleton/5': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 288x1x1 17920',
+                'bnf_apply_wide_kernel<8, 2, true, false> 4x1x1 288x1x1 81936',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 288x1x1 62096',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, false> 4x1x1 288x1x1 72336',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 288x1x1 62096',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, false> 4x1x1 288x1x1 90256',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 288x1x1 17920',
+                'bn_apply_wide_kernel<8, 2> 4x1x1 288x1x1 74752',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 288x1x1 53888',
+                'bn_bwd_apply_wide_kernel<8, 1> 4x1x1 288x1x1 64896',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 288x1x1 53888',
+                'bn_bwd_apply_add_wide_kernel<8, 1> 4x1x1 288x1x1 82816',
+            ],
+        },
+    },
+    'skeleton/6': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bnf_apply_wide_kernel<8, 4, false, false> 4x1x1 288x1x1 81936',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 2, false, false> 4x1x1 288x1x1 80016',
+                'bnf_bwd_apply_wide_kernel<8, 2, false, false, false, false> 4x1x1 288x1x1 90256',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_eval_stats_kernel 2x1x1 128x1x1 0',
+                'bn_apply_wide_kernel<8, 4> 4x1x1 288x1x1 74752',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 2> 4x1x1 288x1x1 71808',
+                'bn_bwd_apply_wide_kernel<8, 2> 4x1x1 288x1x1 91776',
+            ],
+        },
+    },
+    'skeleton/7': {
+        '1': {
+            'fwd': [
+                'bn_stats_big_kernel 4x1x1 576x1x1 35840',
+                'bnf_apply_wide_kernel<8, 2, true, true> 4x1x1 576x1x1 153616',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, true> 4x1x1 576x1x1 115856',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, true> 4x1x1 576x1x1 126096',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, true> 4x1x1 576x1x1 115856',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, true> 4x1x1 576x1x1 161936',
+            ],
+        },
+        '0': REFUSED,
+    },
+    'skeleton/8': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<8> 4x1x1 512x1x1 32768',
+                'bn_apply_wide_kernel<8, 2> 4x1x1 512x1x1 68608',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 512x1x1 65664',
+                'bn_bwd_apply_wide_kernel<8, 1> 4x1x1 512x1x1 84096',
+            ],
+        },
+    },
+    'skeleton/9': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 4x1x1 128x1x1 0',
+                'bnf_apply_wide_kernel<8, 1, true, false> 4x1x1 512x1x1 75792',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 512x1x1 106640',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, false> 4x1x1 512x1x1 116880',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 512x1x1 98432',
+                'bn_bwd_apply_add_wide_kernel<8, 1> 4x1x1 512x1x1 149632',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_eval_stats_kernel 4x1x1 128x1x1 0',
+                'bn_apply_wide_kernel<8, 1> 4x1x1 512x1x1 68608',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 512x1x1 98432',
+                'bn_bwd_apply_wide_kernel<8, 1> 4x1x1 512x1x1 116864',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<8, 1> 4x1x1 512x1x1 98432',
+                'bn_bwd_apply_add_wide_kernel<8, 1> 4x1x1 512x1x1 149632',
+            ],
+        },
+    },
+    'skeleton/10': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<1> 3x1x1 224x1x1 1600',
+                'bnf_apply_wide_kernel<4, 4, true, false> 3x1x1 128x1x1 23056',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<4, 4, true, false> 3x1x1 128x1x1 27536',
+                'bnf_bwd_apply_wide_kernel<4, 4, true, true, false, false> 3x1x1 128x1x1 37776',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<4, 4, true, false> 3x1x1 128x1x1 27536',
+                'bnf_bwd_apply_wide_kernel<4, 4, true, true, true, false> 3x1x1 128x1x1 44176',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<1> 3x1x1 224x1x1 1600',
+                'bn_apply_wide_kernel<1, 4> 3x1x1 224x1x1 15872',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<1, 4> 3x1x1 224x1x1 19328',
+                'bn_bwd_apply_wide_kernel<1, 4> 3x1x1 224x1x1 24576',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<1, 4> 3x1x1 224x1x1 19328',
+                'bn_bwd_apply_add_wide_kernel<1, 4> 3x1x1 224x1x1 30976',
+            ],
+        },
+    },
+    'skeleton_fast/0': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x2x1 352x1x1 10640',
+                'bnf_apply_wide_kernel<8, 2, true, false> 4x2x1 352x1x1 95376',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x2x1 352x1x1 72176',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, false> 4x2x1 352x1x1 82416',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x2x1 352x1x1 72176',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, false> 4x2x1 352x1x1 103696',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x2x1 352x1x1 10640',
+                'bn_apply_wide_kernel<4, 4> 8x2x1 352x1x1 88192',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 2> 8x2x1 352x1x1 63968',
+                'bn_bwd_apply_wide_kernel<4, 2> 8x2x1 352x1x1 76656',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<4, 2> 8x2x1 352x1x1 63968',
+                'bn_bwd_apply_add_wide_kernel<4, 2> 8x2x1 352x1x1 97936',
+            ],
+        },
+    },
+    'skeleton_fast/1': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bnf_apply_wide_kernel<8, 4, false, false> 4x1x1 352x1x1 95376',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 2, false, false> 4x1x1 352x1x1 93456',
+                'bnf_bwd_apply_wide_kernel<8, 2, false, false, false, false> 4x1x1 352x1x1 103696',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 352x1x1 45632',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 4> 8x1x1 352x1x1 85248',
+                'bn_bwd_apply_wide_kernel<4, 4> 8x1x1 352x1x1 108576',
+            ],
+        },
+    },
+    'skeleton_fast/2': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<8> 8x1x1 288x1x1 17920',
+                'bnf_apply_wide_kernel<8, 2, true, false> 8x1x1 288x1x1 81936',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 8x1x1 288x1x1 62096',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, false> 8x1x1 288x1x1 72336',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 8x1x1 288x1x1 62096',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, false> 8x1x1 288x1x1 90256',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<8> 8x1x1 288x1x1 17920',
+                'bn_apply_wide_kernel<8, 2> 8x1x1 288x1x1 74752',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 1> 8x1x1 288x1x1 53888',
+                'bn_bwd_apply_wide_kernel<8, 1> 8x1x1 288x1x1 64896',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<8, 1> 8x1x1 288x1x1 53888',
+                'bn_bwd_apply_add_wide_kernel<8, 1> 8x1x1 288x1x1 82816',
+            ],
+        },
+    },
+    'skeleton_fast/3': {
+        '1': {
+            'fwd': [
+                'bn_eval_stats_kernel 4x1x1 128x1x1 0',
+                'bnf_apply_wide_kernel<8, 4, false, false> 8x1x1 288x1x1 81936',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 2, false, false> 8x1x1 288x1x1 80016',
+                'bnf_bwd_apply_wide_kernel<8, 2, false, false, false, false> 8x1x1 288x1x1 90256',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_eval_stats_kernel 4x1x1 128x1x1 0',
+                'bn_apply_wide_kernel<8, 4> 8x1x1 288x1x1 74752',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<8, 2> 8x1x1 288x1x1 71808',
+                'bn_bwd_apply_wide_kernel<8, 2> 8x1x1 288x1x1 91776',
+            ],
+        },
+    },
+    'skeleton_fast/4': {
+        '1': {
+            'fwd': [
+                'bn_stats_big_kernel 4x1x1 576x1x1 35840',
+                'bnf_apply_wide_kernel<8, 2, true, true> 4x1x1 576x1x1 153616',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, true> 4x1x1 576x1x1 115856',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, false, true> 4x1x1 576x1x1 126096',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, true> 4x1x1 576x1x1 115856',
+                'bnf_bwd_apply_wide_kernel<8, 1, true, true, true, true> 4x1x1 576x1x1 161936',
+            ],
+        },
+        '0': REFUSED,
+    },
+    'skeleton_fast/5': {
+        '1': {
+            'fwd': [
+                'bn_stats_big_kernel 4x1x1 576x1x1 35840',
+                'bnf_apply_wide_kernel<8, 2, false, true> 4x1x1 576x1x1 81936',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<8, 2, false, true> 4x1x1 576x1x1 151696',
+                'bnf_bwd_apply_wide_kernel<8, 2, false, false, false, true> 4x1x1 576x1x1 161936',
+            ],
+        },
+        '0': REFUSED,
+    },
+    'skeleton_fast/6': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 512x1x1 15400',
+                'bn_apply_wide_kernel<4, 2> 8x1x1 512x1x1 64672',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 512x1x1 92528',
+                'bn_bwd_apply_wide_kernel<4, 2> 8x1x1 512x1x1 109976',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 512x1x1 92528',
+                'bn_bwd_apply_add_wide_kernel<4, 1> 8x1x1 512x1x1 71476',
+            ],
+        },
+    },
+    'skeleton_fast/7': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 320x1x1 9504',
+                'bnf_apply_wide_kernel<4, 4, false, false> 8x1x1 320x1x1 48272',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<4, 4, false, false> 8x1x1 320x1x1 84368',
+                'bnf_bwd_apply_wide_kernel<4, 4, false, false, false, false> 8x1x1 320x1x1 94608',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<4> 8x1x1 320x1x1 9504',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 320x1x1 41088',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<4, 4> 8x1x1 320x1x1 76160',
+                'bn_bwd_apply_wide_kernel<4, 4> 8x1x1 320x1x1 97216',
+            ],
+        },
+    },
+    'skeleton_fast/8': {
+        '1': {
+            'fwd': [
+                'bn_stats_kernel<1> 6x1x1 480x1x1 3600',
+                'bnf_apply_wide_kernel<4, 4, true, false> 3x1x1 256x1x1 67856',
+            ],
+            'bwd': [
+                'bnf_bwd_reduce_wide_kernel<4, 4, true, false> 3x1x1 256x1x1 94736',
+                'bnf_bwd_apply_wide_kernel<4, 4, true, true, false, false> 3x1x1 256x1x1 104976',
+            ],
+            'bwd_add': [
+                'bnf_bwd_reduce_wide_kernel<4, 4, true, false> 3x1x1 256x1x1 94736',
+                'bnf_bwd_apply_wide_kernel<4, 2, true, true, true, false> 3x1x1 256x1x1 76176',
+            ],
+        },
+        '0': {
+            'fwd': [
+                'bn_stats_kernel<1> 6x1x1 480x1x1 3600',
+                'bn_apply_wide_kernel<1, 4> 6x1x1 480x1x1 31872',
+            ],
+            'bwd': [
+                'bn_bwd_reduce_kernel<1, 4> 6x1x1 480x1x1 43328',
+                'bn_bwd_apply_wide_kernel<1, 4> 6x1x1 480x1x1 52576',
+            ],
+            'bwd_add': [
+                'bn_bwd_reduce_kernel<1, 4> 6x1x1 480x1x1 43328',
+                'bn_bwd_apply_add_wide_kernel<1, 4> 6x1x1 480x1x1 66976',
+            ],
+        },
+    },
+    'sync/parity/0': {
+        '1': {
+            'fwd_local': [
+                'bn_stats_kernel<2> 16x1x1 416x1x1 6160',
+                'bn_sync_fold_fwd_kernel 16x1x1 256x1x1 512',
+            ],
+            'fwd_global': [
+                'bn_sync_merge_fwd_kernel 3x1x1 128x1x1 0',
+                'bnf_apply_kernel<4, 4, true, false> 8x1x1 416x1x1 101136',
+            ],
+            'bwd_local': [
+                'bnf_bwd_reduce_kernel<4, 2, true, false> 8x1x1 416x1x1 76112',
+                'bn_sync_fold_bwd_kernel 16x1x1 416x1x1 640',
+            ],
+            'bwd_global': [
+                'bnf_bwd_apply_sync_kernel<4, 2, true, true, false, false> 8x1x1 416x1x1 78544',
+            ],
+        },
+        '0': {
+            'fwd_local': [
+                'bn_stats_kernel<2> 16x1x1 416x1x1 6160',
+                'bn_sync_fold_fwd_kernel 16x1x1 256x1x1 512',
+            ],
+            'fwd_global': [
+                'bn_sync_merge_fwd_kernel 3x1x1 128x1x1 0',
+                'bn_apply_kernel<2, 4> 16x1x1 416x1x1 50048',
+            ],
+            'bwd_local': [
+                'bn_bwd_reduce_kernel<2, 4> 16x1x1 416x1x1 74048',
+                'bn_sync_fold_bwd_kernel 16x1x1 416x1x1 640',
+            ],
+            'bwd_global': [
+                'bn_bwd_apply_sync_kernel<2, 4> 16x1x1 416x1x1 86752',
+            ],
+        },
+    },
+    'sync/skeleton/2': {
+        '1': {
+            'fwd_local': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bn_sync_fold_fwd_wide_kernel 8x1x1 256x1x1 2048',
+            ],
+            'fwd_global': [
+                'bn_sync_merge_fwd_kernel 3x1x1 128x1x1 0',
+                'bnf_apply_wide_kernel<8, 2, true, false> 4x1x1 352x1x1 95376',
+            ],
+            'bwd_local': [
+                'bnf_bwd_reduce_wide_kernel<8, 1, true, false> 4x1x1 352x1x1 72176',
+                'bn_sync_fold_bwd_wide_kernel 8x1x1 352x1x1 2176',
+            ],
+            'bwd_global': [
+                'bnf_bwd_apply_sync_wide_kernel<8, 1, true, true, false, false> 4x1x1 352x1x1 82288',
+            ],
+        },
+        '0': {
+            'fwd_local': [
+                'bn_stats_kernel<4> 8x1x1 352x1x1 10640',
+                'bn_sync_fold_fwd_wide_kernel 8x1x1 256x1x1 2048',
+            ],
+            'fwd_global': [
+                'bn_sync_merge_fwd_kernel 3x1x1 128x1x1 0',
+                'bn_apply_wide_kernel<4, 4> 8x1x1 352x1x1 88192',
+            ],
+            'bwd_local': [
+                'bn_bwd_reduce_kernel<4, 2> 8x1x1 352x1x1 63968',
+                'bn_sync_fold_bwd_wide_kernel 8x1x1 352x1x1 2176',
+            ],
+            'bwd_global': [
+                'bn_bwd_apply_sync_wide_kernel<4, 2> 8x1x1 352x1x1 76528',
+            ],
+        },
+    },
+}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("fast", ["1", "0"])
+def test_bn_kernel_launches(fast, monkeypatch):
+    monkeypatch.setenv("DSTD_BN_FAST", fast)
+    for cid, case in BN_CASES.items():
+        want = BN_LAUNCHES[cid].get(fast, BN_LAUNCHES[cid]['1'])
+        if want == REFUSED:
+            with pytest.raises(RuntimeError, match="4096 positions"):
+                bn_launches(case)
+        else:
+            assert bn_launches(case) == want, (cid, fast)
+    for cid in BN_SYNC_CASES:
+        want = BN_LAUNCHES["sync/" + cid]
+        assert bn_sync_launches(BN_CASES[cid]) == want.get(fast, want['1']), (cid, fast)
