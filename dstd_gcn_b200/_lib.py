@@ -107,9 +107,17 @@ SYMBOLS = {
     "dstd_prep_backward": (C.c_int, [View, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dstd_finish_forward": (C.c_int, [View, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dstd_finish_backward": (C.c_int, [C.c_void_p, View, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "dstd_prep_forward_d": (C.c_int, [C.c_void_p, View, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "dstd_prep_backward_d": (C.c_int, [View, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "dstd_finish_forward_d": (C.c_int, [View, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "dstd_finish_backward_d": (C.c_int, [C.c_void_p, View, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                         C.c_void_p]),
     "dstd_mpjpe_workspace_bytes": (C.c_size_t, [C.c_longlong]),
     "dstd_mpjpe_forward_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_float, C.c_int, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dstd_pose_error_workspace_bytes": (C.c_size_t, [C.c_longlong]),
+    "dstd_pose_error_forward_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_int,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "dstd_adam_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_float, C.c_float,
                                  C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p, C.c_void_p,
                                  C.c_void_p]),
@@ -431,33 +439,49 @@ class CudaBackend:
         self._ok(self.lib.dstd_chmix_backward(C.byref(a), _stream()), "dstd_chmix_backward")
         return gx, gw, gb
 
-    # -- head / tail
+    # -- head / tail: x [N,T,V,D]; D = 3 (xyz) runs the original entry points, any other D their `_d` twins
     def prep_forward(self, x):
-        n, t, v, c = x.shape
-        assert c == 3
-        h = torch.empty((n, 6, t, v), dtype=torch.float32, device=x.device)
-        self._ok(self.lib.dstd_prep_forward(_cptr(x, "x"), _view(h, "h"), n, t, v, _stream()), "dstd_prep_forward")
+        n, t, v, d = x.shape
+        h = torch.empty((n, 2 * d, t, v), dtype=torch.float32, device=x.device)
+        if d == 3:
+            self._ok(self.lib.dstd_prep_forward(_cptr(x, "x"), _view(h, "h"), n, t, v, _stream()), "dstd_prep_forward")
+        else:
+            self._ok(self.lib.dstd_prep_forward_d(_cptr(x, "x"), _view(h, "h"), n, t, v, d, _stream()),
+                     "dstd_prep_forward_d")
         return h
 
     def prep_backward(self, gh):
-        n, _, t, v = gh.shape
-        gx = torch.empty((n, t, v, 3), dtype=torch.float32, device=gh.device)
-        self._ok(self.lib.dstd_prep_backward(_view(gh, "gh"), _ptr(gx), n, t, v, _stream()), "dstd_prep_backward")
+        n, c, t, v = gh.shape
+        d = c // 2
+        gx = torch.empty((n, t, v, d), dtype=torch.float32, device=gh.device)
+        if d == 3:
+            self._ok(self.lib.dstd_prep_backward(_view(gh, "gh"), _ptr(gx), n, t, v, _stream()), "dstd_prep_backward")
+        else:
+            self._ok(self.lib.dstd_prep_backward_d(_view(gh, "gh"), _ptr(gx), n, t, v, d, _stream()),
+                     "dstd_prep_backward_d")
         return gx
 
     def finish_forward(self, z, x):
-        n, t, v, _ = x.shape
+        n, t, v, d = x.shape
         y = torch.empty_like(x)
-        self._ok(self.lib.dstd_finish_forward(_view(z, "z"), _cptr(x, "x"), _ptr(y), n, t, v, _stream()),
-                 "dstd_finish_forward")
+        if d == 3:
+            self._ok(self.lib.dstd_finish_forward(_view(z, "z"), _cptr(x, "x"), _ptr(y), n, t, v, _stream()),
+                     "dstd_finish_forward")
+        else:
+            self._ok(self.lib.dstd_finish_forward_d(_view(z, "z"), _cptr(x, "x"), _ptr(y), n, t, v, d, _stream()),
+                     "dstd_finish_forward_d")
         return y
 
     def finish_backward(self, gy, need_gx=True):
-        n, t, v, _ = gy.shape
-        gz = torch.empty((n, 3, t, v), dtype=torch.float32, device=gy.device)
+        n, t, v, d = gy.shape
+        gz = torch.empty((n, d, t, v), dtype=torch.float32, device=gy.device)
         gx = torch.empty_like(gy) if need_gx else None
-        self._ok(self.lib.dstd_finish_backward(_cptr(gy, "gy"), _view(gz, "gz"), _ptr(gx), n, t, v, _stream()),
-                 "dstd_finish_backward")
+        if d == 3:
+            self._ok(self.lib.dstd_finish_backward(_cptr(gy, "gy"), _view(gz, "gz"), _ptr(gx), n, t, v, _stream()),
+                     "dstd_finish_backward")
+        else:
+            self._ok(self.lib.dstd_finish_backward_d(_cptr(gy, "gy"), _view(gz, "gz"), _ptr(gx), n, t, v, d,
+                                                     _stream()), "dstd_finish_backward_d")
         return gz, gx
 
     # -- engine glue
@@ -468,6 +492,17 @@ class CudaBackend:
         self._ok(self.lib.dstd_mpjpe_forward_backward(_cptr(pred, "pred"), _cptr(target, "target"), j, scale,
                                                       int(accumulate), _cptr(loss_accum, "loss"), _ptr(gpred),
                                                       _ptr(ws), ws.numel(), _stream()), "dstd_mpjpe_forward_backward")
+        return gpred
+
+    def pose_error(self, pred, target, scale, loss_accum, accumulate, dims):
+        """mpjpe over D = ``dims`` coordinates per joint (the D-generic entry point)."""
+        j = pred.numel() // dims
+        gpred = torch.empty_like(pred)
+        ws = self._ws(self.lib.dstd_pose_error_workspace_bytes(j), pred.device)
+        self._ok(self.lib.dstd_pose_error_forward_backward(_cptr(pred, "pred"), _cptr(target, "target"), j, dims, scale,
+                                                           int(accumulate), _cptr(loss_accum, "loss"), _ptr(gpred),
+                                                           _ptr(ws), ws.numel(), _stream()),
+                 "dstd_pose_error_forward_backward")
         return gpred
 
     def adam_step(self, param, grad, exp_avg, exp_avg_sq, lr, beta1, beta2, eps, weight_decay, grad_scale, step,

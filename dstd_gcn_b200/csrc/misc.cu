@@ -153,6 +153,124 @@ __global__ void mpjpe_finish_kernel(const float* __restrict__ partial, int nblk,
   }
 }
 
+// ------------------------------------------------------------------------------------------ any coordinate count D
+// The same head, tail and loss for x [N,T,V,D], 1 <= D <= MAX_COORDS (DSTDGCN(input_channels = 2D)).  The kernels above
+// keep serving D = 3.  Coalescing: every [N,T,V,D] array (x, y, gx, gy, pred, target, gpred) is walked one float per
+// thread in memory order, so a warp reads or writes 32 consecutive floats whatever D is; no thread steps through a
+// D-float row.  The [N,C,T,V] side goes through the caller's view: consecutive threads touch D channel planes, each at
+// consecutive joints.  Each element's arithmetic, and its order, is that of the D = 3 kernels, so D = 3 gives their bits.
+constexpr int MAX_COORDS = 32;
+
+// flat element e of a contiguous [N,T,V,D] array -> (n, t, v, c) and the element of the same (n, v, c) at t = T-1
+struct PoseElem {
+  int n, t, v, c;
+  long long last;
+};
+
+__device__ __forceinline__ PoseElem pose_elem(long long e, int T, int V, int D) {
+  PoseElem p;
+  const long long i = e / D;
+  p.c = (int)(e - i * D);
+  p.v = (int)(i % V);
+  const long long r = i / V;
+  p.t = (int)(r % T);
+  p.n = (int)(r / T);
+  p.last = (((long long)p.n * T + (T - 1)) * V + p.v) * D + p.c;
+  return p;
+}
+
+__global__ void prep_fwd_d_kernel(const float* __restrict__ x, View4 h, int N, int T, int V, int D) {
+  const long long total = (long long)N * T * V * D;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const PoseElem p = pose_elem(e, T, V, D);
+    const float a = __ldg(x + e);
+    h.p[vix(h, p.n, p.c, p.t, p.v)] = a;
+    h.p[vix(h, p.n, p.c + D, p.t, p.v)] = a - __ldg(x + p.last);
+  }
+}
+
+// gx[n,t,v,c] = gh[n,c,t,v] + gh[n,D+c,t,v] - (t == T-1) * sum_t' gh[n,D+c,t',v]
+__global__ void prep_bwd_d_kernel(View4 gh, float* __restrict__ gx, int N, int T, int V, int D) {
+  const long long total = (long long)N * T * V * D;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const PoseElem p = pose_elem(e, T, V, D);
+    float g = gh.p[vix(gh, p.n, p.c, p.t, p.v)] + gh.p[vix(gh, p.n, p.c + D, p.t, p.v)];
+    if (p.t == T - 1) {
+      float s = 0.f;
+      for (int u = 0; u < T; ++u) s += gh.p[vix(gh, p.n, p.c + D, u, p.v)];
+      g -= s;
+    }
+    gx[e] = g;
+  }
+}
+
+__global__ void finish_fwd_d_kernel(View4 z, const float* __restrict__ x, float* __restrict__ y, int N, int T, int V,
+                                    int D) {
+  const long long total = (long long)N * T * V * D;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const PoseElem p = pose_elem(e, T, V, D);
+    y[e] = z.p[vix(z, p.n, p.c, p.t, p.v)] + __ldg(x + p.last);
+  }
+}
+
+// the t = T-1 column sum reads gy at stride V*D per frame, but the threads of a warp read consecutive floats each frame
+__global__ void finish_bwd_d_kernel(const float* __restrict__ gy, View4 gz, float* __restrict__ gx, int N, int T, int V,
+                                    int D) {
+  const long long total = (long long)N * T * V * D;
+  const long long frame = (long long)V * D;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const PoseElem p = pose_elem(e, T, V, D);
+    gz.p[vix(gz, p.n, p.c, p.t, p.v)] = __ldg(gy + e);
+    if (gx) {
+      float s = 0.f;
+      if (p.t == T - 1)
+        for (int u = 0; u < T; ++u) s += __ldg(gy + p.last - (long long)(T - 1 - u) * frame);
+      gx[e] = s;
+    }
+  }
+}
+
+// Pose error over J D-vectors.  Thread j of a block owns joint j of the block's current tile of MPJPE_THREADS joints, as
+// in mpjpe_kernel (same joints per thread, same order, same block sum, so the partials and the loss are deterministic
+// and at D = 3 equal mpjpe_kernel's).  The tile's pred - target is staged through shared memory with coalesced loads, the
+// gradient leaves the same way.  Rows are padded to an odd stride so that the per-joint row reads hit 32 banks.
+__global__ void __launch_bounds__(MPJPE_THREADS) pose_error_kernel(const float* __restrict__ pred,
+                                                                   const float* __restrict__ target, long long J, int D,
+                                                                   float gscale, float* __restrict__ gpred,
+                                                                   float* __restrict__ partial) {
+  extern __shared__ float tile[];   // [MPJPE_THREADS][D | 1]
+  __shared__ float red[32];
+  const int ld = D | 1;
+  float acc = 0.f;
+  for (long long j0 = blockIdx.x * (long long)MPJPE_THREADS; j0 < J; j0 += (long long)gridDim.x * MPJPE_THREADS) {
+    const int nj = (int)min((long long)MPJPE_THREADS, J - j0);
+    const long long off = j0 * D;
+    for (int e = threadIdx.x; e < nj * D; e += MPJPE_THREADS) {
+      const int r = e / D;
+      tile[r * ld + (e - r * D)] = pred[off + e] - target[off + e];
+    }
+    __syncthreads();
+    if (threadIdx.x < nj) {
+      float* d = tile + threadIdx.x * ld;
+      // the contraction mpjpe_kernel's dx*dx + dy*dy + dz*dz compiles to
+      float ss = D == 1 ? d[0] * d[0] : fmaf(d[0], d[0], d[1] * d[1]);
+      for (int c = 2; c < D; ++c) ss = fmaf(d[c], d[c], ss);
+      const float nrm = sqrtf(ss);
+      acc += nrm;
+      const float inv = nrm > 0.f ? gscale / nrm : 0.f;
+      for (int c = 0; c < D; ++c) d[c] *= inv;
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < nj * D; e += MPJPE_THREADS) {
+      const int r = e / D;
+      gpred[off + e] = tile[r * ld + (e - r * D)];
+    }
+    __syncthreads();
+  }
+  float tot = block_sum(acc, red);
+  if (threadIdx.x == 0) partial[blockIdx.x] = tot;
+}
+
 // ------------------------------------------------------------------------------------------ Adam
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, long long n, float lr, float b1, float b2, float eps, float wd,
@@ -239,6 +357,72 @@ extern "C" int dstd_mpjpe_forward_backward(const float* pred, const float* targe
   mpjpe_finish_kernel<<<1, 256, 0, st>>>(partial, nblk, scale / (float)J, accumulate, loss_out);
   count_launch();
   return check_launch("mpjpe_finish");
+}
+
+#define REQUIRE_COORDS(what, D)                                                                                    \
+  DSTD_REQUIRE((D) >= 1 && (D) <= MAX_COORDS, DSTD_ERR_UNSUPPORTED,                                                \
+               what ": D=%d coordinates per joint outside the supported 1..%d", (D), MAX_COORDS)
+
+extern "C" int dstd_prep_forward_d(const float* x, dstd_view h, int N, int T, int V, int D, dstd_stream_t stream) {
+  DSTD_REQUIRE(x && h.ptr && N > 0 && T > 0 && V > 0, DSTD_ERR_BAD_ARG, "prep_forward_d: bad args");
+  REQUIRE_COORDS("prep_forward_d", D);
+  prep_fwd_d_kernel<<<grid_for((long long)N * T * V * D, 256), 256, 0, (cudaStream_t)stream>>>(x, mk(h), N, T, V, D);
+  count_launch();
+  return check_launch("prep_fwd_d");
+}
+
+extern "C" int dstd_prep_backward_d(dstd_view gh, float* gx, int N, int T, int V, int D, dstd_stream_t stream) {
+  DSTD_REQUIRE(gx && gh.ptr && N > 0 && T > 0 && V > 0, DSTD_ERR_BAD_ARG, "prep_backward_d: bad args");
+  REQUIRE_COORDS("prep_backward_d", D);
+  prep_bwd_d_kernel<<<grid_for((long long)N * T * V * D, 256), 256, 0, (cudaStream_t)stream>>>(mk(gh), gx, N, T, V, D);
+  count_launch();
+  return check_launch("prep_bwd_d");
+}
+
+extern "C" int dstd_finish_forward_d(dstd_view z, const float* x, float* y, int N, int T, int V, int D,
+                                     dstd_stream_t stream) {
+  DSTD_REQUIRE(x && y && z.ptr && N > 0 && T > 0 && V > 0, DSTD_ERR_BAD_ARG, "finish_forward_d: bad args");
+  REQUIRE_COORDS("finish_forward_d", D);
+  finish_fwd_d_kernel<<<grid_for((long long)N * T * V * D, 256), 256, 0, (cudaStream_t)stream>>>(mk(z), x, y, N, T, V,
+                                                                                                 D);
+  count_launch();
+  return check_launch("finish_fwd_d");
+}
+
+extern "C" int dstd_finish_backward_d(const float* gy, dstd_view gz, float* gx, int N, int T, int V, int D,
+                                      dstd_stream_t stream) {
+  DSTD_REQUIRE(gy && gz.ptr && N > 0 && T > 0 && V > 0, DSTD_ERR_BAD_ARG, "finish_backward_d: bad args");
+  REQUIRE_COORDS("finish_backward_d", D);
+  finish_bwd_d_kernel<<<grid_for((long long)N * T * V * D, 256), 256, 0, (cudaStream_t)stream>>>(gy, mk(gz), gx, N, T,
+                                                                                                 V, D);
+  count_launch();
+  return check_launch("finish_bwd_d");
+}
+
+extern "C" size_t dstd_pose_error_workspace_bytes(long long J) {
+  (void)J;
+  return arena_need({(size_t)MPJPE_BLOCKS * sizeof(float)});
+}
+
+extern "C" int dstd_pose_error_forward_backward(const float* pred, const float* target, long long J, int D, float scale,
+                                                int accumulate, float* loss_out, float* gpred, void* ws,
+                                                size_t ws_bytes, dstd_stream_t stream) {
+  DSTD_REQUIRE(pred && target && loss_out && gpred && J > 0, DSTD_ERR_BAD_ARG, "pose_error: bad args");
+  REQUIRE_COORDS("pose_error", D);
+  DSTD_REQUIRE(ws && ws_bytes >= dstd_pose_error_workspace_bytes(J), DSTD_ERR_WORKSPACE,
+               "pose_error: workspace too small");
+  Arena ar(ws, ws_bytes);
+  float* partial = ar.take<float>(MPJPE_BLOCKS);
+  int nblk = (int)((J + MPJPE_THREADS - 1) / MPJPE_THREADS);
+  if (nblk > MPJPE_BLOCKS) nblk = MPJPE_BLOCKS;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t smem = (size_t)MPJPE_THREADS * (D | 1) * sizeof(float);   // <= 33 KB at D = 32
+  pose_error_kernel<<<nblk, MPJPE_THREADS, smem, st>>>(pred, target, J, D, scale / (float)J, gpred, partial);
+  count_launch();
+  DSTD_LAUNCH_CHECK("pose_error");
+  mpjpe_finish_kernel<<<1, 256, 0, st>>>(partial, nblk, scale / (float)J, accumulate, loss_out);
+  count_launch();
+  return check_launch("pose_error_finish");
 }
 
 extern "C" int dstd_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,

@@ -61,13 +61,14 @@ def _registered_mirror(layout: str):
     return lists
 
 
-def mirror(all_seqs: torch.Tensor, layout: str) -> torch.Tensor:
-    """Left/right mirrored copy of raw windows ``[N, T, 3J]`` (``get_mirror`` of dataset/h36m.py:100-116,
-    dataset/cmu.py:93-105, dataset/pw3d.py:116-128): `m[right] = src[left]`, then `m[left] = src[right]`, then negate x.
-    Runs on the tensor's device.  A layout added with ``graph.register_layout`` uses the lists registered with it."""
+def mirror(all_seqs: torch.Tensor, layout: str, dims: int = 3) -> torch.Tensor:
+    """Left/right mirrored copy of raw windows ``[N, T, D*J]`` of ``dims`` = D coordinates per joint (``get_mirror`` of
+    dataset/h36m.py:100-116, dataset/cmu.py:93-105, dataset/pw3d.py:116-128): `m[right] = src[left]`, then
+    `m[left] = src[right]`, then negate coordinate 0 (x).  Runs on the tensor's device.  A layout added with
+    ``graph.register_layout`` uses the lists registered with it."""
     right, left = _MIRROR[layout] if layout in _MIRROR else _registered_mirror(layout)
     n, t, vc = all_seqs.shape
-    src = all_seqs.view(n, t, vc // 3, 3)
+    src = all_seqs.view(n, t, vc // dims, dims)
     dev = all_seqs.device
     r, l = torch.as_tensor(right, device=dev), torch.as_tensor(left, device=dev)
     out = src.clone()
@@ -91,13 +92,13 @@ class DevicePrefetcher:
 
         for inputs, inputs_inv, targets, all_seqs in DevicePrefetcher(loader, 10, 25, dim_used, device="cuda"): ...
 
-    ``batches`` yields CPU tensors / arrays ``[N, T, 3J]`` (or tuples whose LAST element is that, like the reference's
-    dataset tuple)."""
+    ``batches`` yields CPU tensors / arrays ``[N, T, D*J]`` (or tuples whose LAST element is that, like the reference's
+    dataset tuple); ``dims`` = D coordinates per joint is what ``mirror`` needs."""
 
     def __init__(self, batches, input_n, output_n, dim_used=None, padding=True, device="cuda", mirror_layout=None,
-                 depth=2):
+                 depth=2, dims=3):
         self.batches, self.input_n, self.output_n = batches, input_n, output_n
-        self.dim_used, self.padding, self.mirror_layout = dim_used, padding, mirror_layout
+        self.dim_used, self.padding, self.mirror_layout, self.dims = dim_used, padding, mirror_layout, dims
         self.device = torch.device(device)
         self.depth = max(1, int(depth))
         self.cuda = self.device.type == "cuda"
@@ -136,6 +137,6 @@ class DevicePrefetcher:
             torch.cuda.current_stream(self.device).wait_event(ev)
             dev.record_stream(torch.cuda.current_stream(self.device))
         if self.mirror_layout is not None:
-            dev = torch.cat((dev, mirror(dev, self.mirror_layout)), dim=0)
+            dev = torch.cat((dev, mirror(dev, self.mirror_layout, self.dims)), dim=0)
         a, b, c = window_batch(dev, self.input_n, self.output_n, self.dim_used, self.padding)
         return a, b, c, dev

@@ -63,8 +63,8 @@ class FlatParams:
 class TrainStep:
     """One optimisation step of the reference engine loop on the sm_100a kernels.
 
-    ``inputs``, ``inputs_inv``, ``targets``: raw ``[N, T, 3V]`` fp32 batches already on the device (this rank's shard).
-    Returns the (device, 0-dim) loss of this rank's shard.
+    ``inputs``, ``inputs_inv``, ``targets``: raw ``[N, T, D*V]`` fp32 batches already on the device (this rank's shard),
+    D coordinates per joint as the model takes them (``model.coords``: input_channels / 2, 3 for xyz).  Returns the (device, 0-dim) loss of this rank's shard.
 
     ``sync_bn``: synchronised BatchNorm over the ranks of ``process_group`` (see the module docstring); with one rank
     it changes nothing.
@@ -133,27 +133,28 @@ class TrainStep:
 
     def loss_and_grads(self, inputs, inputs_inv, targets):
         n, t, vc = inputs.shape
-        v = vc // 3
+        d = coords(self.model)
+        v = vc // d
         scale = 0.5 if self.inverse else 1.0
         self.flat.rebind_grads()
         if self.sync_bn:
             # both passes in order on the current stream: every rank issues the BN exchanges in the same order
             with ops.sync_batch_norm(self.pg):
-                return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, vc, scale)
+                return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, d, vc, scale)
         if self.inverse and self._overlap and inputs.is_cuda:
-            return self._loss_and_grads_two_streams(inputs, inputs_inv, targets, n, t, v, vc, scale)
-        return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, vc, scale)
+            return self._loss_and_grads_two_streams(inputs, inputs_inv, targets, n, t, v, d, vc, scale)
+        return self._loss_and_grads_one_stream(inputs, inputs_inv, targets, n, t, v, d, vc, scale)
 
-    def _loss_and_grads_one_stream(self, inputs, inputs_inv, targets, n, t, v, vc, scale):
-        out = self.model(inputs.view(n, t, v, 3))
-        loss = ops.mpjpe(out.reshape(n, t, vc), targets, scale)
+    def _loss_and_grads_one_stream(self, inputs, inputs_inv, targets, n, t, v, d, vc, scale):
+        out = self.model(inputs.view(n, t, v, d))
+        loss = ops.mpjpe(out.reshape(n, t, vc), targets, scale, d)
         # the two passes share nothing but the parameters: back-propagate each as soon as its forward is done (the
         # first pass's saved activations are released before the second forward runs)
         self._pass_grads(loss, self.flat.grad)
         loss = loss.detach()
         if self.inverse:
-            out_i = self.model(inputs_inv.view(n, t, v, 3))
-            loss_i = ops.mpjpe(out_i.reshape(n, t, vc), torch.flip(targets, dims=[1]), scale)
+            out_i = self.model(inputs_inv.view(n, t, v, d))
+            loss_i = ops.mpjpe(out_i.reshape(n, t, vc), torch.flip(targets, dims=[1]), scale, d)
             if self._grad_tmp is None:
                 self._grad_tmp = torch.empty_like(self.flat.grad)
             self._pass_grads(loss_i, self._grad_tmp)
@@ -161,7 +162,7 @@ class TrainStep:
             loss = loss + loss_i.detach()
         return loss
 
-    def _loss_and_grads_two_streams(self, inputs, inputs_inv, targets, n, t, v, vc, scale):
+    def _loss_and_grads_two_streams(self, inputs, inputs_inv, targets, n, t, v, d, vc, scale):
         """The forward pass and the time-reversed pass on two streams (they share nothing but the parameters).  Every hot
         kernel is a persistent one-CTA-per-SM kernel, so the gain is not co-residency but the filling of each kernel's
         tail and set-up with CTAs of the other pass: +9 % on B200 at the H3.6M bench shape (24.7 vs 27.0 ms/step).
@@ -174,12 +175,12 @@ class TrainStep:
             self._grad_tmp = torch.empty_like(self.flat.grad)
         side = self._side
         side.wait_stream(main)
-        out = self.model(inputs.view(n, t, v, 3))
-        loss = ops.mpjpe(out.reshape(n, t, vc), targets, scale)
+        out = self.model(inputs.view(n, t, v, d))
+        loss = ops.mpjpe(out.reshape(n, t, vc), targets, scale, d)
         self._pass_grads(loss, self.flat.grad)
         with torch.cuda.stream(side), ops.defer_bn_updates() as deferred:
-            out_i = self.model(inputs_inv.view(n, t, v, 3))
-            loss_i = ops.mpjpe(out_i.reshape(n, t, vc), torch.flip(targets, dims=[1]), scale)
+            out_i = self.model(inputs_inv.view(n, t, v, d))
+            loss_i = ops.mpjpe(out_i.reshape(n, t, vc), torch.flip(targets, dims=[1]), scale, d)
             self._pass_grads(loss_i, self._grad_tmp)
             loss_i = loss_i.detach()
         main.wait_stream(side)
@@ -265,11 +266,18 @@ class TrainStep:
         return self
 
 
+def coords(model):
+    """Coordinates per joint of the model's input (``DSTDGCN.coords``: input_channels / 2); 3 (xyz) for a module that
+    does not say."""
+    return int(getattr(model, "coords", 3))
+
+
 @torch.no_grad()
 def predict(model, inputs):
-    """Eval-mode forward on raw ``[N, T, 3V]`` batches (engine/prediction.py:340-353)."""
+    """Eval-mode forward on raw ``[N, T, D*V]`` batches (engine/prediction.py:340-353), D = ``coords(model)``."""
     n, t, vc = inputs.shape
-    return model(inputs.view(n, t, vc // 3, 3)).reshape(n, -1, vc)
+    d = coords(model)
+    return model(inputs.view(n, t, vc // d, d)).reshape(n, -1, vc)
 
 
 _EVAL_STREAMS = {}
@@ -277,7 +285,7 @@ _EVAL_STREAMS = {}
 
 @torch.no_grad()
 def forward_overlapped(model, x, parts=2):
-    """Eval-mode forward of ``x [N, T, V, 3]`` as ``parts`` independent sub-batches on separate streams.
+    """Eval-mode forward of ``x [N, T, V, D]`` as ``parts`` independent sub-batches on separate streams.
 
     In eval mode (BatchNorm on running statistics, engine/prediction.py:340-353) the samples of a batch do not
     interact, so the sub-batches are independent kernel chains: the persistent one-CTA-per-SM kernels of one chain
@@ -310,12 +318,13 @@ def forward_overlapped(model, x, parts=2):
 def evaluate(model, batches, input_n, eval_frame, dim_used=None, joint_to_ignore=None, joint_equal=None):
     """Per-frame MPJPE of ``PredictionEngine.test`` (engine/prediction.py:319-430) on the sm_100a forward.
 
-    ``batches`` yields ``(inputs [N, T, 3V], all_seqs [N, T_all, 3J])`` (the 1st and 4th element of the reference's
-    dataset tuple) already on the model's device.  The prediction is scattered into a copy of the ground truth at
+    ``batches`` yields ``(inputs [N, T, D*V], all_seqs [N, T_all, D*J])`` (the 1st and 4th element of the reference's
+    dataset tuple) already on the model's device, D = ``coords(model)`` coordinates per joint.  The prediction is scattered into a copy of the ground truth at
     ``dim_used`` (:374-379), ignored joints take the value of their ``joint_equal`` twin (:385-390), and the metric
     at output frame ``eval_frame[k]`` is the batch-size-weighted mean joint distance (:395-406).
     Returns ``(average over all eval frames and batches, per-frame metric)`` like the reference (``t_l.avg, t_metric``)."""
     eval_frame = [int(j) for j in eval_frame]
+    d = coords(model)
     was_training = model.training
     model.eval()
     metric = torch.zeros(len(eval_frame), dtype=torch.float64)
@@ -340,9 +349,9 @@ def evaluate(model, batches, input_n, eval_frame, dim_used=None, joint_to_ignore
             ign = torch.as_tensor(joint_to_ignore, dtype=torch.long, device=pred.device)
             eq = torch.as_tensor(joint_equal, dtype=torch.long, device=pred.device)
             assert ign.shape == eq.shape
-            pred[:, :, torch.cat((ign * 3, ign * 3 + 1, ign * 3 + 2))] = pred[:, :, torch.cat((eq * 3, eq * 3 + 1, eq * 3 + 2))]
-        p3 = pred.view(n, seq_len, -1, 3)[:, input_n:]
-        t3 = all_seqs.view(n, seq_len, -1, 3)[:, input_n:]
+            pred[:, :, torch.cat([ign * d + c for c in range(d)])] = pred[:, :, torch.cat([eq * d + c for c in range(d)])]
+        p3 = pred.view(n, seq_len, -1, d)[:, input_n:]
+        t3 = all_seqs.view(n, seq_len, -1, d)[:, input_n:]
         fr = torch.as_tensor(eval_frame, dtype=torch.long, device=pred.device)
         dist_ = torch.linalg.vector_norm(t3[:, fr] - p3[:, fr], dim=-1).mean(dim=(0, 2))   # one device->host read per batch
         metric += dist_.double().cpu() * n

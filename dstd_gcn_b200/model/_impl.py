@@ -293,6 +293,7 @@ class _DSTDGCNBase(nn.Module):
     def __init__(self, input_channels, input_time_frame, output_time_frame, st_gcnn_dropout, joints_to_consider,
                  num_feature=64, num_layers=7, layout="h36m"):
         super().__init__()
+        self.input_channels = input_channels
         self.input_time_frame = input_time_frame
         self.output_time_frame = output_time_frame
         self.joints_to_consider = joints_to_consider
@@ -326,11 +327,22 @@ class _DSTDGCNBase(nn.Module):
             return self.do_in(torch.ones((n, c, t, v), dtype=torch.float32, device=device))
         return None
 
+    @property
+    def coords(self):
+        """Coordinates per joint of the input pose x [N, T, V, D]: D = input_channels / 2 (3 for xyz)."""
+        return self.input_channels // 2
+
     def forward(self, x):
-        n, t, v, c = x.shape
+        n, t, v, d = x.shape
         assert t == self.input_time_frame + self.output_time_frame
-        if c != 3 or self.conv_st_in.stgcn[0][0].conv_s[0].in_channels != 6:
-            raise NotImplementedError("the fused head/tail kernels implement the reference's xyz (3 -> 6 channel) input")
+        if self.input_channels != 2 * d:
+            # the network reads cat(x, x - x[:, -1:]): 2*D channels (model/dstdgcn.py:298-303)
+            raise ValueError(f"input_channels = {self.input_channels} needs x [N, T, V, input_channels / 2]"
+                             f"{'' if self.input_channels % 2 else f' = {self.input_channels // 2}'}"
+                             f" coordinates per joint; x has {d}")
+        if d > ops.MAX_COORDS:
+            raise NotImplementedError(f"the head/tail kernels take at most {ops.MAX_COORDS} coordinates per joint "
+                                      f"(input_channels <= {2 * ops.MAX_COORDS}); got {d}")
         fast = self._fast
         h = ops.prep(x)
         z = self.conv_st_in.run(h)

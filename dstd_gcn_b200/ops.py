@@ -241,6 +241,16 @@ def _(pred, target, loss, scale, accumulate):
     return torch.empty_like(pred)
 
 
+@torch.library.custom_op("dstd_b200::pose_error", mutates_args=("loss",))
+def pose_error_op(pred: Tensor, target: Tensor, loss: Tensor, scale: float, accumulate: bool, dims: int) -> Tensor:
+    return _lib.backend().pose_error(pred, target, scale, loss, accumulate, dims)
+
+
+@pose_error_op.register_fake
+def _(pred, target, loss, scale, accumulate, dims):
+    return torch.empty_like(pred)
+
+
 @torch.library.custom_op("dstd_b200::adam_step", mutates_args=("param", "exp_avg", "exp_avg_sq"))
 def adam_step(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, lr: float, beta1: float, beta2: float,
               eps: float, weight_decay: float, grad_scale: float, step: int, lr_dev: Optional[Tensor] = None,
@@ -520,32 +530,43 @@ class _Finish(torch.autograd.Function):
         return gz, _opt(gx)
 
 
+# coordinates per joint the head, tail and loss kernels take (DSTDGCN(input_channels = 2 * D))
+MAX_COORDS = 32
+
+
 def prep(x):
-    """[N,T,V,3] -> motion-augmented [N,6,T,V] (model/dstdgcn.py:298-303)."""
+    """[N,T,V,D] -> motion-augmented [N,2D,T,V] (model/dstdgcn.py:298-303)."""
     return _Prep.apply(x.contiguous())
 
 
 def finish(z, x):
-    """[N,3,T,V] (+ last observed frame of x) -> [N,T,V,3] (model/dstdgcn.py:314-315)."""
+    """[N,D,T,V] (+ last observed frame of x) -> [N,T,V,D] (model/dstdgcn.py:314-315)."""
     return _Finish.apply(z, x.contiguous())
 
 
 class _Mpjpe(torch.autograd.Function):
-    """scale * mean ||pred - target||_2 ; the gradient is produced in the same kernel pass."""
+    """scale * mean ||pred - target||_2 over D-vectors; the gradient is produced in the same kernel pass."""
 
     @staticmethod
-    def forward(ctx, pred, target, scale):
+    def forward(ctx, pred, target, scale, dims):
         loss = torch.zeros((), dtype=torch.float32, device=pred.device)
-        g = torch.ops.dstd_b200.mpjpe(pred, target, loss, scale, False)
+        if dims == 3:
+            g = torch.ops.dstd_b200.mpjpe(pred, target, loss, scale, False)
+        else:
+            g = torch.ops.dstd_b200.pose_error(pred, target, loss, scale, False, dims)
         ctx.save_for_backward(g)
         return loss
 
     @staticmethod
     def backward(ctx, gl):
         (g,) = ctx.saved_tensors
-        return g * gl, None, None
+        return g * gl, None, None, None
 
 
-def mpjpe(pred, target, scale=1.0):
-    """Mean per-joint position error (engine/utils/loss.py:52-65) with fused gradient."""
-    return _Mpjpe.apply(pred.contiguous(), target.contiguous(), float(scale))
+def mpjpe(pred, target, scale=1.0, dims=3):
+    """Mean per-joint position error (engine/utils/loss.py:52-65) with fused gradient: the mean L2 norm over the
+    ``dims``-float vectors of ``pred - target`` (``dims`` = 3: xyz joints; 1 .. 32 supported)."""
+    dims = int(dims)
+    if dims != 3 and (not 1 <= dims <= MAX_COORDS or pred.numel() % dims):
+        raise ValueError(f"mpjpe: dims={dims} must be in 1..{MAX_COORDS} and divide pred's {pred.numel()} elements")
+    return _Mpjpe.apply(pred.contiguous(), target.contiguous(), float(scale), dims)

@@ -240,6 +240,13 @@ int dstd_prep_backward(dstd_view gh, float* gx, int N, int T, int V, dstd_stream
 int dstd_finish_forward(dstd_view z, const float* x, float* y, int N, int T, int V, dstd_stream_t stream);
 /* gz[n,c,t,v] = gy[n,t,v,c]; gx[n,t,v,c] = (t == T-1) ? sum_t' gy[n,t',v,c] : 0 (gx may be NULL) */
 int dstd_finish_backward(const float* gy, dstd_view gz, float* gx, int N, int T, int V, dstd_stream_t stream);
+/* The same four for D coordinates per joint, 1 <= D <= 32 (DSTDGCN(input_channels = 2*D)): x, y, gx, gy are contiguous
+ * [N,T,V,D], h / gh have 2*D channels, z / gz have D.  D = 3 computes the bits of the calls above.  D outside 1..32:
+ * DSTD_ERR_UNSUPPORTED. */
+int dstd_prep_forward_d(const float* x, dstd_view h, int N, int T, int V, int D, dstd_stream_t stream);
+int dstd_prep_backward_d(dstd_view gh, float* gx, int N, int T, int V, int D, dstd_stream_t stream);
+int dstd_finish_forward_d(dstd_view z, const float* x, float* y, int N, int T, int V, int D, dstd_stream_t stream);
+int dstd_finish_backward_d(const float* gy, dstd_view gz, float* gx, int N, int T, int V, int D, dstd_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Engine glue on device (engine/prediction.py:253-258,290-294; engine/utils/loss.py:52-65):
@@ -255,6 +262,13 @@ int dstd_finish_backward(const float* gy, dstd_view gz, float* gx, int N, int T,
 size_t dstd_mpjpe_workspace_bytes(long long J);
 int dstd_mpjpe_forward_backward(const float* pred, const float* target, long long J, float scale, int accumulate,
                                 float* loss_out, float* gpred, void* ws, size_t ws_bytes, dstd_stream_t stream);
+/* pose error: mpjpe over J D-vectors, 1 <= D <= 32 (pred, target, gpred contiguous [J,D]); same deterministic
+ * two-kernel reduction, accumulate and scale; D = 3 computes the bits of dstd_mpjpe_forward_backward.  D outside
+ * 1..32: DSTD_ERR_UNSUPPORTED. */
+size_t dstd_pose_error_workspace_bytes(long long J);
+int dstd_pose_error_forward_backward(const float* pred, const float* target, long long J, int D, float scale,
+                                     int accumulate, float* loss_out, float* gpred, void* ws, size_t ws_bytes,
+                                     dstd_stream_t stream);
 int dstd_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,
                    float beta1, float beta2, float eps, float weight_decay, float grad_scale, int step,
                    const float* lr_dev, const int* step_dev, dstd_stream_t stream);
